@@ -3,16 +3,20 @@
 bench.py -- headline benchmark of the AVA VAE hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one full VAE train step (forward + ELBO + backward + Adam) on one batch of
 synthetic 128x128 spectrograms, `--batch` per GPU (default 1024, the per-GPU batch of
-BASELINE.json's configs[1]/[2]).  Prints ONE JSON line (see the contract in the task
-statement): `value` = whole-job samples/s with inputs resident in HBM, `e2e` = the same
-through the public API with pinned host batches (H2D inside the timed region and a D2H
-read of the loss every step), `roofline` for the dominant entry point (CUDA-event timed per
-native call on the launching stream, in a second identical K-step loop so that the event
-records do not slow the `value` loop), `cpu_baseline` = the oracle's CPU train step timed
-on the host cores (rank 0, N=1 only).
+BASELINE.json's configs[1]/[2]).  Prints ONE JSON line: `value` = whole-job samples/s with
+inputs resident in HBM, `e2e` = the same through the public API with pinned host batches
+(H2D inside the timed region and a D2H read of the loss every step), `roofline` for the
+dominant entry point (CUDA-event timed per native call on the launching stream, in a second
+identical K-step loop so that the event records do not slow the `value` loop), `cpu_baseline`
+= the oracle's CPU train step timed on the host cores (rank 0, N=1 only).
+
+`--dump-outputs DIR`: after the timed loop, rank 0 writes what the last timed step handed its
+caller as DIR/<name>.npy (float32; see step_outputs).  Inputs, parameters and noise are seeded,
+so two builds run with the same arguments can be compared output for output.
 
 `--impl reference`: the CPU restatement of the reference train step (oracle/, torch CPU,
 all host threads) on the same metric; under torchrun only rank 0 works.
@@ -32,6 +36,7 @@ if ROOT not in sys.path:
 PKG = "autoencoded-vocal-analysis_b200"
 METRIC = "vae_train_samples_per_sec"
 UNIT = "samples/s"
+DUMP_SAMPLE = 1 << 20     # positions kept of the 17.4 M-element parameter and gradient vectors
 
 # (cin, cout, stride, h_in, transposed) for layers 0..13
 LAYERS = [(1, 8, 1, 128, 0), (8, 8, 2, 128, 0), (8, 16, 1, 64, 0), (16, 16, 2, 64, 0),
@@ -223,6 +228,25 @@ def cpu_train_samples_per_sec(batch, steps, warmup, seed=0, threads=None):
             times.append(t1 - t0)
     total = sum(times)
     return batch * len(times) / total, 1e3 * total / len(times), torch.get_num_threads()
+
+
+def step_outputs(model, loss):
+    """What a train step hands its caller, as float32 host arrays: the loss it returns, the
+    parameters its Adam update left, the gradient it computed (grad_dict) and the BatchNorm
+    running statistics.  Parameters and gradients are concatenated in registration order (70 MB
+    each) and cut to the same seeded sample of DUMP_SAMPLE positions."""
+    import numpy as np
+    import torch
+    named = list(model.named_parameters())
+    grads = model.grad_dict()
+    params = torch.cat([p.detach().reshape(-1) for _, p in named])
+    grad = torch.cat([grads[k].reshape(-1) for k, _ in named])
+    idx = np.sort(np.random.default_rng(0).choice(params.numel(), DUMP_SAMPLE, replace=False))
+    idx = torch.from_numpy(idx).to(params.device)
+    running = torch.cat([b.reshape(-1) for _, b in model.named_buffers() if b.is_floating_point()])
+    out = {"loss": loss.detach().reshape(1), "params_sample": params[idx], "grads_sample": grad[idx],
+           "bn_running_stats": running}
+    return {k: v.float().cpu().numpy() for k, v in out.items()}
 
 
 def bind_to_gpu_numa_node(local_rank):
@@ -529,7 +553,11 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the get_latent / shotgun blocks")
     ap.add_argument("--latent-specs", type=int, default=10_000_000,
                     help="corpus size of the get_latent block (BASELINE configs[4]: 10 M)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -608,10 +636,12 @@ def main():
     align()
     ev0.record()
     for i in range(args.steps):
-        model.train_step(xs[i % 2])
+        loss = model.train_step(xs[i % 2])
         marks[i].record()        # per-step marks (diagnostic: `step_ms`); the value is ev0 -> ev1
     ev1.record()
     barrier()
+    # taken before the loops below train the model further
+    outputs = step_outputs(model, loss) if args.dump_outputs and rank == 0 else None
     per_step = [(ev0 if i == 0 else marks[i - 1]).elapsed_time(marks[i]) for i in range(args.steps)]
     launches = lib.launch_count() - launches0
     # the same K steps again with a CUDA-event pair around every native call (roofline /
@@ -763,7 +793,7 @@ def main():
             try:
                 sg_model = vae_mod.VAE(save_dir='', device_name='cuda', precision=args.precision)
                 sg_model.train()
-                extra["shotgun"] = extra_shotgun(sg_model, torch, vae_mod, 10)
+                extra["shotgun"] = extra_shotgun(sg_model, torch, vae_mod, args.steps)
                 del sg_model
             except Exception as e:  # noqa: BLE001
                 extra["shotgun"] = {"error": repr(e)}
@@ -847,6 +877,11 @@ def main():
             "dp_check": dp,
             "extra": extra,
         }
+        if outputs is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line))
     if world > 1:
         torch.cuda.synchronize()

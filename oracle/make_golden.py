@@ -13,6 +13,8 @@ not stored.  Large tensors (fc1/fc8 weight grads, x_rec at B=64) are stored as a
 digest: (sum, L2 norm, values at 4096 seeded indices).
 """
 import copy
+import importlib
+import json
 import os
 import sys
 import tempfile
@@ -672,12 +674,123 @@ def round2_cases(ref_win, ref_pre):
     print("round-2 cases: candidates", int(out["rej_seed0_candidates"]), int(out["rej_seed3_candidates"]))
 
 
+CKPT_SEED = 11
+
+
+def checkpoint_recipe(model):
+    """The state the checkpoint interchange tests save, on the reference's VAE or this package's CPU
+    model alike: seeded parameters, BatchNorm buffers and gradients, one step of the model's own
+    torch.optim.Adam (so the optimizer state is populated), epoch 4 and one train / test loss."""
+    g = torch.Generator().manual_seed(CKPT_SEED)
+    with torch.no_grad():
+        for _, p in model.named_parameters():
+            p.copy_(torch.randn(p.shape, generator=g) * 0.05)
+        for k, b in model.named_buffers():
+            if k.endswith("num_batches_tracked"):
+                b.fill_(1)
+            else:
+                b.copy_(torch.rand(b.shape, generator=g) + (0.5 if k.endswith("running_var") else 0.0))
+    for _, p in model.named_parameters():
+        p.grad = torch.randn(p.shape, generator=g) * 0.01
+    model.optimizer.step()
+    model.epoch = 4
+    model.loss['train'][3] = 12.5
+    model.loss['test'][3] = 13.5
+
+
+def _ckpt_positions(numel, salt):
+    return np.random.default_rng(1000 + salt).choice(numel, size=min(numel, 16), replace=False)
+
+
+def checkpoint_digest(ck):
+    """(structure, samples) of a checkpoint in the reference's format (ava/models/vae.py:433-446):
+    the structure as JSON -- top-level keys in order, each layer's keys / shapes / dtypes, the
+    optimizer's param_groups and per-parameter state layout, loss, epoch, z_dim, lr -- and the
+    values of every tensor at up to 16 seeded positions, in the order checkpoint_from_golden
+    rebuilds them."""
+    samples = {}
+
+    def take(key, t):
+        a = t.detach().double().reshape(-1).numpy()
+        samples["sample:" + key] = a[_ckpt_positions(a.size, len(samples))]
+    layers = {}
+    for name, v in ck.items():
+        if name in ("optimizer_state", "loss") or not isinstance(v, dict):
+            continue
+        layers[name] = [[k, list(t.shape), str(t.dtype)] for k, t in v.items()]
+        for k, t in v.items():
+            take(name + "." + k, t)
+    opt = ck["optimizer_state"]
+    state = []
+    for idx, st in opt["state"].items():
+        state.append([idx, [[k, list(t.shape), str(t.dtype)] for k, t in st.items()]])
+        for k, t in st.items():
+            take("opt.%d.%s" % (idx, k), t)
+    structure = {"top_keys": list(ck.keys()), "layers": layers,
+                 "param_groups": json.loads(json.dumps(opt["param_groups"])), "state": state,
+                 "loss": {s: [[e, float(x)] for e, x in d.items()] for s, d in ck["loss"].items()},
+                 "epoch": ck["epoch"], "z_dim": ck["z_dim"], "lr": ck["lr"],
+                 "save_dir": type(ck["save_dir"]).__name__}
+    return json.dumps(structure, sort_keys=True), samples
+
+
+def checkpoint_from_golden(g, save_dir):
+    """A checkpoint in the reference's format rebuilt from checkpoint_case.npz: the stored
+    structure, every tensor filled with seeded values and the stored samples put back at their
+    positions."""
+    s = json.loads(str(g["structure"]))
+    gen = torch.Generator().manual_seed(5)
+    n = [0]
+
+    def make(key, shape, dtype):
+        dt = getattr(torch, dtype.split(".")[1])
+        t = torch.randn(shape, generator=gen, dtype=torch.float64) if dt.is_floating_point else \
+            torch.randint(0, 9, shape, generator=gen)
+        t = t.to(dt)
+        flat = t.view(-1)
+        flat[torch.from_numpy(_ckpt_positions(flat.numel(), n[0]))] = torch.from_numpy(g["sample:" + key]).to(dt)
+        n[0] += 1
+        return t
+    ck = {}
+    for name in s["top_keys"]:
+        if name in s["layers"]:
+            ck[name] = {k: make(name + "." + k, shape, dt) for k, shape, dt in s["layers"][name]}
+    state = {idx: {k: make("opt.%d.%s" % (idx, k), shape, dt) for k, shape, dt in entries}
+             for idx, entries in s["state"]}
+    groups = [dict(pg, betas=tuple(pg["betas"])) for pg in s["param_groups"]]
+    rest = {"optimizer_state": {"state": state, "param_groups": groups},
+            "loss": {k: {e: x for e, x in v} for k, v in s["loss"].items()},
+            "z_dim": s["z_dim"], "epoch": s["epoch"], "lr": s["lr"], "save_dir": save_dir}
+    return {name: ck[name] if name in ck else rest[name] for name in s["top_keys"]}
+
+
+def checkpoint_case(vae_cls, source):
+    """tests/golden/checkpoint_case.npz: structure and sampled values of the checkpoint `vae_cls`
+    writes after checkpoint_recipe."""
+    with tempfile.TemporaryDirectory() as d:
+        model = vae_cls(save_dir=d, device_name='cpu')
+        checkpoint_recipe(model)
+        model.save_state("checkpoint_004.tar")
+        ck = torch.load(os.path.join(d, "checkpoint_004.tar"), map_location="cpu")
+    structure, samples = checkpoint_digest(ck)
+    out = dict(samples, structure=np.array(structure), source=np.array(source), versions=np.array(versions()))
+    np.savez_compressed(os.path.join(GOLDEN, "checkpoint_case.npz"), **out)
+    print("checkpoint case (%s): %d top-level keys, %d sampled tensors" % (source, len(ck), len(samples)))
+
+
 def main():
     os.makedirs(GOLDEN, exist_ok=True)
     torch.set_num_threads(8)
-    ref_vae, ref_pre, ref_win, ref_ds = _ref_import.import_reference()
     which = sys.argv[1:] or ["vae", "adam", "spec", "sampler", "process", "mmd", "container", "pca", "warped",
-                             "round2"]
+                             "round2", "checkpoint"]
+    if which == ["checkpoint"] and not _ref_import.reference_available():
+        # without the reference: this package's save_state, a line-for-line restatement of the
+        # reference's (vae.py:433-446); the interchange test checks the file against the reference
+        # wherever the reference is present
+        vae = importlib.import_module("autoencoded-vocal-analysis_b200.models.vae")
+        checkpoint_case(vae.VAE, "this package's save_state (restates ava/models/vae.py:433-446)")
+        return
+    ref_vae, ref_pre, ref_win, ref_ds = _ref_import.import_reference()
     if "vae" in which:
         vae_case(ref_vae, "vae_train_b7", seed=0, batch=7, train=True)
         vae_case(ref_vae, "vae_eval_b7", seed=1, batch=7, train=False)
@@ -701,6 +814,8 @@ def main():
         warped_case(ref_win, ref_pre)
     if "round2" in which:
         round2_cases(ref_win, ref_pre)
+    if "checkpoint" in which:
+        checkpoint_case(ref_vae.VAE, "reference ava/models/vae.py save_state")
 
 
 if __name__ == "__main__":

@@ -2,6 +2,7 @@
 (no compute calls), and the host-side mirror of the reference interface behaves like the
 reference's (parameter registration, checkpoint layout, loud failure without CUDA)."""
 import importlib
+import json
 import os
 import re
 
@@ -170,6 +171,63 @@ def test_checkpoints_interchange_with_the_real_reference(tmp_path, monkeypatch):
     ref2.forward(x).backward()
     ref2.optimizer.step()
     assert float(ref2.optimizer.state[r2params["fc1.weight"]]['step']) == 2.0
+    # the stored checkpoint golden is what the reference itself writes
+    from oracle import make_golden
+    ref3 = ref_vae.VAE(save_dir=rdir, device_name='cpu')
+    make_golden.checkpoint_recipe(ref3)
+    ref3.save_state("golden.tar")
+    structure, samples = make_golden.checkpoint_digest(torch.load(os.path.join(rdir, "golden.tar"), map_location="cpu"))
+    g = load_golden("checkpoint_case")
+    assert json.loads(structure) == json.loads(str(g["structure"]))
+    assert sorted(samples) == sorted(k for k in g.files if k.startswith("sample:"))
+    for k, v in samples.items():
+        assert np.array_equal(v, g[k]), k
+
+
+def test_checkpoints_interchange_with_reference_golden(tmp_path):
+    """The checkpoint format of the reference (ava/models/vae.py:433-472) from the stored golden
+    (tests/golden/checkpoint_case.npz: structure and sampled values of the checkpoint written after
+    oracle.make_golden.checkpoint_recipe): what this package writes has that structure and those
+    values, and a checkpoint rebuilt from the golden loads here -- parameters, BatchNorm buffers,
+    Adam moments and step, epoch and loss history -- and is written back unchanged."""
+    from oracle import make_golden
+    vae = importlib.import_module(PKG + ".models.vae")
+    g = load_golden("checkpoint_case")
+    want = json.loads(str(g["structure"]))
+    sample_keys = sorted(k for k in g.files if k.startswith("sample:"))
+
+    def check(path):
+        structure, samples = make_golden.checkpoint_digest(torch.load(path, map_location="cpu"))
+        assert json.loads(structure) == want
+        assert sorted(samples) == sample_keys
+        for k, v in samples.items():
+            assert np.array_equal(v, g[k]), k
+    # ours -> golden
+    ours = vae.VAE(save_dir=str(tmp_path), device_name='cpu')
+    make_golden.checkpoint_recipe(ours)
+    ours.save_state("ours.tar")
+    check(str(tmp_path / "ours.tar"))
+    # golden -> ours
+    ck = make_golden.checkpoint_from_golden(g, str(tmp_path))
+    torch.save(ck, str(tmp_path / "golden.tar"))
+    model = vae.VAE(save_dir=str(tmp_path), device_name='cpu')
+    model.load_state(str(tmp_path / "golden.tar"))
+    assert model.epoch == ck["epoch"] == 4 and model.loss == ck["loss"]
+    sd = model.state_dict()
+    for name, layer in ck.items():
+        if name in want["layers"]:
+            for k, t in layer.items():
+                assert torch.equal(sd[name + "." + k], t), name + "." + k
+    names = [k for k, _ in model.named_parameters()]
+    state = ck["optimizer_state"]["state"]
+    assert sorted(state) == list(range(len(names)))
+    for idx, st in state.items():
+        assert torch.equal(model._views_m[names[idx]], st["exp_avg"]), names[idx]
+        assert torch.equal(model._views_v[names[idx]], st["exp_avg_sq"]), names[idx]
+    assert model._step_host == int(state[0]["step"]) == 1
+    # ... and written back in the same format with the same values
+    model.save_state("again.tar")
+    check(str(tmp_path / "again.tar"))
 
 
 def test_time_bracketing_matches_oracle_coordinates():

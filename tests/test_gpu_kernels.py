@@ -445,8 +445,14 @@ def test_bias_grads_batched(L, M):
     L.call("ava_b200_bias_grads", jobs, len(shapes), ws.data_ptr(), need, stream())
     torch.cuda.synchronize()
     first = [o.clone() for o in outs]
-    for o, w in zip(outs, want):
-        assert rel_err(o.cpu().numpy(), w.numpy()) <= 1e-5
+    for j, (o, w) in enumerate(zip(outs, want)):
+        got, ref = o.cpu().numpy().astype(np.float64), w.numpy()
+        bad = np.flatnonzero(~(np.abs(got - ref) <= 1e-5 * np.abs(ref).max()))
+        # says which job and how: columns never written (still 3.0), NaN, or wrong sums
+        assert rel_err(got, ref) <= 1e-5, (
+            "job %d %s: %d bad columns, %d still 3.0, %d NaN; first %s got %s want %s"
+            % (j, shapes[j], bad.size, int((got[bad] == 3.0).sum()), int(np.isnan(got[bad]).sum()),
+               bad[:8].tolist(), got[bad[:8]].tolist(), ref[bad[:8]].tolist()))
     L.call("ava_b200_bias_grads", jobs, len(shapes), ws.data_ptr(), need, stream())
     torch.cuda.synchronize()
     for o, f in zip(outs, first):
