@@ -31,11 +31,8 @@ SIGNATURES = {
     "ava_b200_linear_bwd_data": (P, I, P, P, P, I, I, I, I, I, LL, LL, LL, I, I, P, LL, P),
     "ava_b200_linear_bwd_weight": (P, I, P, P, I, P, P, I, I, I, I, LL, LL, LL, LL, I, P, LL, P),
     "ava_b200_linear_ws_bytes": (I, I, I),
-    "ava_b200_linear_bwd_weight_multi": (P, I, P),
     "ava_b200_bias_grads": (P, I, P, LL, P),
     "ava_b200_bias_grads_ws_bytes": (P, I),
-    "ava_b200_mlp_fwd": (P, P),
-    "ava_b200_mlp_bwd": (P, P),
     "ava_b200_latent_fwd": (P, P, P, I, I, P, P, P, P),
     "ava_b200_latent_bwd": (P, P, P, P, P, I, I, P, P),
     "ava_b200_recon": (P, P, LL, F, P, P, P, I, I, P),

@@ -1,6 +1,5 @@
 // Error reporting / bookkeeping of the C ABI.
 #include <stdarg.h>
-#include <stdlib.h>
 
 #include <atomic>
 
@@ -16,15 +15,6 @@ void set_error(const char* fmt, ...) {
   va_start(ap, fmt);
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
-}
-
-bool pdl_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("AVA_B200_PDL");
-    on = (e != nullptr && e[0] == '1') ? 1 : 0;
-  }
-  return on != 0;
 }
 
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }

@@ -39,37 +39,6 @@ inline int check_launch(const char* what) {
     }                            \
   } while (0)
 
-// Programmatic dependent launch.  A kernel launched through launch_pdl() may be scheduled while the
-// kernel before it in the stream is still draining; it must call pdl_wait() before it reads or
-// writes anything an earlier kernel of the stream produced (parameters are the exception the
-// prologues use: within a step only the optimizer kernels write them, and those never trigger
-// their dependents early).  pdl_launch_dependents() -- always AFTER pdl_wait(), so that an early
-// started kernel only ever overlaps its immediate predecessor -- lets the next kernel's CTAs
-// take the SM resources this kernel's CTAs free as they finish, instead of waiting for the whole
-// grid to retire and a launch gap on top.  Both are no-ops for a normally launched kernel.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-// Measured (profiles/r02_summary.md): inside the captured CUDA graph of the step the attribute
-// buys nothing (7.11 vs 7.06 ms at batch 1024, 1.337 vs 1.326 ms at batch 64 -- graph launches
-// already leave no gap worth hiding), so it is OFF unless AVA_B200_PDL=1.
-bool pdl_enabled();
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
-                              Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-}
-
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -501,10 +501,6 @@ __global__ void __launch_bounds__(GconvCfg<KIND, CI, CO, TW, INMODE, TERMS>::NT,
       s_w[idx] = P.w[(size_t)co * P.w_so + (size_t)ci * P.w_si + kk];
     }
   }
-  // everything above reads parameters only and may overlap the previous kernel's tail (programmatic
-  // dependent launch, common.cuh); activations and statistics are touched from here on
-  pdl_wait();
-  pdl_launch_dependents();
   if ((int)blockIdx.x < ngroups) issue(blockIdx.x, 0, 0);
   if (INMODE == IN_AFFINE && tid < CI) {
     BnCoef k = bn_coef(P.stats, tid, P.in_count, P.gamma, P.beta, P.rmean, P.rvar, P.train != 0);
@@ -1634,7 +1630,7 @@ static int launch_gconv(const GconvParams& P, cudaStream_t stream) {
   if (make_act_map(&map_in, P.in, (long long)P.B * CI, P.H_in, P.W_in, C::BOX_W, G::IN_ROWS, C::CIC)) return 1;
   const long long ngroups = (ntiles + C::NSUB - 1) / C::NSUB;
   int grid = (int)(ngroups < max_ctas ? ngroups : max_ctas);
-  launch_pdl(kern, dim3(grid), dim3(C::NT), smem, stream, map_in, P);
+  kern<<<grid, C::NT, smem, stream>>>(map_in, P);
   return check_launch("gconv");
 }
 
@@ -1750,8 +1746,6 @@ __global__ void __launch_bounds__(256, 2)
     cv_tma_load_3d(sg, &map_g, tx * TWG, ty * T::THG, n * CG, &s_bar[st]);
     cv_tma_load_3d(sg + G_PAD, &map_i, S * tx * TWG - 4, S * ty * T::THG - 1, n * CI, &s_bar[st]);
   };
-  pdl_wait();                 // (programmatic dependent launch, common.cuh)
-  pdl_launch_dependents();
   // coefficients
   if (tid < 32) {
     const int c = tid;
@@ -2008,8 +2002,6 @@ __global__ void __launch_bounds__((((CG + 15) / 16) * (CI / 8) == 6) ? 192 : 256
     cv_tma_prefetch_3d(&map_g, tx * TWG, ty * T::THG, n * CG);
     cv_tma_prefetch_3d(&map_i, S * tx * TWG - 4, S * ty * T::THG - 1, n * CI);
   };
-  pdl_wait();                 // (programmatic dependent launch, common.cuh)
-  pdl_launch_dependents();
   if (tid < 32) {
     constexpr int CA = CONVT ? CG : CI;
     if (tid < CA) {
@@ -2264,8 +2256,8 @@ __global__ void __launch_bounds__((((CG + 15) / 16) * (CI / 8) == 6) ? 192 : 256
 constexpr int kWgradMaxCtas = 8 * kNumSMs;  // per-CTA partial slots in the workspace
 
 // Border-trimmed sums of dz: T_k[c] = sum of dz[c] over the pixels whose tap-k partner lies inside
-// the image, from the 9 per-channel sums `ts` ([slot][32] doubles) that ava_b200_dz_border_sums (or a
-// producing kernel's epilogue) accumulated:
+// the image, from the 9 per-channel sums `ts` ([slot][32] doubles) that the kernel producing dz
+// accumulated in its epilogue (as ava_b200_dz_border_sums defines them):
 //   mode 0 (conv layers, stride-1 conv-transpose): 0 total, 1 first row, 2 last row, 3 first column,
 //          4 last column, 5..8 corners (first/last row x first/last column)
 //   mode 1 (stride-2 conv-transpose; dz at 2x resolution, tap (ky,kx) reads dz[2p+k-1]):
@@ -2321,8 +2313,6 @@ struct FinalizeParams {
 constexpr int kFinWarps = 32;
 __global__ void __launch_bounds__(kFinWarps * 32) bnconv_finalize_kernel(const FinalizeParams P) {
   __shared__ double s_part[kFinWarps][33];
-  pdl_wait();
-  pdl_launch_dependents();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int j = blockIdx.x * 32 + lane;
   const int NW = P.Cx * P.Cz * 9;
@@ -2386,8 +2376,6 @@ __global__ void __launch_bounds__(kFinWarps * 32) bnconv_finalize_kernel(const F
 __global__ void __launch_bounds__(256)
 dz_border_sums_kernel(const float* __restrict__ dz, int B, int C, int H, int W, int mode, double* tsums) {
   __shared__ double s_red[8][9];
-  pdl_wait();
-  pdl_launch_dependents();
   const int c = blockIdx.y;
   const int w4 = W >> 2, hw4 = (H * W) >> 2;
   const long long total4 = (long long)B * hw4;
@@ -2457,7 +2445,7 @@ static int launch_finalize(const WgradParams& P, FinalizeParams F, int nparts, c
   F.stats = P.stats;
   F.count = P.bn_count;
   const int n = CG * CI * 9 + F.Cz;
-  launch_pdl(bnconv_finalize_kernel, dim3((n + 31) / 32), dim3(kFinWarps * 32), 0, stream, F);
+  bnconv_finalize_kernel<<<(n + 31) / 32, kFinWarps * 32, 0, stream>>>(F);
   return check_launch("bnconv_finalize");
 }
 
@@ -2491,7 +2479,7 @@ static int launch_wgrad(WgradParams P, const FinalizeParams& F, void* ws, cudaSt
   if (make_act_map(&map_g, P.g_a, (long long)P.B * CG, P.Hg, P.Wg, GW, GROWS, CG)) return 1;
   if (make_act_map(&map_i, P.i_a, (long long)P.B * CI, S * P.Hg, S * P.Wg, T::I_PITCH, T::I_ROWS, CI)) return 1;
   P.partial = reinterpret_cast<float*>(ws);
-  launch_pdl(kern, dim3(grid), dim3(256), smem, stream, map_g, map_i, P);
+  kern<<<grid, 256, smem, stream>>>(map_g, map_i, P);
   if (check_launch("wgrad")) return 1;
   return launch_finalize<S, CG, CI, CONVT>(P, F, grid, stream);
 }
@@ -2527,7 +2515,7 @@ static int launch_wgrad_mma(WgradParams P, const FinalizeParams& F, void* ws, cu
   if (make_act_map(&map_g, P.g_a, (long long)P.B * CG, P.Hg, P.Wg, T::G_W, T::G_ROWS_BOX, CG)) return 1;
   if (make_act_map(&map_i, P.i_a, (long long)P.B * CI, S * P.Hg, S * P.Wg, T::I_PITCH, T::I_ROWS_BOX, CI)) return 1;
   P.partial = reinterpret_cast<float*>(ws);
-  launch_pdl(kern, dim3(grid), dim3(NTHR), smem, stream, map_g, map_i, P);
+  kern<<<grid, NTHR, smem, stream>>>(map_g, map_i, P);
   if (check_launch("wgrad_mma")) return 1;
   return launch_finalize<S, CG, CI, CONVT>(P, F, grid, stream);
 }
@@ -2771,6 +2759,6 @@ extern "C" int ava_b200_dz_border_sums(const float* dz, int B, int C, int H, int
   int gx = (int)(want < 1 ? 1 : want);
   const int cap = (8 * kNumSMs + C - 1) / C;
   if (gx > cap) gx = cap;
-  launch_pdl(dz_border_sums_kernel, dim3(gx, C), dim3(256), 0, (cudaStream_t)stream, dz, B, C, H, W, mode, tsums);
+  dz_border_sums_kernel<<<dim3(gx, C), 256, 0, (cudaStream_t)stream>>>(dz, B, C, H, W, mode, tsums);
   return check_launch("dz_border_sums");
 }

@@ -58,25 +58,17 @@ __device__ __forceinline__ float4 mask4(float4 v, float4 m) {
   return make_float4(m.x > 0.f ? v.x : 0.f, m.y > 0.f ? v.y : 0.f, m.z > 0.f ? v.z : 0.f, m.w > 0.f ? v.w : 0.f);
 }
 
-// Tensor-core inner product for the same tiles (TERMS = 1: TF32; 3: error-compensated 3xTF32,
-// fp32-level accuracy), as in the conv kernels (conv.cu): hi = x rounded to nearest TF32,
-// lo = x - hi (exact); a_hi*b_hi per 8-deep step on a zero accumulator, a_lo*b_hi + a_hi*b_lo
-// chained separately, everything summed with round-to-nearest FADDs.
-__device__ __forceinline__ uint32_t gm_tf32_hi(float x) { return (__float_as_uint(x) + 0x1000u) & 0xFFFFE000u; }
+// Tensor-core inner product for the same tiles (TERMS = 1: single-pass TF32): each 8-deep step
+// on a zero accumulator, summed with round-to-nearest FADDs.
 __device__ __forceinline__ void gm_mma_zero(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
   asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%10,%10,%10,%10};"
       : "=f"(d[0]), "=f"(d[1]), "=f"(d[2]), "=f"(d[3])
       : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1), "f"(0.f));
 }
-__device__ __forceinline__ void gm_mma(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
 
 // A_KCONTIG: A' contiguous along k (sak == 1) else along m (sam == 1)
 // B_NCONTIG: B' contiguous along n (sbn == 1) else along k (sbk == 1)
-// TERMS: 0 = fp32 FMA (4x4 register micro-tiles); 1 / 3 = tensor cores (mma.sync m16n8k8 TF32):
+// TERMS: 0 = fp32 FMA (4x4 register micro-tiles); 1 = tensor cores (mma.sync m16n8k8 TF32):
 //   warp w owns rows 16*(w&3).. and columns 32*(w>>2).. of the 64x64 tile (4 n8 tiles); the
 //   row pitch of the staged tiles is 72 floats (8 mod 32) so fragment loads are conflict-free.
 template <bool A_KCONTIG, bool B_NCONTIG, bool MASK, int TERMS>
@@ -176,44 +168,25 @@ __device__ __forceinline__ void sgemm_body(const GemmParams& P, const int bx, co
       }
     } else {
       // acc[nt][0..3] = C fragment of n8-tile nt: rows fg / fg+8, columns 2*ft / 2*ft+1.
-      // The tensor core adds into a non-zero accumulator with truncation, so every hi*hi product
+      // The tensor core adds into a non-zero accumulator with truncation, so every product
       // block starts from a zero accumulator and is added to the running sum with a
-      // round-to-nearest FADD; only the small cross terms (2^-12 of the magnitude) are chained.
-      float cs[4][4];
+      // round-to-nearest FADD.
 #pragma unroll
       for (int ks = 0; ks < BK / 8; ++ks) {
         const int k0 = ks * 8;
         const float av[4] = {As[buf][k0 + ft][wm0 + fg], As[buf][k0 + ft][wm0 + fg + 8],
                              As[buf][k0 + ft + 4][wm0 + fg], As[buf][k0 + ft + 4][wm0 + fg + 8]};
-        uint32_t ah[4], al[4];
+        uint32_t ah[4];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          ah[j] = (TERMS == 3) ? gm_tf32_hi(av[j]) : __float_as_uint(av[j]);
-          al[j] = (TERMS == 3) ? __float_as_uint(av[j] - __uint_as_float(ah[j])) : 0u;
-        }
+        for (int j = 0; j < 4; ++j) ah[j] = __float_as_uint(av[j]);
 #pragma unroll
         for (int nt = 0; nt < 4; ++nt) {
           const float b0 = Bs[buf][k0 + ft][wn0 + nt * 8 + fg], b1 = Bs[buf][k0 + ft + 4][wn0 + nt * 8 + fg];
-          const uint32_t bh0 = (TERMS == 3) ? gm_tf32_hi(b0) : __float_as_uint(b0);
-          const uint32_t bh1 = (TERMS == 3) ? gm_tf32_hi(b1) : __float_as_uint(b1);
-          if constexpr (TERMS == 3) {
-            const uint32_t bl0 = __float_as_uint(b0 - __uint_as_float(bh0));
-            const uint32_t bl1 = __float_as_uint(b1 - __uint_as_float(bh1));
-            if (ks == 0) gm_mma_zero(cs[nt], al, bh0, bh1);
-            else gm_mma(cs[nt], al, bh0, bh1);
-            gm_mma(cs[nt], ah, bl0, bl1);
-          }
           float cf[4];
-          gm_mma_zero(cf, ah, bh0, bh1);
+          gm_mma_zero(cf, ah, __float_as_uint(b0), __float_as_uint(b1));
 #pragma unroll
           for (int j = 0; j < 4; ++j) acc[nt][j] += cf[j];
         }
-      }
-      if constexpr (TERMS == 3) {
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-          for (int j = 0; j < 4; ++j) acc[nt][j] += cs[nt][j];
       }
     }
   };
@@ -308,25 +281,8 @@ __device__ __forceinline__ void sgemm_body(const GemmParams& P, const int bx, co
 }
 
 template <bool A_KCONTIG, bool B_NCONTIG, bool MASK, int TERMS>
-__global__ void __launch_bounds__(256, TERMS == 3 ? 3 : 4) sgemm_kernel(const GemmParams P) {
+__global__ void __launch_bounds__(256, 4) sgemm_kernel(const GemmParams P) {
   sgemm_body<A_KCONTIG, B_NCONTIG, MASK, TERMS>(P, blockIdx.x, blockIdx.y, blockIdx.z);
-}
-
-// Several weight-gradient GEMMs (dW = (dY (.) mask)^T X of the small dense layers) as ONE launch: the
-// grid is the concatenation of the jobs' 64x64 output tiles, every tile reduces over the whole batch
-// (no split-K: the six small layers of the VAE happen to make 148 tiles -- one wave).
-struct GemmJobs {
-  GemmParams p[AVA_MAX_WGRAD_JOBS];
-  int blk0[AVA_MAX_WGRAD_JOBS + 1];
-  int n;
-};
-__global__ void __launch_bounds__(256, 4) sgemm_jobs_kernel(const GemmJobs J) {
-  int j = 0;
-  while (j + 1 < J.n && (int)blockIdx.x >= J.blk0[j + 1]) ++j;
-  const GemmParams& P = J.p[j];
-  const int local = blockIdx.x - J.blk0[j];
-  const int tx = (P.N + BN - 1) / BN, ty = (P.M + BM - 1) / BM;
-  sgemm_body<false, true, true, 0>(P, local % tx, (local / tx) % ty, local / (tx * ty));
 }
 
 __global__ void __launch_bounds__(256)
@@ -520,9 +476,7 @@ static int run_gemm(GemmParams P, int a_kcontig, int b_ncontig, void* ws, long l
   const bool mask = P.Amask != nullptr;
 #define AVA_GEMM_LAUNCH(AK, BNC, MK)                                                  \
   do {                                                                                \
-    if (terms == 3)                                                                   \
-      sgemm_kernel<AK, BNC, MK, 3><<<grid, 256, 0, stream>>>(P);                      \
-    else if (terms == 1)                                                              \
+    if (terms == 1)                                                                   \
       sgemm_kernel<AK, BNC, MK, 1><<<grid, 256, 0, stream>>>(P);                      \
     else                                                                              \
       sgemm_kernel<AK, BNC, MK, 0><<<grid, 256, 0, stream>>>(P);                      \
@@ -556,20 +510,14 @@ static int run_gemm(GemmParams P, int a_kcontig, int b_ncontig, void* ws, long l
 // for it to matter (>= 256 K weights): the same 64x64x16 kernel with its inner product on the
 // tensor cores (mma.sync) --
 //   precision 1 ('tf32'): single TF32 term;
-//   precision 2 ('tf32x3'/'auto'): stays on the fp32 FMA inner product.  The 3-term mma.sync
-//   variant is as accurate (measured at the fc1 shape, batch 64: 4.6e-8 rms / no bias vs
-//   6.3e-8 for FMA) but no faster: at batch 64 these GEMMs are bound by the weight stream, not
-//   by the inner product.  AVA_B200_GEMM_MMA3=1 selects it (diagnostics).
+//   precision 2 ('tf32x3'/'auto'): stays on the fp32 FMA inner product.  A 3-term (3xTF32)
+//   mma.sync inner product was measured as accurate (fc1 shape, batch 64: 4.6e-8 rms / no bias
+//   vs 6.3e-8 for FMA) but no faster: at batch 64 these GEMMs are bound by the weight stream,
+//   not by the inner product.
 static int mma_terms(int precision, int groups, int M, int N, int K) {
   (void)M;
-  if (precision < 1 || groups != 1 || (long long)N * K < (1 << 18)) return 0;
-  if (precision == 1) return 1;
-  static int force3 = -1;
-  if (force3 < 0) {
-    const char* e = getenv("AVA_B200_GEMM_MMA3");
-    force3 = (e != nullptr && e[0] == '1') ? 1 : 0;
-  }
-  return force3 ? 3 : 0;
+  if (precision != 1 || groups != 1 || (long long)N * K < (1 << 18)) return 0;
+  return 1;
 }
 
 }  // namespace ava
@@ -690,29 +638,4 @@ extern "C" int ava_b200_bias_grads(const ava_b200_bias_job* h_jobs, int njobs, v
   if (check_launch("bias_partial")) return 1;
   bias_finish_kernel<<<(col + 255) / 256, 256, 0, stream>>>(J, reinterpret_cast<const float*>(ws));
   return check_launch("bias_finish");
-}
-
-extern "C" int ava_b200_linear_bwd_weight_multi(const ava_b200_wgrad_job* h_jobs, int njobs, void* stream_) {
-  AVA_REQUIRE(h_jobs != nullptr && njobs >= 1 && njobs <= AVA_MAX_WGRAD_JOBS, "linear_bwd_weight_multi: 1..%d jobs",
-              AVA_MAX_WGRAD_JOBS);
-  GemmJobs J = {};
-  J.n = njobs;
-  int blk = 0;
-  for (int j = 0; j < njobs; ++j) {
-    const ava_b200_wgrad_job& h = h_jobs[j];
-    AVA_REQUIRE(h.dy && h.x && h.dw && h.M > 0 && h.N > 0 && h.K > 0 && h.groups >= 1, "linear_bwd_weight_multi: bad job %d", j);
-    // dW[N,K] = dY^T[N,M] . X[M,K] -> gemm (N, K, M); A'(n,m) = dY[m*lddy + n]
-    GemmParams& P = J.p[j];
-    P.A = h.dy; P.Amask = h.ymask; P.sam = 1; P.sak = h.lddy;
-    P.B = h.x; P.sbk = h.ldx; P.sbn = 1;
-    P.C = h.dw; P.ldc = h.K;
-    P.M = h.N; P.N = h.K; P.K = h.M; P.act = 0;
-    P.splits = 1; P.kchunk = (h.M + BK - 1) / BK * BK;
-    P.groups = h.groups; P.a_gs = h.dy_gs; P.b_gs = h.x_gs; P.c_gs = h.dw_gs;
-    J.blk0[j] = blk;
-    blk += ((P.M + BM - 1) / BM) * ((P.N + BN - 1) / BN) * h.groups;
-  }
-  J.blk0[njobs] = blk;
-  sgemm_jobs_kernel<<<blk, 256, 0, (cudaStream_t)stream_>>>(J);
-  return check_launch("sgemm_jobs");
 }

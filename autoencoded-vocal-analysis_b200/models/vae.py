@@ -50,32 +50,9 @@ _BN_MOMENTUM = 0.1
 # worst gradient error vs float64 4.2e-5 / 4.4e-5 / 4.0e-5 / 7.2e-5 and 191 / 191 / 260 / 403 ReLU units on
 # the other side of zero (the float32 reference itself: 129; bar: 4x that).  6 costs nothing in gradient
 # accuracy; 4 ('tf32x3c') holds the 1e-4 bar with 1.4x margin and stays opt-in.
-_AUTO_CONV_MODE = int(os.environ.get("AVA_B200_AUTO_CONV_MODE", "6"))
+_AUTO_CONV_MODE = 6
 _DP_MULTIMEM_MIN_WORLD = 4
 _DP_MAX_WORLD = 8          # AVA_DP_MAX_WORLD, include/ava_b200.h
-
-
-# The row-wise fused kernels of csrc/mlp.cu are parity-green but measured SLOWER than the per-layer
-# GEMM launches under graph replay (batch 1024: 7.32 vs 7.04 ms/step, batch 64: 1.43 vs 1.30 ms;
-# gpurun_out s16/s17): each CTA re-streams the 2.6 MB of weights for its R <= 8 rows.  Off unless asked for.
-_FUSED_MLP = os.environ.get("AVA_B200_FUSED_MLP", "0") == "1"
-
-
-class _MlpParams(ctypes.Structure):
-    """ava_b200_mlp_params (include/ava_b200.h)."""
-    _fields_ = [("B", ctypes.c_int), ("Z", ctypes.c_int), ("stages", ctypes.c_int)] + \
-        [(n, ctypes.c_void_p) for n in
-         ("w2", "b2", "w3", "b3", "w4", "b4", "w5", "b5", "w6", "b6", "w7", "b7", "eps_w", "eps_d",
-          "h1", "h2", "h3", "heads", "z", "d", "t5", "t6", "t7",
-          "dt7", "dt6", "dt5", "gz", "gheads", "dh3", "dh2", "dh1", "acc")]
-
-
-class _WgradJob(ctypes.Structure):
-    """ava_b200_wgrad_job (include/ava_b200.h)."""
-    _fields_ = [("dy", ctypes.c_void_p), ("ymask", ctypes.c_void_p), ("x", ctypes.c_void_p),
-                ("dw", ctypes.c_void_p), ("lddy", ctypes.c_int), ("ldx", ctypes.c_int), ("M", ctypes.c_int),
-                ("N", ctypes.c_int), ("K", ctypes.c_int), ("groups", ctypes.c_int),
-                ("dy_gs", ctypes.c_longlong), ("x_gs", ctypes.c_longlong), ("dw_gs", ctypes.c_longlong)]
 
 
 class _BiasJob(ctypes.Structure):
@@ -89,9 +66,6 @@ class _DpPeers(ctypes.Structure):
     _fields_ = [("grad", ctypes.c_void_p * _DP_MAX_WORLD), ("param", ctypes.c_void_p * _DP_MAX_WORLD),
                 ("flags", ctypes.c_void_p * _DP_MAX_WORLD), ("grad_mc", ctypes.c_void_p),
                 ("param_mc", ctypes.c_void_p)]
-# the backward-data kernels accumulate the border sums of the dz they write in their epilogue
-# (AVA_B200_FUSED_TSUMS=0: a separate ava_b200_dz_border_sums pass per layer instead)
-_FUSED_TSUMS = os.environ.get("AVA_B200_FUSED_TSUMS", "1") != "0"
 # The dense layers' weight and bias gradients are off the backward pass's critical path (only the
 # data gradients feed the next layer): they are issued on a second stream that forks where their
 # inputs are complete and joins before a gradient bucket is declared final / before the optimizer
@@ -255,8 +229,8 @@ class VAE(nn.Module):
         backward-data kernels / also the decoder's forward kernels / all three conv kernel
         families (include/ava_b200.h, ava_b200_set_conv_precision modes 3 / 5 / 6 / 4; all hold
         rtol 1e-4, with decreasing margin).  'tf32': single-pass TF32, the opt-in reduced-precision mode (stated
-        tolerance 1e-2 forward).  'auto' (default): 'tf32x3' dense layers with the conv mode
-        named by _AUTO_CONV_MODE.
+        tolerance 1e-2 forward).  'auto' (default): 'tf32x3' dense layers and 'tf32x3e' conv
+        layers (mode 6, chosen by measurement: see _AUTO_CONV_MODE).
     """
 
     def __init__(self, save_dir='', lr=1e-3, z_dim=32, model_precision=10.0,
@@ -530,7 +504,7 @@ class VAE(nn.Module):
              K, act, groups, x_gs, w_gs, b_gs, y_gs, tc, ptr(ws), ws.numel(), _stream())
 
     def _linear_bwd(self, dy, lddy, ymask, x, ldx, wkey, bkey, dx, lddx, M, N, K, groups=1,
-                    dy_gs=0, x_gs=0, w_gs=0, b_gs=0, dx_gs=0, tc=0, bias_jobs=None, wgrad_jobs=None):
+                    dy_gs=0, x_gs=0, w_gs=0, b_gs=0, dx_gs=0, tc=0, bias_jobs=None):
         """dW, db into the flat gradient buffer; dx (if not None) = (dy*mask) W.  With `bias_jobs`
         the bias gradient is not computed here but queued for one batched ava_b200_bias_grads call
         per backward segment (_flush_bias; the groups of a grouped layer are adjacent column blocks
@@ -542,12 +516,6 @@ class VAE(nn.Module):
             assert groups == 1 or (dy_gs == N and b_gs == N)
             bias_jobs.append((ptr(dy), ptr(ymask), gb, lddy, M, N * groups))
             gb = None
-        if wgrad_jobs is not None:
-            # (small layer: its weight gradient joins one multi-job launch, _flush_wgrad)
-            assert gb is None and dx is None
-            wgrad_jobs.append((ptr(dy), ptr(ymask), ptr(x), self._g(wkey), lddy, ldx, M, N, K, groups,
-                               dy_gs, x_gs, w_gs))
-            return
         if _SIDE_STREAM and gb is None:
             side = self._side_fork()
             ws2 = self._ws_side(self._scratch_need)
@@ -560,42 +528,6 @@ class VAE(nn.Module):
         if dx is not None:
             call("ava_b200_linear_bwd_data", ptr(dy), lddy, ptr(ymask), self._p(wkey), ptr(dx), lddx,
                  M, N, K, groups, dy_gs, w_gs, dx_gs, 0, tc, ptr(ws), ws.numel(), s)
-
-    def _mlp_ok(self):
-        """The fused row-wise kernels of csrc/mlp.cu serve z_dim % 4 == 0, z_dim <= 64."""
-        return _FUSED_MLP and self.z_dim % 4 == 0 and 4 <= self.z_dim <= 64
-
-    def _mlp_params(self, bufs, stages, z=None, backward=False):
-        P = _MlpParams()
-        P.B, P.Z, P.stages = bufs.B, self.z_dim, stages
-        for f, key in (("w2", "fc2.weight"), ("b2", "fc2.bias"), ("w3", "fc31.weight"), ("b3", "fc31.bias"),
-                       ("w4", "fc41.weight"), ("b4", "fc41.bias"), ("w5", "fc5.weight"), ("b5", "fc5.bias"),
-                       ("w6", "fc6.weight"), ("b6", "fc6.bias"), ("w7", "fc7.weight"), ("b7", "fc7.bias")):
-            setattr(P, f, self._p(key))
-        for f in ("h1", "h2", "h3", "heads", "d", "t5", "t6", "t7"):
-            setattr(P, f, ptr(getattr(bufs, f)))
-        P.z = ptr(z if z is not None else bufs.z)
-        P.acc = bufs.acc.data_ptr()
-        if stages & 2 or backward:
-            P.eps_w, P.eps_d = ptr(bufs.eps_w), ptr(bufs.eps_d)
-        if backward:
-            for f in ("dt7", "dt6", "dt5", "gz", "gheads", "dh3", "dh2", "dh1"):
-                setattr(P, f, ptr(getattr(bufs, f)))
-        return P
-
-    def _mlp_fwd(self, bufs, stages, z=None):
-        """fc2 .. heads (1) | reparameterised sample + latent loss terms (2) | fc5 .. fc7 (4) as one
-        launch (csrc/mlp.cu)."""
-        call("ava_b200_mlp_fwd", ctypes.byref(self._mlp_params(bufs, stages, z)), _stream())
-
-    def _flush_wgrad(self, jobs):
-        """The queued small-layer weight gradients in one launch."""
-        if not jobs:
-            return
-        arr = (_WgradJob * len(jobs))()
-        for a, j in zip(arr, jobs):
-            (a.dy, a.ymask, a.x, a.dw, a.lddy, a.ldx, a.M, a.N, a.K, a.groups, a.dy_gs, a.x_gs, a.dw_gs) = j
-        call("ava_b200_linear_bwd_weight_multi", arr, len(jobs), _stream())
 
     def _flush_bias(self, jobs):
         """All queued bias gradients of a backward segment in two launches."""
@@ -620,9 +552,8 @@ class VAE(nn.Module):
              st + 8 * 64 * l, self._rm(l), self._rv(l), 1 if train else 0,
              (st + 8 * 64 * (l + 1)) if want_stats_out else None, _stream())
 
-    def _encode_native(self, x, bufs, train, tail=True):
-        """x [B,128,128] -> bufs.heads (mu | u | log d).  ava/models/vae.py:216-232.
-        tail=False stops after fc1 (the caller runs the small layers fused with what follows)."""
+    def _encode_native(self, x, bufs, train):
+        """x [B,128,128] -> bufs.heads (mu | u | log d).  ava/models/vae.py:216-232."""
         B, Z, s = bufs.B, self.z_dim, _stream()
         if train:
             call("ava_b200_channel_stats", ptr(x), B, 1, X_DIM, bufs.stats.data_ptr(), s)
@@ -632,11 +563,6 @@ class VAE(nn.Module):
             h = bufs.act[l]
         tc = self._tc
         self._linear(h, 8192, "fc1.weight", "fc1.bias", bufs.h1, 1024, B, 1024, 8192, 1, tc=tc)
-        if not tail:
-            return
-        if self._mlp_ok():
-            self._mlp_fwd(bufs, 1)
-            return
         self._linear(bufs.h1, 1024, "fc2.weight", "fc2.bias", bufs.h2, 256, B, 256, 1024, 1, tc=tc)
         # fc31|fc32|fc33 share their input: one [192,256] layer
         self._linear(bufs.h2, 256, "fc31.weight", "fc31.bias", bufs.h3, 192, B, 192, 256, 1)
@@ -644,17 +570,13 @@ class VAE(nn.Module):
         self._linear(bufs.h3, 192, "fc41.weight", "fc41.bias", bufs.heads, 3 * Z, B, Z, 64, 0,
                      groups=3, x_gs=64, w_gs=Z * 64, b_gs=Z, y_gs=Z)
 
-    def _decode_native(self, z, bufs, train, head=True):
-        """z [B,Z] -> bufs.act[13] = x_rec [B,1,128,128].  ava/models/vae.py:258-270.
-        head=False: fc5..fc7 have already run (fused with the encoder tail)."""
+    def _decode_native(self, z, bufs, train):
+        """z [B,Z] -> bufs.act[13] = x_rec [B,1,128,128].  ava/models/vae.py:258-270."""
         B, Z, s = bufs.B, self.z_dim, _stream()
         tc = self._tc
-        if head and self._mlp_ok():
-            self._mlp_fwd(bufs, 4, z=z)
-        elif head:
-            self._linear(z, Z, "fc5.weight", "fc5.bias", bufs.t5, 64, B, 64, Z, 1)
-            self._linear(bufs.t5, 64, "fc6.weight", "fc6.bias", bufs.t6, 256, B, 256, 64, 1)
-            self._linear(bufs.t6, 256, "fc7.weight", "fc7.bias", bufs.t7, 1024, B, 1024, 256, 1, tc=tc)
+        self._linear(z, Z, "fc5.weight", "fc5.bias", bufs.t5, 64, B, 64, Z, 1)
+        self._linear(bufs.t5, 64, "fc6.weight", "fc6.bias", bufs.t6, 256, B, 256, 64, 1)
+        self._linear(bufs.t6, 256, "fc7.weight", "fc7.bias", bufs.t7, 1024, B, 1024, 256, 1, tc=tc)
         self._linear(bufs.t7, 1024, "fc8.weight", "fc8.bias", bufs.t8, 8192, B, 8192, 1024, 1, tc=tc)
         if train:
             call("ava_b200_channel_stats", ptr(bufs.t8), B, 32, 256,
@@ -692,25 +614,20 @@ class VAE(nn.Module):
         self._scratch_need = self._scratch_need_for(B)
         s = _stream()
         bufs.accum.zero_()
-        fused = self._mlp_ok()
-        self._encode_native(x, bufs, train, tail=not fused)
+        self._encode_native(x, bufs, train)
         ew, ed = noise if noise is not None else self._draw_noise(B)
         ew = ew.to(torch.float32).contiguous()
         ed = ed.to(torch.float32).contiguous()
         bufs.eps_w, bufs.eps_d = ew, ed
-        if fused:
-            # fc2 .. heads, the reparameterised sample and fc5 .. fc7: one launch
-            self._mlp_fwd(bufs, 7)
-        else:
-            call("ava_b200_latent_fwd", ptr(bufs.heads), ptr(ew), ptr(ed), B, self.z_dim, ptr(bufs.z),
-                 ptr(bufs.d), bufs.acc.data_ptr(), s)
-        self._decode_native(bufs.z, bufs, train, head=not fused)
+        call("ava_b200_latent_fwd", ptr(bufs.heads), ptr(ew), ptr(ed), B, self.z_dim, ptr(bufs.z),
+             ptr(bufs.d), bufs.acc.data_ptr(), s)
+        self._decode_native(bufs.z, bufs, train)
         g = None
         if want_grad_seed:
             bufs.alloc_backward(self.z_dim)
             g = bufs.g[0]
         # (the gradient written here is convt7's dz: its nine border sums are accumulated on the way)
-        ts13 = (bufs.tsums.data_ptr() + 8 * 288 * 13) if (g is not None and _FUSED_TSUMS) else None
+        ts13 = (bufs.tsums.data_ptr() + 8 * 288 * 13) if g is not None else None
         call("ava_b200_recon", ptr(x), ptr(bufs.act[13]), B * X_DIM, float(self.model_precision),
              ptr(g), bufs.acc.data_ptr(), ts13, X_SHAPE[0], X_SHAPE[1], s)
         call("ava_b200_elbo_finalize", bufs.acc.data_ptr(), self.z_dim, X_DIM,
@@ -728,37 +645,30 @@ class VAE(nn.Module):
             cache[B] = self._scratch_bytes(B)
         return cache[B]
 
-    def _conv_bwd(self, l, bufs, dz, x, dz_prev, have_tsums=False):
-        """Backward of fused layer l given dz = the gradient w.r.t. its pre-activation output.
-        (1) the nine border sums of dz; (2) weight / bias gradients into the flat gradient
-        buffer AND this layer's BatchNorm-backward reductions dstats[l] (both from the same
-        centred raw product, see include/ava_b200.h); (3) the data gradient, pushed through this
-        layer's BatchNorm backward and the previous layer's ReLU in the kernel's epilogue, lands
-        in dz_prev as the previous layer's dz -- the gradient w.r.t. the BatchNorm output never
-        goes to memory.  `have_tsums`: the kernel that wrote dz already accumulated its border
-        sums (step 1 is then skipped); returns whether that holds for dz_prev."""
+    def _conv_bwd(self, l, bufs, dz, x, dz_prev):
+        """Backward of fused layer l given dz = the gradient w.r.t. its pre-activation output,
+        whose nine border sums the kernel that wrote dz has already accumulated into tsums[l].
+        (1) weight / bias gradients into the flat gradient buffer AND this layer's
+        BatchNorm-backward reductions dstats[l] (both from the same centred raw product, see
+        include/ava_b200.h); (2) the data gradient, pushed through this layer's BatchNorm backward
+        and the previous layer's ReLU in the kernel's epilogue, lands in dz_prev as the previous
+        layer's dz -- the gradient w.r.t. the BatchNorm output never goes to memory."""
         B = bufs.B
-        name, _, co, stride, _ = _LAYERS[l]
+        name = _LAYERS[l][0]
         st, ds, ts = bufs.stats.data_ptr(), bufs.dstats.data_ptr(), bufs.tsums.data_ptr()
         s = _stream()
-        ho = _out_hw(l)
-        mode = 1 if (l >= 7 and stride == 2) else 0
         gamma, beta = self._p("bn%d.weight" % (l + 1)), self._p("bn%d.bias" % (l + 1))
-        if not have_tsums:
-            call("ava_b200_dz_border_sums", ptr(dz), B, co, ho, ho, mode, ts + 8 * 288 * l, s)
         ws = self._ws(self._scratch_need)
         _set_conv_precision(self._tc_conv)
         call("ava_b200_bnconv_bwd_weight", l, B, ptr(dz), ptr(x), self._p(name + ".weight"), gamma, beta,
              st + 8 * 64 * l, ts + 8 * 288 * l, self._g(name + ".weight"), self._g(name + ".bias"),
              ds + 8 * 64 * l, ptr(ws), s)
         if dz_prev is not None:
-            # the epilogue also accumulates the border sums of the dz it writes (layer l-1's)
-            fuse = _FUSED_TSUMS and l >= 1 and l != 7
+            # the epilogue also accumulates the border sums of the dz it writes (layer l-1's; layer
+            # 7 writes fc8's output gradient, which has none)
             call("ava_b200_bnconv_bwd_data", l, B, ptr(dz), self._p(name + ".weight"), ptr(x), gamma,
                  st + 8 * 64 * l, ds + 8 * 64 * l, 1, ptr(dz_prev),
-                 (ts + 8 * 288 * (l - 1)) if fuse else None, s)
-            return fuse
-        return False
+                 (ts + 8 * 288 * (l - 1)) if l != 7 else None, s)
 
     def _bwd_decoder(self, bufs):
         """Backward segment 1: decoder conv stack (layers 13..7) and fc8..fc5.  Afterwards the
@@ -768,29 +678,20 @@ class VAE(nn.Module):
         g_cur, g_nxt = bufs.g[0], bufs.g[1]      # g[0] holds dL/dx_rec = convt7's dz (recon kernel)
         # layer 7 writes the gradient w.r.t. fc8's pre-activation output (bn8 backward + fc8's
         # ReLU) straight into dt8
-        have = _FUSED_TSUMS      # (accumulated by the recon kernel)
         for l in range(13, 6, -1):
             xin = bufs.act[l - 1] if l > 7 else bufs.t8
             out = g_nxt if l > 7 else bufs.dt8
-            have = self._conv_bwd(l, bufs, g_cur, xin, out, have)
+            self._conv_bwd(l, bufs, g_cur, xin, out)
             g_cur, g_nxt = g_nxt, g_cur
         jobs = []
         self._linear_bwd(bufs.dt8, 8192, None, bufs.t7, 1024, "fc8.weight", "fc8.bias", bufs.dt7, 1024,
                          B, 8192, 1024, tc=self._tc, bias_jobs=jobs)
-        fused = self._mlp_ok()
-        if fused:
-            # every data gradient between fc8 and fc1 (dt6, dt5, gz, the latent gradient gheads,
-            # dh3, dh2, dh1) in one launch; the per-layer calls below only form weight gradients
-            call("ava_b200_mlp_bwd", ctypes.byref(self._mlp_params(bufs, 7, backward=True)), _stream())
-        wj = [] if fused else None
-        self._linear_bwd(bufs.dt7, 1024, bufs.t7, bufs.t6, 256, "fc7.weight", "fc7.bias",
-                         None if fused else bufs.dt6, 256, B, 1024, 256, tc=self._tc, bias_jobs=jobs,
-                         wgrad_jobs=wj)
-        self._linear_bwd(bufs.dt6, 256, bufs.t6, bufs.t5, 64, "fc6.weight", "fc6.bias",
-                         None if fused else bufs.dt5, 64, B, 256, 64, bias_jobs=jobs, wgrad_jobs=wj)
-        self._linear_bwd(bufs.dt5, 64, bufs.t5, bufs.z, Z, "fc5.weight", "fc5.bias",
-                         None if fused else bufs.gz, Z, B, 64, Z, bias_jobs=jobs, wgrad_jobs=wj)
-        self._flush_wgrad(wj)
+        self._linear_bwd(bufs.dt7, 1024, bufs.t7, bufs.t6, 256, "fc7.weight", "fc7.bias", bufs.dt6, 256,
+                         B, 1024, 256, tc=self._tc, bias_jobs=jobs)
+        self._linear_bwd(bufs.dt6, 256, bufs.t6, bufs.t5, 64, "fc6.weight", "fc6.bias", bufs.dt5, 64,
+                         B, 256, 64, bias_jobs=jobs)
+        self._linear_bwd(bufs.dt5, 64, bufs.t5, bufs.z, Z, "fc5.weight", "fc5.bias", bufs.gz, Z,
+                         B, 64, Z, bias_jobs=jobs)
         self._flush_bias(jobs)
 
     def _bwd_dense_encoder(self, bufs):
@@ -798,21 +699,15 @@ class VAE(nn.Module):
         encoder's dense layers.  Afterwards the gradients of fc1..fc43 are final (fc1.weight is
         half of all parameters)."""
         B, Z, s = bufs.B, self.z_dim, _stream()
-        fused = self._mlp_ok()       # (then gheads, dh3, dh2, dh1 came from ava_b200_mlp_bwd)
-        if not fused:
-            call("ava_b200_latent_bwd", ptr(bufs.heads), ptr(bufs.eps_w), ptr(bufs.eps_d), ptr(bufs.z),
-                 ptr(bufs.gz), B, Z, ptr(bufs.gheads), s)
+        call("ava_b200_latent_bwd", ptr(bufs.heads), ptr(bufs.eps_w), ptr(bufs.eps_d), ptr(bufs.z),
+             ptr(bufs.gz), B, Z, ptr(bufs.gheads), s)
         jobs = []
-        wj = [] if fused else None
-        self._linear_bwd(bufs.gheads, 3 * Z, None, bufs.h3, 192, "fc41.weight", "fc41.bias",
-                         None if fused else bufs.dh3, 192, B, Z, 64, groups=3, dy_gs=Z, x_gs=64,
-                         w_gs=Z * 64, b_gs=Z, dx_gs=64, bias_jobs=jobs, wgrad_jobs=wj)
-        self._linear_bwd(bufs.dh3, 192, bufs.h3, bufs.h2, 256, "fc31.weight", "fc31.bias",
-                         None if fused else bufs.dh2, 256, B, 192, 256, bias_jobs=jobs, wgrad_jobs=wj)
-        self._linear_bwd(bufs.dh2, 256, bufs.h2, bufs.h1, 1024, "fc2.weight", "fc2.bias",
-                         None if fused else bufs.dh1, 1024, B, 256, 1024, tc=self._tc, bias_jobs=jobs,
-                         wgrad_jobs=wj)
-        self._flush_wgrad(wj)
+        self._linear_bwd(bufs.gheads, 3 * Z, None, bufs.h3, 192, "fc41.weight", "fc41.bias", bufs.dh3, 192,
+                         B, Z, 64, groups=3, dy_gs=Z, x_gs=64, w_gs=Z * 64, b_gs=Z, dx_gs=64, bias_jobs=jobs)
+        self._linear_bwd(bufs.dh3, 192, bufs.h3, bufs.h2, 256, "fc31.weight", "fc31.bias", bufs.dh2, 256,
+                         B, 192, 256, bias_jobs=jobs)
+        self._linear_bwd(bufs.dh2, 256, bufs.h2, bufs.h1, 1024, "fc2.weight", "fc2.bias", bufs.dh1, 1024,
+                         B, 256, 1024, tc=self._tc, bias_jobs=jobs)
         self._linear_bwd(bufs.dh1, 1024, bufs.h1, bufs.act[6], 8192, "fc1.weight", "fc1.bias",
                          bufs.da6, 8192, B, 1024, 8192, tc=self._tc, bias_jobs=jobs)
         self._flush_bias(jobs)
@@ -822,16 +717,15 @@ class VAE(nn.Module):
         parameter gradients of all 14 layers."""
         B, s = bufs.B, _stream()
         # conv7's ReLU on the gradient arriving from fc1 (no BatchNorm at this seam)
-        ts6 = (bufs.tsums.data_ptr() + 8 * 288 * 6) if _FUSED_TSUMS else None
+        # (and the nine border sums of the dz it writes, conv7's)
         call("ava_b200_bn_relu_bwd_apply", ptr(bufs.da6), ptr(bufs.act[6]), None, None, None, B, 32, 256,
-             1, ptr(bufs.da6), ts6, 16, s)
+             1, ptr(bufs.da6), bufs.tsums.data_ptr() + 8 * 288 * 6, 16, s)
         g_cur = bufs.da6
         free = [bufs.g[0], bufs.g[1]]
-        have = _FUSED_TSUMS
         for l in range(6, -1, -1):          # (layer 0 needs no data gradient)
             xin = bufs.act[l - 1] if l > 0 else bufs.x
             out = free[0] if l > 0 else None
-            have = self._conv_bwd(l, bufs, g_cur, xin, out, have)
+            self._conv_bwd(l, bufs, g_cur, xin, out)
             g_cur, free = out, [free[1], free[0]]
         st, ds = bufs.stats.data_ptr(), bufs.dstats.data_ptr()
         counts = [B * _LAYERS[l][4] ** 2 for l in range(14)]
@@ -1100,8 +994,6 @@ class VAE(nn.Module):
     def _graph_wanted(self, B):
         if self._flat_p.device.type != "cuda":
             return False
-        if self._dp_world > 1 and os.environ.get("AVA_B200_DP_GRAPHS", "1") == "0":
-            return False    # (opt-out switch for the segmented data-parallel graphs)
         if self.cuda_graphs == 'auto':
             return True     # measured: 1.41 vs 1.68 ms at batch 64, 8.13 vs 8.46 ms at batch 1024
         return bool(self.cuda_graphs)

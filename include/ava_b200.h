@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AVA_B200_ABI_VERSION 3
+#define AVA_B200_ABI_VERSION 4
 #define AVA_NUM_BN_LAYERS 14
 #define AVA_STATS_STRIDE 64 /* doubles per layer in a stats block: [0..31]=sum, [32..63]=sum of squares */
 
@@ -99,10 +99,14 @@ int ava_b200_get_conv_precision(void);
 /* Backward of layer `layer`.  `dz` is the gradient w.r.t. this layer's PRE-activation conv output
  * (for layer 13 -- no ReLU, nothing after it -- the loss gradient itself).  Order per layer:
  *
- *   1. ava_b200_dz_border_sums(dz)  -> tsums: nine per-channel sums of dz (total / first and last
- *      row and column / corners; for the stride-2 conv-transpose layers 8, 10, 12 the four
- *      row-parity x column-parity classes and the last row / column), from which the sum of dz over
- *      the pixels whose tap-k partner lies inside the image follows for each of the 9 taps.
+ *   1. tsums: nine per-channel sums of dz (total / first and last row and column / corners; for the
+ *      stride-2 conv-transpose layers 8, 10, 12 the four row-parity x column-parity classes and the
+ *      last row / column), from which the sum of dz over the pixels whose tap-k partner lies inside
+ *      the image follows for each of the 9 taps.  The kernel that writes dz accumulates them in its
+ *      epilogue (ava_b200_recon for layer 13, ava_b200_bn_relu_bwd_apply for layer 6,
+ *      ava_b200_bnconv_bwd_data of layer+1 for the others).  ava_b200_dz_border_sums is the
+ *      stand-alone pass: it defines the nine sums and is the reference the tests compare the
+ *      epilogue-accumulated sums against.
  *   2. ava_b200_bnconv_bwd_weight   -> dw, db (OVERWRITTEN) and this layer's two BatchNorm-backward
  *      reductions dstats = (sum g, sum g*(x-mean)), ACCUMULATED (zero them first).  g is the gradient
  *      w.r.t. the BatchNorm output; it is never materialised: both reductions are linear in the
@@ -129,7 +133,7 @@ long long ava_b200_bnconv_bwd_weight_ws(int layer, int B);
 
 /* gamma == NULL: no BatchNorm backward (dz_prev = [x > 0] * g).
  * tsums_prev (optional): the nine border sums of dz_prev -- layer-1's tsums block -- are accumulated
- * in the epilogue, which saves step 1 (a full read of dz_prev) for layer-1. */
+ * in the epilogue (step 1 for layer-1, without a second read of dz_prev). */
 int ava_b200_bnconv_bwd_data(int layer, int B, const float* dz, const float* w, const float* x,
                              const float* gamma, const double* stats_in, const double* dstats, int relu_mask,
                              float* dz_prev, double* tsums_prev, void* stream);
@@ -173,20 +177,6 @@ int ava_b200_linear_bwd_weight(const float* dy, int lddy, const float* ymask, co
                                long long dw_gs, long long db_gs, int precision, void* ws, long long ws_bytes,
                                void* stream);
 
-/* The weight gradients of up to AVA_MAX_WGRAD_JOBS small Linear layers in ONE launch (fp32 FMA, no
- * split-K, no workspace): job j is ava_b200_linear_bwd_weight's dW for (dy, ymask, x) of shape
- * M x N / M x K with `groups` strided groups (ymask may be NULL).  h_jobs is a HOST array. */
-#define AVA_MAX_WGRAD_JOBS 8
-typedef struct {
-  const float* dy;
-  const float* ymask;
-  const float* x;
-  float* dw;
-  int lddy, ldx, M, N, K, groups;
-  long long dy_gs, x_gs, dw_gs;
-} ava_b200_wgrad_job;
-int ava_b200_linear_bwd_weight_multi(const ava_b200_wgrad_job* h_jobs, int njobs, void* stream);
-
 /* Bias gradients of up to AVA_MAX_BIAS_JOBS Linear layers in two launches: job j computes
  * db[n] = sum_m (mask > 0 ? dy : 0)[m, n] over dy [M, N] (row stride ld; mask may be NULL) --
  * what ava_b200_linear_bwd_weight does per layer when given db; the step passes db = NULL there
@@ -228,28 +218,6 @@ int ava_b200_recon(const float* x, const float* x_rec, long long n, float precis
  * accumulator replacing loss.item() per step, ava/models/vae.py:351). */
 int ava_b200_elbo_finalize(const double* acc, int Z, int xdim, float precision, float* loss, double* loss_sum,
                            void* stream);
-
-/* ------------------------------------------------------- fused small dense layers
- * The chain between the two 8192x1024 layers as ONE row-wise kernel per direction (csrc/mlp.cu):
- *   forward  (ava/models/vae.py:226-232, 298-316, 258-260): stages bit 0: h1 -fc2-> h2 -fc31|32|33->
- *            h3 -fc41|42|43-> heads = (mu | u | log d); bit 1: z = mu + u eps_w + sqrt(d) eps_d,
- *            acc[0] += sum z^2, acc[2] += entropy (as ava_b200_latent_fwd); bit 2: z -fc5-> t5 -fc6->
- *            t6 -fc7-> t7.  Every intermediate is also written out (saved for the backward pass).
- *   backward (autograd of the same): dt7 -> dt6 -> dt5 -> gz -> gheads (analytic latent gradient, as
- *            ava_b200_latent_bwd) -> dh3 -> dh2 -> dh1; gradients w.r.t. post-activation outputs,
- *            stored unmasked (ava_b200_linear_bwd_weight / ava_b200_bias_grads apply the ReLU masks).
- * w3/b3 and w4/b4 are the stacked fc31|fc32|fc33 and fc41|fc42|fc43 parameters.  z_dim: a multiple
- * of 4, <= 64.  h_params is a HOST struct of DEVICE pointers.  fp32 FMA arithmetic. */
-typedef struct {
-  int B, Z, stages;
-  const float *w2, *b2, *w3, *b3, *w4, *b4, *w5, *b5, *w6, *b6, *w7, *b7;
-  const float *eps_w, *eps_d;
-  float *h1, *h2, *h3, *heads, *z, *d, *t5, *t6, *t7;
-  float *dt7, *dt6, *dt5, *gz, *gheads, *dh3, *dh2, *dh1;
-  double* acc;
-} ava_b200_mlp_params;
-int ava_b200_mlp_fwd(const ava_b200_mlp_params* h_params, void* stream);
-int ava_b200_mlp_bwd(const ava_b200_mlp_params* h_params, void* stream);
 
 /* ----------------------------------------------------------------------- Adam
  * torch.optim.Adam (defaults: no weight decay, no amsgrad), one launch over the flat

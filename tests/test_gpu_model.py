@@ -120,15 +120,6 @@ def test_forward_backward_matches_reference_golden(vae_mod, name, precision):
             assert rel_err(sd[kk].cpu().numpy(), g[k]) <= FWD_TOL, kk
 
 
-@pytest.mark.parametrize("name", ["vae_train_b7", "vae_train_b64"])
-def test_fused_mlp_path_matches_reference_golden(vae_mod, name, monkeypatch):
-    """The opt-in fused small-layer path (AVA_B200_FUSED_MLP=1: csrc/mlp.cu forward / backward chains
-    + ava_b200_linear_bwd_weight_multi) through the same golden / float64-oracle bars as the
-    default per-layer path."""
-    monkeypatch.setattr(vae_mod, "_FUSED_MLP", True)
-    test_forward_backward_matches_reference_golden(vae_mod, name, "tf32x3b")
-
-
 @pytest.mark.parametrize("graphs", [False, True])
 def test_forked_stream_changes_scheduling_only(vae_mod, monkeypatch, graphs):
     """The dense layers' weight / bias gradients run on a second stream beside the conv backward
