@@ -167,7 +167,8 @@ int ava_b200_bn_relu_bwd_apply(const float* g, const float* a, const float* gamm
 int ava_b200_linear_fwd(const float* x, int ldx, const float* w, const float* b, float* y, int ldy, int M, int N,
                         int K, int act, int groups, long long x_gs, long long w_gs, long long b_gs,
                         long long y_gs, int precision, void* ws, long long ws_bytes, void* stream);
-/* dX[M,K] = (dY (.) mask) . W ; mask = [Ymask>0] if Ymask != NULL (ReLU backward). */
+/* dX[M,K] = (dY (.) mask) . W ; mask = [Ymask>0] if Ymask != NULL (ReLU backward).  Overwrites:
+ * `accumulate` must be 0 -- any other value returns an error and leaves dx unchanged. */
 int ava_b200_linear_bwd_data(const float* dy, int lddy, const float* ymask, const float* w, float* dx, int lddx,
                              int M, int N, int K, int groups, long long dy_gs, long long w_gs, long long dx_gs,
                              int accumulate, int precision, void* ws, long long ws_bytes, void* stream);
