@@ -40,6 +40,7 @@ SIGNATURES = {
     "ava_b200_adam_step": (P, P, P, P, LL, P, D, D, D, D, F, P),
     "ava_b200_adam_step_dev": (P, P, P, P, LL, P, P, F, P),
     "ava_b200_adam_step_dp": (P, I, I, P, P, LL, P, P, F, P, P),
+    "ava_b200_bn_stats_exchange": (P, I, I, P, I, LL, P, I, I, P, F, P, P),
     "ava_b200_get_spec_batch": (P, I, P, P, I, I, I, I, P, D, P, P, I, P, P, I, I, D, D, P, P, P),
     "ava_b200_quantile_normalize": (P, P, I, I, D, P),
     "ava_b200_window_time_tables": (P, P, P, I, P, P, I, I, P, P, P),

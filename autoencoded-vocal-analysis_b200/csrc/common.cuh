@@ -80,6 +80,45 @@ __device__ __forceinline__ void adam_update(const AdamCoef& k, float gg, float& 
   p = __fmaf_rn(-k.step_size, __fdiv_rn(m, denom), p);
 }
 
+// Cross-GPU flag handshake of the data-parallel kernels (dp.cu, bnsync.cu): flags hold monotonically
+// increasing sequence numbers; a waiter gives up after kDpTimeoutNs and records it in *status.
+constexpr unsigned long long kDpTimeoutNs = 20ull * 1000ull * 1000ull * 1000ull;
+
+__device__ __forceinline__ unsigned long long dp_now_ns() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+__device__ __forceinline__ void dp_signal(unsigned int* flag, unsigned int seq) {
+  asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(flag), "r"(seq) : "memory");
+}
+__device__ __forceinline__ void dp_wait(const unsigned int* flag, unsigned int seq, unsigned int* status) {
+  const unsigned long long t0 = dp_now_ns();
+  for (;;) {
+    unsigned int v;
+    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
+    if ((int)(v - seq) >= 0) return;
+    if (dp_now_ns() - t0 > kDpTimeoutNs) {
+      atomicExch(status, 1u);
+      return;
+    }
+    __nanosleep(64);
+  }
+}
+
+// BatchNorm running-buffer update of channel c from the sums of a stats block over n values (torch's
+// momentum form, unbiased variance): bn_update_running_kernel (elbo.cu) and the synchronised-BatchNorm
+// exchange (bnsync.cu) share it so that both round alike.
+__device__ __forceinline__ void bn_running_update(const double* st, int c, double n, float* rm, float* rv,
+                                                  float momentum) {
+  double mean = st[c] / n;
+  double var = st[32 + c] / n - mean * mean;
+  if (var < 0) var = 0;
+  double unb = (n > 1) ? var * n / (n - 1) : var;
+  rm[c] = (1.f - momentum) * rm[c] + momentum * (float)mean;
+  rv[c] = (1.f - momentum) * rv[c] + momentum * (float)unb;
+}
+
 // BatchNorm coefficients for one channel from accumulated sums (train) or running
 // buffers (eval):  bn(x) = x*scale + shift.
 struct BnCoef {

@@ -31,8 +31,6 @@
 
 namespace ava {
 
-constexpr unsigned long long kDpTimeoutNs = 20ull * 1000ull * 1000ull * 1000ull;
-
 struct DpPeers {
   const float* grad[AVA_DP_MAX_WORLD];
   float* param[AVA_DP_MAX_WORLD];
@@ -41,27 +39,6 @@ struct DpPeers {
   float* param_mc;
 };
 
-__device__ __forceinline__ unsigned long long dp_now_ns() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-__device__ __forceinline__ void dp_signal(unsigned int* flag, unsigned int seq) {
-  asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(flag), "r"(seq) : "memory");
-}
-__device__ __forceinline__ void dp_wait(const unsigned int* flag, unsigned int seq, unsigned int* status) {
-  const unsigned long long t0 = dp_now_ns();
-  for (;;) {
-    unsigned int v;
-    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(flag) : "memory");
-    if ((int)(v - seq) >= 0) return;
-    if (dp_now_ns() - t0 > kDpTimeoutNs) {
-      atomicExch(status, 1u);
-      return;
-    }
-    __nanosleep(64);
-  }
-}
 __device__ __forceinline__ float4 dp_ld_peer(const float* p) {
   float4 v;
   // (strong system-scope accesses throughout: weak ones measured no faster -- 156 vs 155 us at 2

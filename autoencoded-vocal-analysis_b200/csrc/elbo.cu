@@ -82,16 +82,8 @@ __global__ void bn_update_running_kernel(const double* stats, BnTable T, float* 
   if (T.counts[l] == 0) return;  // layer not run this pass (e.g. encoder-only get_latent)
   if (c == 0) nbt[l] += 1;
   if (c >= T.channels[l]) return;
-  const double n = (double)T.counts[l];
-  const double* st = stats + (size_t)l * kStatsStride;
-  double mean = st[c] / n;
-  double var = st[32 + c] / n - mean * mean;
-  if (var < 0) var = 0;
-  double unb = (n > 1) ? var * n / (n - 1) : var;
-  float* rm = running + T.off_a[l];
-  float* rv = running + T.off_b[l];
-  rm[c] = (1.f - momentum) * rm[c] + momentum * (float)mean;
-  rv[c] = (1.f - momentum) * rv[c] + momentum * (float)unb;
+  bn_running_update(stats + (size_t)l * kStatsStride, c, (double)T.counts[l], running + T.off_a[l],
+                    running + T.off_b[l], momentum);
 }
 
 __global__ void bn_param_grads_kernel(const double* stats, const double* dstats, BnTable T, float* grads) {

@@ -66,6 +66,13 @@ class _DpPeers(ctypes.Structure):
     _fields_ = [("grad", ctypes.c_void_p * _DP_MAX_WORLD), ("param", ctypes.c_void_p * _DP_MAX_WORLD),
                 ("flags", ctypes.c_void_p * _DP_MAX_WORLD), ("grad_mc", ctypes.c_void_p),
                 ("param_mc", ctypes.c_void_p)]
+
+
+class _BnSyncPeers(ctypes.Structure):
+    """ava_b200_bn_sync_peers (include/ava_b200.h): per-rank slot and flag pointers, symmetric memory."""
+    _fields_ = [("slots", ctypes.c_void_p * _DP_MAX_WORLD), ("flags", ctypes.c_void_p * _DP_MAX_WORLD)]
+_BN_SYNC_SLOT = 65         # AVA_BN_SYNC_SLOT, include/ava_b200.h
+
 # The dense layers' weight and bias gradients are off the backward pass's critical path (only the
 # data gradients feed the next layer): they are issued on a second stream that forks where their
 # inputs are complete and joins before a gradient bucket is declared final / before the optimizer
@@ -269,6 +276,8 @@ class VAE(nn.Module):
         self._graphs = {}
         self._dp_group = None
         self._dp_world = 1
+        self._bn_sync = None       # synchronised BatchNorm state (enable_data_parallel(sync_bn=True))
+        self._bn_sync_on = False   # set by train_step only: the exchanges run inside a training step
         self.to(self.device)
 
     # ------------------------------------------------------------------ network
@@ -559,6 +568,8 @@ class VAE(nn.Module):
             call("ava_b200_channel_stats", ptr(x), B, 1, X_DIM, bufs.stats.data_ptr(), s)
         h = x
         for l in range(7):
+            if train and self._bn_sync_on:
+                self._bn_exchange(l, B, bufs.stats, forward=True)
             self._conv_fwd(l, B, h, bufs.act[l], bufs, train, train and l < 6)
             h = bufs.act[l]
         tc = self._tc
@@ -583,6 +594,8 @@ class VAE(nn.Module):
                  bufs.stats.data_ptr() + 8 * 64 * 7, s)
         h = bufs.t8
         for l in range(7, 14):
+            if train and self._bn_sync_on:
+                self._bn_exchange(l, B, bufs.stats, forward=True)
             self._conv_fwd(l, B, h, bufs.act[l], bufs, train, train and l < 13)
             h = bufs.act[l]
 
@@ -632,7 +645,7 @@ class VAE(nn.Module):
              ptr(g), bufs.acc.data_ptr(), ts13, X_SHAPE[0], X_SHAPE[1], s)
         call("ava_b200_elbo_finalize", bufs.acc.data_ptr(), self.z_dim, X_DIM,
              float(self.model_precision), ptr(bufs.loss), ptr(self._loss_sum), s)
-        if train:
+        if train and not self._bn_sync_on:      # (synchronised BatchNorm: done by the exchanges)
             self._update_running(B, 0, 14)
         bufs.x = x
         return bufs
@@ -664,6 +677,8 @@ class VAE(nn.Module):
              st + 8 * 64 * l, ts + 8 * 288 * l, self._g(name + ".weight"), self._g(name + ".bias"),
              ds + 8 * 64 * l, ptr(ws), s)
         if dz_prev is not None:
+            if self._bn_sync_on:
+                self._bn_exchange(l, B, bufs.dstats, forward=False)
             # the epilogue also accumulates the border sums of the dz it writes (layer l-1's; layer
             # 7 writes fc8's output gradient, which has none)
             call("ava_b200_bnconv_bwd_data", l, B, ptr(dz), self._p(name + ".weight"), ptr(x), gamma,
@@ -839,7 +854,7 @@ class VAE(nn.Module):
         return self.forward(x, noise=noise)
 
     # ------------------------------------------------------------ data parallel
-    def enable_data_parallel(self, process_group=None, fused=None):
+    def enable_data_parallel(self, process_group=None, fused=None, sync_bn=False):
         """Shard batches over the ranks of `process_group` (default: WORLD), one process
         per GPU.  Semantics (SURVEY.md section 5): the loss is a batch SUM, so rank
         gradients are SUMMED (not averaged) -- the update equals the reference's at the
@@ -853,9 +868,29 @@ class VAE(nn.Module):
         ONE kernel per rank over NVLink peer memory (csrc/dp.cu: each rank sums its 1/world
         slice of everybody's gradient, applies Adam to that slice, stores the new parameters
         into every rank's buffer); gradients, parameters and flags then live in symmetric
-        memory.  Otherwise: bucketed NCCL all-reduces overlapped with the backward pass."""
+        memory.  Otherwise: bucketed NCCL all-reduces overlapped with the backward pass.
+
+        `sync_bn=True`: synchronised BatchNorm.  Every BatchNorm layer of a training step
+        (``train_step``, and so ``train_epoch`` / ``train_loop``) normalises with the statistics of
+        the GLOBAL batch -- the concatenation of the ranks' shards, which is what the reference's
+        single process sees -- so loss, summed gradients, update and running buffers are the
+        reference's at the global batch (up to rounding), for any split of the batch over the ranks,
+        empty shards included.  Each step exchanges 14 forward and 13 backward statistics blocks
+        over NVLink peer memory (csrc/bnsync.cu); the running buffers are updated from the global
+        statistics, identically on every rank, and are not re-averaged at epoch ends.  Works with
+        both optimizer paths.  Needs CUDA ranks of one NCCL group with at most 8 ranks and symmetric
+        memory; otherwise this raises.  ``encode``, ``decode``, ``forward``, ``test_epoch`` and
+        ``get_latent`` keep per-rank statistics (they are not collectives: ranks need not call them
+        in lockstep)."""
         import torch.distributed as dist
-        self._dp_group = process_group if process_group is not None else dist.group.WORLD
+        group = process_group if process_group is not None else dist.group.WORLD
+        if sync_bn and not (self._flat_p.is_cuda and dist.get_backend(group) == "nccl"
+                            and dist.get_world_size(group) <= _DP_MAX_WORLD):
+            raise RuntimeError("ava_b200: synchronised BatchNorm needs CUDA ranks of one NCCL group with at "
+                               "most %d ranks (got backend %r, %d ranks, model on %s)"
+                               % (_DP_MAX_WORLD, dist.get_backend(group), dist.get_world_size(group),
+                                  self._flat_p.device))
+        self._dp_group = group
         self._dp_world = dist.get_world_size(self._dp_group)
         self._dp_rank = dist.get_rank(self._dp_group)
         for t in (self._flat_p, self._flat_run, self._nbt, self._flat_m, self._flat_v):
@@ -877,7 +912,57 @@ class VAE(nn.Module):
             elif fused:
                 raise RuntimeError("ava_b200: fused data parallelism needs CUDA ranks of one NCCL group "
                                    "with at most %d ranks" % _DP_MAX_WORLD)
+        self._bn_sync = None
+        if sync_bn and self._dp_world > 1:
+            try:
+                self._enable_sync_bn()
+            except Exception as e:
+                raise RuntimeError("ava_b200: synchronised BatchNorm could not set up its symmetric-memory "
+                                   "exchange buffer (%s: %s)" % (type(e).__name__, e)) from e
         return self
+
+    def _enable_sync_bn(self):
+        """Each rank's two exchange slots and its flag in one small symmetric-memory allocation of
+        its own (independent of the fused optimizer's); the table of peer pointers for
+        csrc/bnsync.cu."""
+        import torch.distributed as dist
+        import torch.distributed._symmetric_memory as symm
+        dev, W = self._flat_p.device, self._dp_world
+        buf = symm.empty(2 * _BN_SYNC_SLOT + 1, dtype=torch.float64, device=dev)   # slots | flag
+        buf.zero_()
+        hdl = symm.rendezvous(buf, self._dp_group)
+        ptrs = [int(a) for a in hdl.buffer_ptrs]
+        assert len(ptrs) == W and ptrs[self._dp_rank] == buf.data_ptr()
+        peers = _BnSyncPeers()
+        for r in range(W):
+            peers.slots[r] = ptrs[r]
+            peers.flags[r] = ptrs[r] + 8 * 2 * _BN_SYNC_SLOT
+        local = torch.zeros(2, dtype=torch.int32, device=dev)
+        zeros = torch.zeros(2 * 14 * 64, dtype=torch.float64, device=dev)   # an empty shard's stats | dstats
+        torch.cuda.synchronize(dev)
+        dist.barrier(group=self._dp_group)       # every rank's flag is zero before anyone signals
+        self._bn_sync = {"buf": buf, "hdl": hdl, "peers": peers, "local": local, "zeros": zeros}
+        self._graphs = {}
+
+    def _bn_exchange(self, l, B, block, forward):
+        """Synchronised BatchNorm: layer l's sums in `block` (the stats or dstats of a _Buffers) become
+        the global sums scaled by B / global batch (csrc/bnsync.cu); a forward exchange also applies the
+        layer's running-buffer update from the global statistics."""
+        f = self._bn_sync
+        call("ava_b200_bn_stats_exchange", ctypes.byref(f["peers"]), self._dp_rank, self._dp_world,
+             block.data_ptr() + 8 * 64 * l, self._bn_channels[l], B * _LAYERS[l][4] ** 2,
+             ptr(self._flat_run) if forward else None, 64 * l, 64 * l + 32,
+             (self._nbt.data_ptr() + 8 * l) if forward else None, _BN_MOMENTUM, ptr(f["local"]), _stream())
+
+    def _bn_exchange_empty(self):
+        """An empty shard's part of a step's 27 exchanges, in the order a step issues them: it
+        contributes zero sums and a zero count, and still applies the running-buffer updates."""
+        zeros = self._bn_sync["zeros"]
+        zeros.zero_()
+        for l in range(14):
+            self._bn_exchange(l, 0, zeros, forward=True)
+        for l in range(13, 0, -1):
+            self._bn_exchange(l, 0, zeros[14 * 64:], forward=False)
 
     def _rebind_flat(self, flat_p, flat_g):
         """Move the flat parameter / gradient storage into the given buffers (same layout) and
@@ -947,6 +1032,10 @@ class VAE(nn.Module):
         if f is not None and int(f["local"][2].item()) != 0:
             raise RuntimeError("ava_b200: a data-parallel peer did not arrive within the kernel's timeout; "
                                "the replicas are out of step")
+        b = getattr(self, "_bn_sync", None)
+        if b is not None and int(b["local"][1].item()) != 0:
+            raise RuntimeError("ava_b200: a data-parallel peer did not arrive at a BatchNorm statistics "
+                               "exchange within the kernel's timeout; the replicas are out of step")
 
     def _gather_moment_shards(self):
         """Fused data parallelism shards the Adam moments (rank r keeps slice r current): bring every
@@ -1095,11 +1184,15 @@ class VAE(nn.Module):
         self._require_cuda()
         self._sync_hyper()
         x = self._as_input(x)
-        if x.shape[0] == 0:
-            return self._train_step_empty()
-        if self._graph_wanted(x.shape[0]):
-            return self._train_step_graph(x, noise)
-        return self._train_step_eager(x, noise)
+        self._bn_sync_on = self._bn_sync is not None
+        try:
+            if x.shape[0] == 0:
+                return self._train_step_empty()
+            if self._graph_wanted(x.shape[0]):
+                return self._train_step_graph(x, noise)
+            return self._train_step_eager(x, noise)
+        finally:
+            self._bn_sync_on = False
 
     def _train_step_empty(self):
         """This rank's shard of the global batch is empty (a ragged last batch smaller than the
@@ -1108,6 +1201,8 @@ class VAE(nn.Module):
         (_epoch_loss counts them once per global batch)."""
         if self._dp_world <= 1:
             raise ValueError("train_step: empty batch")
+        if self._bn_sync is not None:
+            self._bn_exchange_empty()
         self._flat_g.zero_()
         if self._dp_fused is not None:
             self._adam_dp_native()
@@ -1181,11 +1276,13 @@ class VAE(nn.Module):
     def _epoch_loss(self, n_steps):
         """Sum of the per-batch losses of this epoch (one device->host read).  Under data
         parallelism: summed over ranks, with the per-batch constants counted once per
-        GLOBAL batch as the reference would, and the BN running buffers re-averaged."""
+        GLOBAL batch as the reference would, and the BN running buffers re-averaged (not under
+        synchronised BatchNorm: there they are already identical on every rank)."""
         if self._dp_world > 1:
             import torch.distributed as dist
             dist.all_reduce(self._loss_sum, op=dist.ReduceOp.SUM, group=self._dp_group)
-            self._sync_bn_buffers()
+            if self._bn_sync is None:
+                self._sync_bn_buffers()
             return float(self._loss_sum.item()) - (self._dp_world - 1) * n_steps * self.loss_constant()
         return float(self._loss_sum.item())
 

@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AVA_B200_ABI_VERSION 4
+#define AVA_B200_ABI_VERSION 5
 #define AVA_NUM_BN_LAYERS 14
 #define AVA_STATS_STRIDE 64 /* doubles per layer in a stats block: [0..31]=sum, [32..63]=sum of squares */
 
@@ -260,6 +260,37 @@ typedef struct {
 int ava_b200_adam_step_dp(const ava_b200_dp_peers* h_peers, int rank, int world, float* m, float* v,
                           long long n, float* step_count, const double* hyper, float grad_scale,
                           unsigned int* local, void* stream);
+
+/* Synchronised BatchNorm for data-parallel training (csrc/bnsync.cu): one layer's BatchNorm sums
+ * exchanged over NVLink peer memory so that every rank normalises with the statistics of the GLOBAL
+ * batch, as torch.nn.BatchNorm2d does in the reference's single process on the concatenated batch
+ * (ava/models/vae.py:135-141,162-168).  One single-CTA launch per layer and pass: rank r publishes its
+ * sums and element count, every rank adds the world copies in rank order 0..world-1 in fp64 (so all
+ * ranks get the same bits) and writes back
+ *     sums[c] = (sum over ranks of sums[c]) * (local_count / global_count),   c < channels, 32 + c,
+ * i.e. the global sums scaled to this rank's share: every kernel that divides `sums` by its own local
+ * count then sees the global mean and biased variance (forward stats), or the global c1 and q of the
+ * BatchNorm backward (dstats).  Entries of channels >= `channels` are left untouched.
+ *   h_peers:     HOST struct of DEVICE pointers into symmetric (peer-mapped) memory, index = rank:
+ *                slots[r] = rank r's 2 * AVA_BN_SYNC_SLOT doubles, flags[r] = rank r's uint32 flag;
+ *                both zero-initialised once, before any rank's first call
+ *   local_count: B * H * W of this rank's shard (0 for an empty shard: it contributes zeros)
+ *   running:     NULL for the backward (dstats) exchanges; otherwise the forward exchange also applies
+ *                the running-buffer update of ava_b200_bn_update_running with the global sums and count
+ *                to running[rm_off + c] / running[rv_off + c] and adds 1 to nbt[0] (skipped when the
+ *                global count is 0) -- identical on every rank
+ *   local:       LOCAL device uint32[2], zero-initialised once: [0] exchange sequence number (advanced by
+ *                the kernel, so graph replays need no host involvement), [1] set to 1 if a peer did not
+ *                arrive within 20 s (the kernel then carries on; the caller checks it)
+ * Every rank must make the same sequence of calls.  world <= AVA_DP_MAX_WORLD, 1 <= channels <= 32. */
+#define AVA_BN_SYNC_SLOT 65 /* doubles per slot: [0..63] a stats block, [64] the element count */
+typedef struct {
+  double* slots[AVA_DP_MAX_WORLD];
+  unsigned int* flags[AVA_DP_MAX_WORLD];
+} ava_b200_bn_sync_peers;
+int ava_b200_bn_stats_exchange(const ava_b200_bn_sync_peers* h_peers, int rank, int world, double* sums,
+                               int channels, long long local_count, float* running, int rm_off, int rv_off,
+                               long long* nbt, float momentum, unsigned int* local, void* stream);
 
 /* ------------------------------------------------------------------- get_spec
  * Batched spectrogram front end: ava/preprocessing/utils.py:18-110 (get_spec) with
