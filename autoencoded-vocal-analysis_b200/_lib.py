@@ -23,9 +23,12 @@ SIGNATURES = {
     "ava_b200_bnconv_bwd_data": (I, I, P, P, P, P, P, P, I, P, P, P),
     "ava_b200_bnconv_bwd_weight": (I, I, P, P, P, P, P, P, P, P, P, P, P, P),
     "ava_b200_bnconv_bwd_weight_ws": (I, I),
+    "ava_b200_bnconv_bwd_data_ex": (I, I, P, P, P, P, P, P, I, P, I, P, P, P),
+    "ava_b200_bnconv_bwd_weight_ex": (I, I, P, P, P, P, P, P, P, P, I, P, P, P, P, P, P),
     "ava_b200_set_conv_precision": (I,),
     "ava_b200_get_conv_precision": (),
     "ava_b200_bn_param_grads": (P, P, P, P, P, P, P, P),
+    "ava_b200_bn_param_grads_ex": (P, P, P, P, P, P, P, P, P, I, P),
     "ava_b200_bn_relu_bwd_apply": (P, P, P, P, P, I, I, I, I, P, P, I, P),
     "ava_b200_linear_fwd": (P, I, P, P, P, I, I, I, I, I, I, LL, LL, LL, LL, I, P, LL, P),
     "ava_b200_linear_bwd_data": (P, I, P, P, P, I, I, I, I, I, LL, LL, LL, I, I, P, LL, P),
@@ -35,6 +38,8 @@ SIGNATURES = {
     "ava_b200_bias_grads_ws_bytes": (P, I),
     "ava_b200_latent_fwd": (P, P, P, I, I, P, P, P, P),
     "ava_b200_latent_bwd": (P, P, P, P, P, I, I, P, P),
+    "ava_b200_latent_heads_grad": (P, P, P, P, I, I, P, P),
+    "ava_b200_recon_input_grad": (P, P, P, LL, F, P, P),
     "ava_b200_recon": (P, P, LL, F, P, P, P, I, I, P),
     "ava_b200_elbo_finalize": (P, I, I, F, P, P, P),
     "ava_b200_adam_step": (P, P, P, P, LL, P, D, D, D, D, F, P),

@@ -154,11 +154,13 @@ __device__ __forceinline__ BnCoef bn_coef(const double* stats, int c, double cou
 // Evaluated in fp64: the two terms cancel heavily (BN backward projects out the mean and
 // the xhat direction), and a coefficient rounded to fp32 would add a *coherent* error to
 // every element of the channel, which bias / BN-affine gradients then sum up.
+// Eval mode (rvar != NULL): the BatchNorm is the fixed affine map of the running buffers, so
+// dx = gamma*invstd_r*dy: p = gamma/sqrt(rvar + eps), q = c1 = 0.
 struct DzCoef {
   double p, q, mean, c1;
 };
 __device__ __forceinline__ DzCoef dz_coef(const float* gamma, const double* stats, const double* dstats, int c,
-                                          double count) {
+                                          double count, const float* rvar = nullptr) {
   DzCoef k;
   if (gamma == nullptr) {
     k.p = 1.0;
@@ -167,15 +169,22 @@ __device__ __forceinline__ DzCoef dz_coef(const float* gamma, const double* stat
     k.c1 = 0.0;
     return k;
   }
-  double mean = stats[c] / count;
-  double var = stats[32 + c] / count - mean * mean;
-  if (var < 0.0) var = 0.0;
+  double mean = 0.0, var, s = 0.0, c1 = 0.0;
+  if (rvar != nullptr) {
+    var = (double)rvar[c];
+  } else {
+    mean = stats[c] / count;
+    var = stats[32 + c] / count - mean * mean;
+    if (var < 0.0) var = 0.0;
+    s = dstats[32 + c];
+    c1 = dstats[c] / count;
+  }
   double invstd = rsqrt(var + (double)kBnEps);
   double g = (double)gamma[c];
   k.p = g * invstd;
-  k.q = -g * invstd * invstd * invstd * dstats[32 + c] / count;
+  k.q = -g * invstd * invstd * invstd * s / count;
   k.mean = mean;
-  k.c1 = dstats[c] / count;
+  k.c1 = c1;
   return k;
 }
 __device__ __forceinline__ float dz_apply(const DzCoef& k, float g, float y) {

@@ -63,6 +63,7 @@ struct GconvParams {
   const double* stats_self;
   const float* gamma_self;
   const double* dstats_in;
+  const float* rvar_self;   // eval-mode BatchNorm: its running variance (NULL: train mode, batch statistics)
   int mask_in;
   // EPI_BWD, optional: the nine per-channel border sums of the dz written here (what
   // ava_b200_dz_border_sums would compute in a separate pass; mode 0 / 1 as there), accumulated
@@ -513,7 +514,7 @@ __global__ void __launch_bounds__(GconvCfg<KIND, CI, CO, TW, INMODE, TERMS>::NT,
       // out = p*(g - c1) + q*(x - mean) = p*g + q*x + k: p, q rounded to fp32 (a relative error of
       // 6e-8 on a whole channel's gradient), k = -(p*c1 + q*mean) formed in fp64 from the ROUNDED
       // p, q, then rounded once (a constant shift of <= 6e-8 |k| for the whole channel)
-      const DzCoef k = dz_coef(P.gamma_self, P.stats_self, P.dstats_in, tid, P.out_count);
+      const DzCoef k = dz_coef(P.gamma_self, P.stats_self, P.dstats_in, tid, P.out_count, P.rvar_self);
       const float pf = (float)k.p, qf = (float)k.q;
       s_dzf[tid] = pf;
       s_dzf[32 + tid] = qf;
@@ -1661,6 +1662,9 @@ struct WgradParams {
   const float* beta;
   const double* stats;
   double bn_count;
+  // eval mode (train == 0): x is centred at the running mean instead of the batch mean
+  const float* rmean;
+  int train;
   float* partial;  // [grid][CG*CI*9 + 32]
   int B, Hg, Wg;   // dims of the G tensor
 };
@@ -1752,10 +1756,11 @@ __global__ void __launch_bounds__(256, 2)
     constexpr int CA = CONVT ? CG : CI;  // channels of x
     if (c < CA) {
       // centred raw input: x - mean (mean rounded to fp32; the finalize pass corrects for the
-      // rounding and applies gamma*invstd / beta, see bnconv_finalize_kernel)
-      BnCoef k = bn_coef(P.stats, c, P.bn_count, nullptr, nullptr, nullptr, nullptr, true);
+      // rounding and applies gamma*invstd / beta, see bnconv_finalize_kernel); eval mode: x - running mean
+      const float mean =
+          P.train ? bn_coef(P.stats, c, P.bn_count, nullptr, nullptr, nullptr, nullptr, true).mean : P.rmean[c];
       s_aff[c] = 1.f;
-      s_aff[32 + c] = -k.mean;
+      s_aff[32 + c] = -mean;
     }
   }
   // per-thread transform work lists (identical for every tile)
@@ -2005,9 +2010,10 @@ __global__ void __launch_bounds__((((CG + 15) / 16) * (CI / 8) == 6) ? 192 : 256
   if (tid < 32) {
     constexpr int CA = CONVT ? CG : CI;
     if (tid < CA) {
-      BnCoef k = bn_coef(P.stats, tid, P.bn_count, nullptr, nullptr, nullptr, nullptr, true);
+      const float mean =
+          P.train ? bn_coef(P.stats, tid, P.bn_count, nullptr, nullptr, nullptr, nullptr, true).mean : P.rmean[tid];
       s_aff[tid] = 1.f;        // centred raw input, see wgrad_kernel
-      s_aff[32 + tid] = -k.mean;
+      s_aff[32 + tid] = -mean;
     }
   }
 
@@ -2297,6 +2303,9 @@ struct FinalizeParams {
   const float* beta;
   const double* stats;    // sum x | sum x^2 of this layer's input
   double count;
+  const float* rmean;     // eval mode (train == 0): the running buffers replace the batch statistics
+  const float* rvar;
+  int train;
   const double* tsums;    // [9][32], see trimmed_dz_sum
   float* dw;
   float* db;
@@ -2360,11 +2369,18 @@ __global__ void __launch_bounds__(kFinWarps * 32) bnconv_finalize_kernel(const F
     cx = j / (9 * P.Cz);
   }
   const double T = trimmed_dz_sum(P.tsums, cz, k / 3, k % 3, P.convt, P.s2);
-  const double mean = P.stats[cx] / P.count;
-  double var = P.stats[32 + cx] / P.count - mean * mean;
-  if (var < 0.0) var = 0.0;
+  double mean, var;
+  if (P.train) {
+    mean = P.stats[cx] / P.count;
+    var = P.stats[32 + cx] / P.count - mean * mean;
+    if (var < 0.0) var = 0.0;
+  } else {
+    mean = (double)P.rmean[cx];
+    var = (double)P.rvar[cx];
+  }
   const double invstd = rsqrt(var + (double)kBnEps);
   // the kernels centred with the fp32-rounded mean: sum dz*(x-mean) = sum dz*(x-mean32) + (mean32-mean)*T
+  // (zero in eval mode, where the running mean is fp32 already)
   const double rc = r + ((double)(float)mean - mean) * T;
   const double wv = (double)P.w[j];
   P.dw[j] = (float)((double)P.gamma[cx] * invstd * rc + (double)P.beta[cx] * T);
@@ -2444,6 +2460,8 @@ static int launch_finalize(const WgradParams& P, FinalizeParams F, int nparts, c
   F.s2 = (S == 2);
   F.stats = P.stats;
   F.count = P.bn_count;
+  F.rmean = P.rmean;
+  F.train = P.train;
   const int n = CG * CI * 9 + F.Cz;
   bnconv_finalize_kernel<<<(n + 31) / 32, kFinWarps * 32, 0, stream>>>(F);
   return check_launch("bnconv_finalize");
@@ -2632,11 +2650,14 @@ extern "C" int ava_b200_bnconv_fwd(int layer, int B, const float* x, float* y, c
   return 1;
 }
 
-extern "C" int ava_b200_bnconv_bwd_data(int layer, int B, const float* dz, const float* w, const float* x,
-                                        const float* gamma, const double* stats_in, const double* dstats,
-                                        int relu_mask, float* dz_prev, double* tsums_prev, void* stream_) {
+extern "C" int ava_b200_bnconv_bwd_data_ex(int layer, int B, const float* dz, const float* w, const float* x,
+                                           const float* gamma, const double* stats_in, const float* running_var,
+                                           int train, const double* dstats, int relu_mask, float* dz_prev,
+                                           double* tsums_prev, void* stream_) {
   AVA_REQUIRE(layer >= 0 && layer < 14, "bnconv_bwd_data: bad layer %d", layer);
   AVA_REQUIRE(dz_prev != nullptr && x != nullptr, "bnconv_bwd_data: output and layer input required");
+  AVA_REQUIRE(train || gamma == nullptr || running_var != nullptr,
+              "bnconv_bwd_data: eval mode needs the running variance");
   if (B <= 0) return 0;
   cudaStream_t stream = (cudaStream_t)stream_;
   const LayerGeom& L = kLayers[layer];
@@ -2649,6 +2670,7 @@ extern "C" int ava_b200_bnconv_bwd_data(int layer, int B, const float* dz, const
   P.stats_self = stats_in;
   P.gamma_self = gamma;
   P.dstats_in = dstats;
+  P.rvar_self = train ? nullptr : running_var;
   P.mask_in = relu_mask;
   P.tsums_out = tsums_prev;
   // the dz written here belongs to layer-1: parity classes if that is a stride-2 conv-transpose
@@ -2684,6 +2706,13 @@ extern "C" int ava_b200_bnconv_bwd_data(int layer, int B, const float* dz, const
   return 1;
 }
 
+extern "C" int ava_b200_bnconv_bwd_data(int layer, int B, const float* dz, const float* w, const float* x,
+                                        const float* gamma, const double* stats_in, const double* dstats,
+                                        int relu_mask, float* dz_prev, double* tsums_prev, void* stream) {
+  return ava_b200_bnconv_bwd_data_ex(layer, B, dz, w, x, gamma, stats_in, nullptr, 1, dstats, relu_mask, dz_prev,
+                                     tsums_prev, stream);
+}
+
 extern "C" long long ava_b200_bnconv_bwd_weight_ws(int layer, int B) {
   (void)B;
   if (layer < 0 || layer >= 14) return 0;
@@ -2692,13 +2721,16 @@ extern "C" long long ava_b200_bnconv_bwd_weight_ws(int layer, int B) {
   return (long long)kWgradMaxCtas * (L.cin * L.cout * 9 + 32) * (long long)sizeof(float);
 }
 
-extern "C" int ava_b200_bnconv_bwd_weight(int layer, int B, const float* dz, const float* x, const float* w,
-                                          const float* gamma, const float* beta, const double* stats_in,
-                                          const double* tsums, float* dw, float* db, double* dstats, void* ws,
-                                          void* stream_) {
+extern "C" int ava_b200_bnconv_bwd_weight_ex(int layer, int B, const float* dz, const float* x, const float* w,
+                                             const float* gamma, const float* beta, const double* stats_in,
+                                             const float* running_mean, const float* running_var, int train,
+                                             const double* tsums, float* dw, float* db, double* dstats, void* ws,
+                                             void* stream_) {
   AVA_REQUIRE(layer >= 0 && layer < 14, "bnconv_bwd_weight: bad layer %d", layer);
   AVA_REQUIRE(ws != nullptr, "bnconv_bwd_weight: workspace required");
   AVA_REQUIRE(w != nullptr && tsums != nullptr && dstats != nullptr, "bnconv_bwd_weight: w, tsums, dstats required");
+  AVA_REQUIRE(train ? stats_in != nullptr : (running_mean != nullptr && running_var != nullptr),
+              "bnconv_bwd_weight: %s required", train ? "stats_in" : "running_mean and running_var");
   if (B <= 0) return 0;
   cudaStream_t stream = (cudaStream_t)stream_;
   const LayerGeom& L = kLayers[layer];
@@ -2706,8 +2738,11 @@ extern "C" int ava_b200_bnconv_bwd_weight(int layer, int B, const float* dz, con
   WgradParams P = {};
   P.stats = stats_in;
   P.bn_count = (double)B * L.h_in * L.h_in;
+  P.rmean = running_mean;
+  P.train = train ? 1 : 0;
   P.B = B;
   FinalizeParams F = {};
+  F.rvar = running_var;
   F.w = w;
   F.gamma = gamma;
   F.beta = beta;
@@ -2747,6 +2782,14 @@ extern "C" int ava_b200_bnconv_bwd_weight(int layer, int B, const float* dz, con
     }
     return rc;
   }
+}
+
+extern "C" int ava_b200_bnconv_bwd_weight(int layer, int B, const float* dz, const float* x, const float* w,
+                                          const float* gamma, const float* beta, const double* stats_in,
+                                          const double* tsums, float* dw, float* db, double* dstats, void* ws,
+                                          void* stream) {
+  return ava_b200_bnconv_bwd_weight_ex(layer, B, dz, x, w, gamma, beta, stats_in, nullptr, nullptr, 1, tsums, dw, db,
+                                       dstats, ws, stream);
 }
 
 extern "C" int ava_b200_dz_border_sums(const float* dz, int B, int C, int H, int W, int mode, double* tsums,

@@ -86,15 +86,26 @@ __global__ void bn_update_running_kernel(const double* stats, BnTable T, float* 
                     running + T.off_b[l], momentum);
 }
 
-__global__ void bn_param_grads_kernel(const double* stats, const double* dstats, BnTable T, float* grads) {
+// eval-mode BatchNorm (running != NULL): layer l's running variance at running[rv_off[l]]
+struct BnRunVar {
+  int rv_off[AVA_NUM_BN_LAYERS];
+};
+
+__global__ void bn_param_grads_kernel(const double* stats, const double* dstats, BnTable T, float* grads,
+                                      const float* running, BnRunVar R) {
   const int l = blockIdx.x, c = threadIdx.x;
   if (c >= T.channels[l] || T.counts[l] == 0) return;
-  const double n = (double)T.counts[l];
-  const double* st = stats + (size_t)l * kStatsStride;
   const double* ds = dstats + (size_t)l * kStatsStride;
-  double mean = st[c] / n;
-  double var = st[32 + c] / n - mean * mean;
-  if (var < 0) var = 0;
+  double var;
+  if (running == nullptr) {
+    const double n = (double)T.counts[l];
+    const double* st = stats + (size_t)l * kStatsStride;
+    double mean = st[c] / n;
+    var = st[32 + c] / n - mean * mean;
+    if (var < 0) var = 0;
+  } else {
+    var = (double)running[R.rv_off[l] + c];
+  }
   double invstd = rsqrt(var + (double)kBnEps);
   grads[T.off_a[l] + c] = (float)(invstd * ds[32 + c]);  // dgamma
   grads[T.off_b[l] + c] = (float)ds[c];                  // dbeta
@@ -255,6 +266,38 @@ latent_bwd_kernel(const float* __restrict__ heads, const float* __restrict__ eps
   }
 }
 
+// encode()'s backward seed: g_heads = (dmu | du | dd * d), d = exp(logd) as the forward returned it;
+// a NULL seed is zero
+__global__ void __launch_bounds__(256)
+latent_heads_grad_kernel(const float* __restrict__ dmu, const float* __restrict__ du, const float* __restrict__ dd,
+                         const float* __restrict__ d, long long n, int Z, float* __restrict__ g_heads) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const long long b = i / Z;
+    float* grow = g_heads + b * 3 * Z + (i - b * Z);
+    grow[0] = dmu ? dmu[i] : 0.f;
+    grow[Z] = du ? du[i] : 0.f;
+    grow[2 * Z] = dd ? dd[i] * d[i] : 0.f;
+  }
+}
+
+// forward()'s input gradient: the encoder's part plus the direct reconstruction term,
+// dx = dx_enc - prec * (x_rec - x)
+__global__ void __launch_bounds__(256)
+recon_input_grad_kernel(const float* dx_enc, const float* __restrict__ x, const float* __restrict__ xr,
+                        long long n4, float prec, float* dx) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
+       i += (long long)gridDim.x * blockDim.x) {
+    const float4 a = __ldg(reinterpret_cast<const float4*>(x) + i);
+    const float4 r = __ldg(reinterpret_cast<const float4*>(xr) + i);
+    float4 e = dx_enc ? reinterpret_cast<const float4*>(dx_enc)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+    e.x -= prec * (r.x - a.x);
+    e.y -= prec * (r.y - a.y);
+    e.z -= prec * (r.z - a.z);
+    e.w -= prec * (r.w - a.w);
+    reinterpret_cast<float4*>(dx)[i] = e;
+  }
+}
+
 // ------------------------------------------------------------------------------ recon
 // tsums (optional): the border sums of the written gradient g viewed as [*, 1, H, W] planes
 __global__ void __launch_bounds__(256)
@@ -341,12 +384,26 @@ extern "C" int ava_b200_bn_update_running(const double* stats, const int* h_chan
   return check_launch("bn_update_running");
 }
 
+extern "C" int ava_b200_bn_param_grads_ex(const double* stats, const double* dstats, const int* h_channels,
+                                          const long long* h_counts, float* grads, const int* h_dgamma_off,
+                                          const int* h_dbeta_off, const float* running, const int* h_rv_off,
+                                          int train, void* stream) {
+  AVA_REQUIRE(train || (running != nullptr && h_rv_off != nullptr),
+              "bn_param_grads: eval mode needs the running buffers and their offsets");
+  BnTable T = make_table(h_channels, h_counts, h_dgamma_off, h_dbeta_off);
+  BnRunVar R = {};
+  if (!train)
+    for (int l = 0; l < AVA_NUM_BN_LAYERS; ++l) R.rv_off[l] = h_rv_off[l];
+  bn_param_grads_kernel<<<AVA_NUM_BN_LAYERS, 32, 0, (cudaStream_t)stream>>>(stats, dstats, T, grads,
+                                                                          train ? nullptr : running, R);
+  return check_launch("bn_param_grads");
+}
+
 extern "C" int ava_b200_bn_param_grads(const double* stats, const double* dstats, const int* h_channels,
                                        const long long* h_counts, float* grads, const int* h_dgamma_off,
                                        const int* h_dbeta_off, void* stream) {
-  BnTable T = make_table(h_channels, h_counts, h_dgamma_off, h_dbeta_off);
-  bn_param_grads_kernel<<<AVA_NUM_BN_LAYERS, 32, 0, (cudaStream_t)stream>>>(stats, dstats, T, grads);
-  return check_launch("bn_param_grads");
+  return ava_b200_bn_param_grads_ex(stats, dstats, h_channels, h_counts, grads, h_dgamma_off, h_dbeta_off, nullptr,
+                                    nullptr, 1, stream);
 }
 
 extern "C" int ava_b200_bn_relu_bwd_apply(const float* g, const float* a, const float* gamma, const double* stats,
@@ -380,6 +437,29 @@ extern "C" int ava_b200_latent_bwd(const float* heads, const float* eps_w, const
   if (B <= 0) return 0;
   latent_bwd_kernel<<<(B + 7) / 8, 256, 0, (cudaStream_t)stream>>>(heads, eps_w, eps_d, z, gz, B, Z, g_heads);
   return check_launch("latent_bwd");
+}
+
+extern "C" int ava_b200_latent_heads_grad(const float* dmu, const float* du, const float* dd, const float* d, int B,
+                                          int Z, float* g_heads, void* stream) {
+  AVA_REQUIRE(Z >= 1 && B >= 0, "latent_heads_grad: B=%d Z=%d", B, Z);
+  AVA_REQUIRE(dd == nullptr || d != nullptr, "latent_heads_grad: a seed on d needs d");
+  if (B == 0) return 0;
+  const long long n = (long long)B * Z;
+  long long grid = (n + 255) / 256;
+  if (grid > 8 * kNumSMs) grid = 8 * kNumSMs;
+  latent_heads_grad_kernel<<<(int)grid, 256, 0, (cudaStream_t)stream>>>(dmu, du, dd, d, n, Z, g_heads);
+  return check_launch("latent_heads_grad");
+}
+
+extern "C" int ava_b200_recon_input_grad(const float* dx_enc, const float* x, const float* x_rec, long long n,
+                                         float precision, float* dx, void* stream) {
+  AVA_REQUIRE(n % 4 == 0 && n >= 0, "recon_input_grad: n=%lld must be a non-negative multiple of 4", n);
+  if (n == 0) return 0;
+  const long long n4 = n / 4;
+  long long grid = (n4 + 255) / 256;
+  if (grid > 8 * kNumSMs) grid = 8 * kNumSMs;
+  recon_input_grad_kernel<<<(int)grid, 256, 0, (cudaStream_t)stream>>>(dx_enc, x, x_rec, n4, precision, dx);
+  return check_launch("recon_input_grad");
 }
 
 extern "C" int ava_b200_recon(const float* x, const float* x_rec, long long n, float precision, float* g,

@@ -15,7 +15,9 @@ if the model is not on a CUDA device or the native library is missing.
 
 Additions over the reference API (keyword-only / new methods, defaults preserve
 behaviour): ``precision=`` constructor argument, ``train_step``, ``compute_loss``,
-``grad_dict``, ``load_flat_state``.
+``grad_dict``, ``load_flat_state``.  ``encode``, ``decode`` and ``forward`` are differentiable
+as the reference's autograd graphs are, in train and eval mode, w.r.t. their input and the
+parameters they touch (native backward kernels; no double backward).
 """
 import ctypes
 import math
@@ -128,6 +130,20 @@ class _Buffers:
         self.loss = torch.zeros(1, **f32)
         # backward scratch (allocated lazily)
         self.g = None
+        # eval-mode autograd: the running buffers the forward normalised with ([14][64] as
+        # VAE._flat_run), which the backward must use even if a train-mode call moves the live ones;
+        # None for train mode (batch statistics)
+        self.run = None
+        self._run_store = None
+
+    def snapshot_running(self, flat_run, train):
+        if train:
+            self.run = None
+            return
+        if self._run_store is None:
+            self._run_store = torch.empty_like(flat_run)
+        self._run_store.copy_(flat_run)
+        self.run = self._run_store
 
     def alloc_backward(self, z_dim):
         if self.g is not None:
@@ -271,6 +287,7 @@ class VAE(nn.Module):
         self.epoch = 0
         self.loss = {'train': {}, 'test': {}}
         self._bufs = {}
+        self._grad_pool = {}       # free activation sets of the autograd paths, see _grad_buffers
         self._scratch = None
         self._step_host = 0
         self._graphs = {}
@@ -402,6 +419,7 @@ class VAE(nn.Module):
         self._hyper_host = None
         self._loss_sum = torch.zeros(1, dtype=torch.float64, device=dev)
         self._bufs, self._scratch, self._graphs = {}, None, {}
+        self._grad_pool = {}
         # host-side tables for the two BN bookkeeping kernels
         self._h_channels = (ctypes.c_int * 14)(*self._bn_channels)
         self._h_rm_off = (ctypes.c_int * 14)(*[i * 64 for i in range(14)])
@@ -460,6 +478,26 @@ class VAE(nn.Module):
             b = _Buffers(B, self.z_dim, self._flat_p.device)
         self._bufs[B] = b          # most recently used last
         return b
+
+    def _grad_buffers(self, B):
+        """Activation workspace for a call that records an autograd graph.  The graph owns it until
+        its backward has run or it is freed (_Lease): such sets never come from the _buffers_for cache,
+        so neither a later call nor a captured train_step graph writes into them.  Sets come back to a
+        small per-size free list, so a forward/backward loop allocates nothing after warm-up."""
+        free = self._grad_pool.get(B)
+        if free:
+            return free.pop()
+        return _Buffers(B, self.z_dim, self._flat_p.device)
+
+    def _release_grad_buffers(self, bufs):
+        if bufs.h1.device != self._flat_p.device:
+            return                 # (the model moved while the graph was alive)
+        free = self._grad_pool.pop(bufs.B, [])
+        if len(free) < 2:
+            free.append(bufs)
+        self._grad_pool[bufs.B] = free         # most recently used last
+        while len(self._grad_pool) > self._MAX_BATCH_SIZES:
+            self._grad_pool.pop(next(iter(self._grad_pool)))
 
     def _side_fork(self):
         """The second stream, waiting for everything issued so far on the current one."""
@@ -616,13 +654,15 @@ class VAE(nn.Module):
         ed = torch.randn(B, self.z_dim, dtype=torch.float32, device=dev)
         return ew, ed
 
-    def _forward_native(self, x, noise, train, want_grad_seed):
-        """Full forward pass; returns the _Buffers holding every intermediate.
-        Loss (fp32) lands in bufs.loss; if want_grad_seed, dL/dx_rec in bufs.g[0]."""
+    def _forward_native(self, x, noise, train, want_grad_seed, bufs=None):
+        """Full forward pass; returns the _Buffers holding every intermediate (`bufs`, or the
+        cached set of this batch size).  Loss (fp32) lands in bufs.loss; if want_grad_seed,
+        dL/dx_rec in bufs.g[0]."""
         self._require_cuda()
         x = self._as_input(x)
         B = x.shape[0]
-        bufs = self._buffers_for(B)
+        if bufs is None:
+            bufs = self._buffers_for(B)
         self._cur = bufs
         self._scratch_need = self._scratch_need_for(B)
         s = _stream()
@@ -658,32 +698,38 @@ class VAE(nn.Module):
             cache[B] = self._scratch_bytes(B)
         return cache[B]
 
-    def _conv_bwd(self, l, bufs, dz, x, dz_prev):
+    def _conv_bwd(self, l, bufs, dz, x, dz_prev, relu_mask=1):
         """Backward of fused layer l given dz = the gradient w.r.t. its pre-activation output,
         whose nine border sums the kernel that wrote dz has already accumulated into tsums[l].
         (1) weight / bias gradients into the flat gradient buffer AND this layer's
         BatchNorm-backward reductions dstats[l] (both from the same centred raw product, see
         include/ava_b200.h); (2) the data gradient, pushed through this layer's BatchNorm backward
         and the previous layer's ReLU in the kernel's epilogue, lands in dz_prev as the previous
-        layer's dz -- the gradient w.r.t. the BatchNorm output never goes to memory."""
+        layer's dz -- the gradient w.r.t. the BatchNorm output never goes to memory.
+        bufs.run set: eval-mode BatchNorm with those running buffers.  relu_mask=0: no ReLU factor
+        (layer 0's data gradient is the gradient w.r.t. the input spectrogram)."""
         B = bufs.B
         name = _LAYERS[l][0]
         st, ds, ts = bufs.stats.data_ptr(), bufs.dstats.data_ptr(), bufs.tsums.data_ptr()
         s = _stream()
         gamma, beta = self._p("bn%d.weight" % (l + 1)), self._p("bn%d.bias" % (l + 1))
+        train, rm, rv = 1, None, None
+        if bufs.run is not None:
+            train, rm = 0, bufs.run.data_ptr() + 4 * 64 * l
+            rv = rm + 4 * 32
         ws = self._ws(self._scratch_need)
         _set_conv_precision(self._tc_conv)
-        call("ava_b200_bnconv_bwd_weight", l, B, ptr(dz), ptr(x), self._p(name + ".weight"), gamma, beta,
-             st + 8 * 64 * l, ts + 8 * 288 * l, self._g(name + ".weight"), self._g(name + ".bias"),
-             ds + 8 * 64 * l, ptr(ws), s)
+        call("ava_b200_bnconv_bwd_weight_ex", l, B, ptr(dz), ptr(x), self._p(name + ".weight"), gamma, beta,
+             st + 8 * 64 * l, rm, rv, train, ts + 8 * 288 * l, self._g(name + ".weight"),
+             self._g(name + ".bias"), ds + 8 * 64 * l, ptr(ws), s)
         if dz_prev is not None:
             if self._bn_sync_on:
                 self._bn_exchange(l, B, bufs.dstats, forward=False)
             # the epilogue also accumulates the border sums of the dz it writes (layer l-1's; layer
-            # 7 writes fc8's output gradient, which has none)
-            call("ava_b200_bnconv_bwd_data", l, B, ptr(dz), self._p(name + ".weight"), ptr(x), gamma,
-                 st + 8 * 64 * l, ds + 8 * 64 * l, 1, ptr(dz_prev),
-                 (ts + 8 * 288 * (l - 1)) if l != 7 else None, s)
+            # 7 writes fc8's output gradient and layer 0 the input's, which need none)
+            call("ava_b200_bnconv_bwd_data_ex", l, B, ptr(dz), self._p(name + ".weight"), ptr(x), gamma,
+                 st + 8 * 64 * l, rv, train, ds + 8 * 64 * l, relu_mask, ptr(dz_prev),
+                 (ts + 8 * 288 * (l - 1)) if l not in (0, 7) else None, s)
 
     def _bwd_decoder(self, bufs):
         """Backward segment 1: decoder conv stack (layers 13..7) and fc8..fc5.  Afterwards the
@@ -709,13 +755,15 @@ class VAE(nn.Module):
                          B, 64, Z, bias_jobs=jobs)
         self._flush_bias(jobs)
 
-    def _bwd_dense_encoder(self, bufs):
+    def _bwd_dense_encoder(self, bufs, latent=True):
         """Backward segment 2: latent (analytic gradients of sample + prior + entropy) and the
         encoder's dense layers.  Afterwards the gradients of fc1..fc43 are final (fc1.weight is
-        half of all parameters)."""
+        half of all parameters).  latent=False: bufs.gheads already holds the heads' gradient
+        (encode's backward)."""
         B, Z, s = bufs.B, self.z_dim, _stream()
-        call("ava_b200_latent_bwd", ptr(bufs.heads), ptr(bufs.eps_w), ptr(bufs.eps_d), ptr(bufs.z),
-             ptr(bufs.gz), B, Z, ptr(bufs.gheads), s)
+        if latent:
+            call("ava_b200_latent_bwd", ptr(bufs.heads), ptr(bufs.eps_w), ptr(bufs.eps_d), ptr(bufs.z),
+                 ptr(bufs.gz), B, Z, ptr(bufs.gheads), s)
         jobs = []
         self._linear_bwd(bufs.gheads, 3 * Z, None, bufs.h3, 192, "fc41.weight", "fc41.bias", bufs.dh3, 192,
                          B, Z, 64, groups=3, dy_gs=Z, x_gs=64, w_gs=Z * 64, b_gs=Z, dx_gs=64, bias_jobs=jobs)
@@ -727,9 +775,10 @@ class VAE(nn.Module):
                          bufs.da6, 8192, B, 1024, 8192, tc=self._tc, bias_jobs=jobs)
         self._flush_bias(jobs)
 
-    def _bwd_conv_encoder(self, bufs):
+    def _bwd_conv_encoder(self, bufs, dx=None, n_bn=14):
         """Backward segment 3: encoder conv stack (layers 6..0) and the BatchNorm affine
-        parameter gradients of all 14 layers."""
+        parameter gradients of layers 0..n_bn-1.  dx (optional): the gradient w.r.t. the input
+        spectrogram, layer 0's data gradient."""
         B, s = bufs.B, _stream()
         # conv7's ReLU on the gradient arriving from fc1 (no BatchNorm at this seam)
         # (and the nine border sums of the dz it writes, conv7's)
@@ -737,21 +786,27 @@ class VAE(nn.Module):
              1, ptr(bufs.da6), bufs.tsums.data_ptr() + 8 * 288 * 6, 16, s)
         g_cur = bufs.da6
         free = [bufs.g[0], bufs.g[1]]
-        for l in range(6, -1, -1):          # (layer 0 needs no data gradient)
+        for l in range(6, -1, -1):          # (layer 0's data gradient only for dx)
             xin = bufs.act[l - 1] if l > 0 else bufs.x
-            out = free[0] if l > 0 else None
-            self._conv_bwd(l, bufs, g_cur, xin, out)
+            out = free[0] if l > 0 else dx
+            self._conv_bwd(l, bufs, g_cur, xin, out, relu_mask=1 if l > 0 else 0)
             g_cur, free = out, [free[1], free[0]]
-        st, ds = bufs.stats.data_ptr(), bufs.dstats.data_ptr()
-        counts = [B * _LAYERS[l][4] ** 2 for l in range(14)]
-        h_counts = (ctypes.c_longlong * 14)(*counts)
-        call("ava_b200_bn_param_grads", st, ds, self._h_channels, h_counts, ptr(self._flat_g),
-             self._h_dg_off, self._h_db_off, s)
+        self._bn_param_grads(bufs, 0, n_bn)
 
-    def _backward_native(self, bufs, after_decoder=None, after_dense=None):
+    def _bn_param_grads(self, bufs, first, last):
+        """BatchNorm affine parameter gradients of layers first..last-1 from their dstats (one launch;
+        eval mode with the running buffers in bufs.run)."""
+        counts = [bufs.B * _LAYERS[l][4] ** 2 if first <= l < last else 0 for l in range(14)]
+        h_counts = (ctypes.c_longlong * 14)(*counts)
+        call("ava_b200_bn_param_grads_ex", bufs.stats.data_ptr(), bufs.dstats.data_ptr(), self._h_channels,
+             h_counts, ptr(self._flat_g), self._h_dg_off, self._h_db_off, ptr(bufs.run), self._h_rv_off,
+             1 if bufs.run is None else 0, _stream())
+
+    def _backward_native(self, bufs, after_decoder=None, after_dense=None, dx=None):
         """Backward of the whole loss; leaves every parameter gradient in the flat
         gradient buffer (overwritten, not accumulated).  Replaces loss.backward(),
-        ava/models/vae.py:352.  The two callbacks fire where a gradient bucket becomes final."""
+        ava/models/vae.py:352.  The two callbacks fire where a gradient bucket becomes final.
+        dx (optional): the encoder's part of the input gradient, see _bwd_conv_encoder."""
         self._bwd_decoder(bufs)
         if after_decoder is not None:
             self._side_join()
@@ -760,7 +815,7 @@ class VAE(nn.Module):
         if after_dense is not None:
             self._side_join()
             after_dense()
-        self._bwd_conv_encoder(bufs)
+        self._bwd_conv_encoder(bufs, dx=dx)
         self._side_join()
 
     def _sync_hyper(self):
@@ -790,12 +845,33 @@ class VAE(nn.Module):
         return x.contiguous()
 
     # ------------------------------------------------------------------ public API
+    def _grad_wanted(self, x, params):
+        return torch.is_grad_enabled() and (
+            (torch.is_tensor(x) and x.requires_grad) or any(p.requires_grad for p in params))
+
+    def _params_of(self, part):
+        """The parameters a call touches: 'encoder' (conv1-7, bn1-7, fc1-fc43), 'decoder' (fc5-8,
+        convt1-7, bn8-14) or 'all', in registration order."""
+        def is_enc(name):
+            layer = name.split(".")[0]
+            if layer.startswith("bn"):
+                return int(layer[2:]) <= 7
+            return (layer.startswith("conv") and not layer.startswith("convt")) or \
+                layer in ("fc1", "fc2", "fc31", "fc32", "fc33", "fc41", "fc42", "fc43")
+        return [(n, p) for n, p in self.named_parameters()
+                if part == "all" or is_enc(n) == (part == "encoder")]
+
     def encode(self, x):
         """Compute q(z|x) = N(mu, u u^T + diag(d)).  ava/models/vae.py:189-233.
 
         Returns mu [B,z], u [B,z,1], d [B,z].  BatchNorm follows ``self.training``
         exactly as in the reference (batch statistics + running-buffer update in
-        train mode).  Not differentiable (use ``forward`` for training)."""
+        train mode).  Differentiable, in train and eval mode, w.r.t. `x` and the encoder's
+        parameters (conv1-7, bn1-7, fc1, fc2, fc31-33, fc41-43) when grad mode is on and one of
+        them requires grad; the backward is native (_EncodeFn)."""
+        enc = self._params_of("encoder")
+        if self._grad_wanted(x, [p for _, p in enc]):
+            return _EncodeFn.apply(self, x, [n for n, _ in enc], *[p for _, p in enc])
         self._require_cuda()
         x = self._as_input(x)
         B, Z = x.shape[0], self.z_dim
@@ -815,7 +891,12 @@ class VAE(nn.Module):
         return mu, u, bufs.d.clone()
 
     def decode(self, z):
-        """Compute the mean of p(x|z).  ava/models/vae.py:236-270.  Returns [B,16384]."""
+        """Compute the mean of p(x|z).  ava/models/vae.py:236-270.  Returns [B,16384].
+        Differentiable, in train and eval mode, w.r.t. `z` and the decoder's parameters (fc5-8,
+        convt1-7, bn8-14) when grad mode is on and one of them requires grad (_DecodeFn)."""
+        dec = self._params_of("decoder")
+        if self._grad_wanted(z, [p for _, p in dec]):
+            return _DecodeFn.apply(self, z, [n for n, _ in dec], *[p for _, p in dec])
         self._require_cuda()
         z = z.to(device=self._flat_p.device, dtype=torch.float32).contiguous()
         B = z.shape[0]
@@ -832,13 +913,18 @@ class VAE(nn.Module):
     def forward(self, x, return_latent_rec=False, noise=None):
         """Send `x` round trip and compute the loss (negative ELBO summed over the
         batch; ava/models/vae.py:273-327).  The returned loss supports
-        ``.backward()``: gradients come from the native backward pass.
+        ``.backward()`` in train and eval mode (eval: BatchNorm with the running buffers, which the
+        backward leaves unchanged): gradients w.r.t. every parameter and, if `x` requires grad, the
+        input come from the native backward pass.
 
         `noise` (optional, addition): (eps_W [B,1], eps_D [B,z]) to use instead of
-        drawing them with torch.randn."""
-        need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
-        if need_grad:
-            loss, z, x_rec = _LossFn.apply(self, x, noise, *list(self.parameters()))
+        drawing them with torch.randn.
+
+        Under ``enable_data_parallel`` this, ``encode`` and ``decode`` and their backward passes
+        stay local to the rank: no collectives and no BatchNorm statistics exchange."""
+        params = self._params_of("all")
+        if self._grad_wanted(x, [p for _, p in params]):
+            loss, z, x_rec = _LossFn.apply(self, x, noise, [n for n, _ in params], *[p for _, p in params])
         else:
             bufs = self._forward_native(x, noise, self.training, want_grad_seed=False)
             loss = bufs.loss[0].clone()
@@ -1437,26 +1523,171 @@ class VAE(nn.Module):
         return dev_latent.cpu().numpy().astype(np.float64)
 
 
-class _LossFn(torch.autograd.Function):
-    """Autograd glue: loss = VAE.forward(x) with the native backward pass."""
+class _Lease:
+    """An activation set checked out by a call that recorded an autograd graph (VAE._grad_buffers).
+    It goes back to the model's free list when the graph's backward has run (a second backward of
+    the same graph raises) or when the graph is freed without one."""
+
+    def __init__(self, model, bufs):
+        self.model, self.bufs = model, bufs
+
+    def release(self):
+        if self.bufs is not None:
+            self.model._release_grad_buffers(self.bufs)
+            self.bufs = None
+
+    __del__ = release
+
+
+def _checkout(ctx, model, B, train):
+    """Start of a recording forward: an owned activation set (running buffers snapshotted in eval
+    mode), made the model's current one."""
+    bufs = model._grad_buffers(B)
+    bufs.snapshot_running(model._flat_run, train)
+    ctx.lease = _Lease(model, bufs)
+    model._cur = bufs
+    model._scratch_need = model._scratch_need_for(B)
+    return bufs
+
+
+def _begin_backward(ctx):
+    bufs = ctx.lease.bufs
+    if bufs is None:
+        raise RuntimeError("ava_b200: this graph's backward has already run; its activations are released "
+                           "(a second backward through the same VAE call is not supported)")
+    ctx.lease.model._scratch_need = ctx.lease.model._scratch_need_for(bufs.B)
+    bufs.alloc_backward(ctx.lease.model.z_dim)
+    return ctx.lease.model, bufs
+
+
+def _param_grads(ctx, model, names, scale=None):
+    """The flat gradient buffer's entries for the call's parameters, copied out (the buffer is
+    shared with every other backward and with train_step); None where no gradient is wanted."""
+    out = []
+    for i, n in enumerate(names):          # (ctx.first: index of the first parameter among the inputs)
+        if not ctx.needs_input_grad[ctx.first + i]:
+            out.append(None)
+        else:
+            g = model._views_g[n]
+            out.append(g * scale if scale is not None else g.clone())
+    return tuple(out)
+
+
+class _EncodeFn(torch.autograd.Function):
+    """encode(x) -> (mu, u, d) with the native backward: latent_heads_grad, the dense encoder
+    backward and the conv encoder backward (+ layer 0's data gradient when x requires grad)."""
 
     @staticmethod
-    def forward(ctx, model, x, noise, *params):
-        if not model.training:
-            raise NotImplementedError("ava_b200: backward through eval-mode BatchNorm is not "
-                                      "implemented; call forward under torch.no_grad()")
-        bufs = model._forward_native(x, noise, True, want_grad_seed=True)
-        ctx.model, ctx.bufs = model, bufs
+    def forward(ctx, model, x, names, *params):
+        model._require_cuda()
+        ctx.x_meta = (x.device, x.dtype) if torch.is_tensor(x) else None
+        x = model._as_input(x)
+        B, Z, train = x.shape[0], model.z_dim, model.training
+        bufs = _checkout(ctx, model, B, train)
+        bufs.accum.zero_()
+        model._encode_native(x, bufs, train)
+        if train:
+            model._update_running(B, 0, 7)
+        model._linear(bufs.h3[:, 128:], 192, "fc43.weight", "fc43.bias", bufs.d, Z, B, Z, 64, 2)
+        bufs.x = x
+        ctx.names, ctx.first = names, 3
+        ctx.set_materialize_grads(False)
+        heads = bufs.heads
+        return heads[:, :Z].clone(), heads[:, Z:2 * Z].clone().unsqueeze(-1), bufs.d.clone()
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dmu, du, dd):
+        model, bufs = _begin_backward(ctx)
+        B, Z, s = bufs.B, model.z_dim, _stream()
+        seeds = [None if t is None else t.to(torch.float32).reshape(B, Z).contiguous() for t in (dmu, du, dd)]
+        bufs.dstats[:7 * 64].zero_()
+        bufs.tsums[:7 * 288].zero_()
+        call("ava_b200_latent_heads_grad", ptr(seeds[0]), ptr(seeds[1]), ptr(seeds[2]), ptr(bufs.d), B, Z,
+             ptr(bufs.gheads), s)
+        model._bwd_dense_encoder(bufs, latent=False)
+        dx = torch.empty_like(bufs.x) if ctx.needs_input_grad[1] else None
+        model._bwd_conv_encoder(bufs, dx=dx, n_bn=7)
+        model._side_join()
+        grads = _param_grads(ctx, model, ctx.names)
+        ctx.lease.release()
+        if dx is not None:
+            dx = dx.to(device=ctx.x_meta[0], dtype=ctx.x_meta[1])
+        return (None, dx, None) + grads
+
+
+class _DecodeFn(torch.autograd.Function):
+    """decode(z) -> x_rec [B,16384] with the native backward: the seed's border sums
+    (ava_b200_dz_border_sums) and the decoder backward, whose fc5 data gradient is dL/dz."""
+
+    @staticmethod
+    def forward(ctx, model, z, names, *params):
+        model._require_cuda()
+        ctx.z_meta = (z.device, z.dtype)
+        B, train = z.shape[0], model.training
+        bufs = _checkout(ctx, model, B, train)
+        bufs.z.copy_(z.detach().reshape(B, model.z_dim))      # fc5's input, kept for its weight gradient
+        bufs.accum.zero_()
+        model._decode_native(bufs.z, bufs, train)
+        if train:
+            model._update_running(B, 7, 14)
+        ctx.names, ctx.first = names, 3
+        ctx.set_materialize_grads(False)
+        return bufs.act[13].reshape(B, X_DIM).clone()
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, gx):
+        if gx is None:
+            ctx.lease.release()
+            return (None,) * (3 + len(ctx.names))
+        model, bufs = _begin_backward(ctx)
+        B, s = bufs.B, _stream()
+        bufs.dstats[7 * 64:].zero_()
+        bufs.tsums[7 * 288:].zero_()
+        seed = bufs.g[0][:B * X_DIM]          # convt7's dz (no ReLU after it): the seed itself
+        seed.copy_(gx.reshape(-1))
+        call("ava_b200_dz_border_sums", ptr(seed), B, 1, X_SHAPE[0], X_SHAPE[1], 0,
+             bufs.tsums.data_ptr() + 8 * 288 * 13, s)
+        model._bwd_decoder(bufs)
+        model._bn_param_grads(bufs, 7, 14)
+        model._side_join()
+        grads = _param_grads(ctx, model, ctx.names)
+        gz = bufs.gz.to(device=ctx.z_meta[0], dtype=ctx.z_meta[1], copy=True) if ctx.needs_input_grad[1] else None
+        ctx.lease.release()
+        return (None, gz, None) + grads
+
+
+class _LossFn(torch.autograd.Function):
+    """Autograd glue: loss = VAE.forward(x) with the native backward pass (train or eval mode;
+    the input gradient when x requires grad)."""
+
+    @staticmethod
+    def forward(ctx, model, x, noise, names, *params):
+        model._require_cuda()
+        ctx.x_meta = (x.device, x.dtype) if torch.is_tensor(x) else None
+        x = model._as_input(x)
+        train = model.training
+        bufs = _checkout(ctx, model, x.shape[0], train)
+        model._forward_native(x, noise, train, want_grad_seed=True, bufs=bufs)
+        ctx.names, ctx.first = names, 4
         ctx.mark_non_differentiable(bufs.z, bufs.act[13])
         return bufs.loss[0].clone(), bufs.z, bufs.act[13]
 
     @staticmethod
+    @torch.autograd.function.once_differentiable
     def backward(ctx, grad_loss, _gz, _gx):
-        model, bufs = ctx.model, ctx.bufs
-        model._backward_native(bufs)
-        names = [k for k, _ in model.named_parameters()]
-        grads = tuple(model._views_g[k] * grad_loss for k in names)
-        return (None, None, None) + grads
+        model, bufs = _begin_backward(ctx)
+        dx = torch.empty_like(bufs.x) if ctx.needs_input_grad[1] else None
+        model._backward_native(bufs, dx=dx)
+        if dx is not None:
+            # (the reconstruction seed in g[0] is gone by now: recomputed from x and x_rec)
+            call("ava_b200_recon_input_grad", ptr(dx), ptr(bufs.x), ptr(bufs.act[13]), bufs.B * X_DIM,
+                 float(model.model_precision), ptr(dx), _stream())
+            dx = (dx * grad_loss).to(device=ctx.x_meta[0], dtype=ctx.x_meta[1])
+        grads = _param_grads(ctx, model, ctx.names, scale=grad_loss)
+        ctx.lease.release()
+        return (None, dx, None, None) + grads
 
 
 if __name__ == '__main__':

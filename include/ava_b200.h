@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AVA_B200_ABI_VERSION 5
+#define AVA_B200_ABI_VERSION 6
 #define AVA_NUM_BN_LAYERS 14
 #define AVA_STATS_STRIDE 64 /* doubles per layer in a stats block: [0..31]=sum, [32..63]=sum of squares */
 
@@ -130,6 +130,17 @@ int ava_b200_bnconv_bwd_weight(int layer, int B, const float* dz, const float* x
                                const double* tsums, float* dw, float* db, double* dstats, void* ws,
                                void* stream);
 long long ava_b200_bnconv_bwd_weight_ws(int layer, int B);
+/* The same with the BatchNorm mode of the forward, as in ava_b200_bnconv_fwd: train != 0 is exactly
+ * ava_b200_bnconv_bwd_weight (running_mean / running_var unused).  train == 0: eval-mode BatchNorm,
+ * the fixed affine map of the running buffers (invstd_r = 1/sqrt(running_var + eps)); the kernels centre x
+ * at running_mean, so Rc = sum dz*(x - running_mean)_pad and
+ *    dw = gamma*invstd_r*Rc + beta*T_k,  dstats = (<w, T_k>, <w, Rc>) = (sum g, sum g*(x - running_mean)).
+ * stats_in is not read in eval mode (may be NULL). */
+int ava_b200_bnconv_bwd_weight_ex(int layer, int B, const float* dz, const float* x, const float* w,
+                                  const float* gamma, const float* beta, const double* stats_in,
+                                  const float* running_mean, const float* running_var, int train,
+                                  const double* tsums, float* dw, float* db, double* dstats, void* ws,
+                                  void* stream);
 
 /* gamma == NULL: no BatchNorm backward (dz_prev = [x > 0] * g).
  * tsums_prev (optional): the nine border sums of dz_prev -- layer-1's tsums block -- are accumulated
@@ -137,12 +148,27 @@ long long ava_b200_bnconv_bwd_weight_ws(int layer, int B);
 int ava_b200_bnconv_bwd_data(int layer, int B, const float* dz, const float* w, const float* x,
                              const float* gamma, const double* stats_in, const double* dstats, int relu_mask,
                              float* dz_prev, double* tsums_prev, void* stream);
+/* The same with the BatchNorm mode of the forward: train != 0 is exactly ava_b200_bnconv_bwd_data
+ * (running_var unused).  train == 0 (eval-mode BatchNorm): dz_prev = [x > 0] * gamma*invstd_r * g with
+ * invstd_r = 1/sqrt(running_var + eps); stats_in and dstats are not read (may be NULL). */
+int ava_b200_bnconv_bwd_data_ex(int layer, int B, const float* dz, const float* w, const float* x,
+                                const float* gamma, const double* stats_in, const float* running_var, int train,
+                                const double* dstats, int relu_mask, float* dz_prev, double* tsums_prev,
+                                void* stream);
 
 /* BN backward finalisation: dgamma[c] = invstd*dstats[32+c], dbeta[c] = dstats[c]
  * for all 14 layers (dstats[32+c] holds sum g*(x-mean)). */
 int ava_b200_bn_param_grads(const double* stats, const double* dstats, const int* h_channels,
                             const long long* h_counts, float* grads, const int* h_dgamma_off,
                             const int* h_dbeta_off, void* stream);
+/* The same with the BatchNorm mode of the forward: train != 0 is exactly ava_b200_bn_param_grads
+ * (running, h_rv_off unused).  train == 0: invstd from layer l's running variance at running[h_rv_off[l]]
+ * (element offsets, as in ava_b200_bn_update_running); dstats[32+c] then holds sum g*(x - running_mean).
+ * A layer with count 0 is skipped in both modes. */
+int ava_b200_bn_param_grads_ex(const double* stats, const double* dstats, const int* h_channels,
+                               const long long* h_counts, float* grads, const int* h_dgamma_off,
+                               const int* h_dbeta_off, const float* running, const int* h_rv_off, int train,
+                               void* stream);
 
 /* out = [a>0] * (p*(g - c1) + q*(a - mean)), per channel c = (i / HW) % C: the backward of
  * the BatchNorm that consumes `a` (train mode; fp64 coefficient math) followed by the ReLU
@@ -207,6 +233,16 @@ int ava_b200_latent_fwd(const float* heads, const float* eps_w, const float* eps
  * decoder (prior term z added here): analytic, SURVEY.md 8(a) "Analytic gradients". */
 int ava_b200_latent_bwd(const float* heads, const float* eps_w, const float* eps_d, const float* z,
                         const float* gz, int B, int Z, float* g_heads, void* stream);
+/* Backward seed of encode() (VAE.encode returns mu, u, d = exp(logd)): the gradient w.r.t. the heads
+ * g_heads [B, 3*Z] = (dmu | du | dd * d) from the seeds dmu, du, dd [B, Z] on encode's three outputs;
+ * a NULL seed counts as zero.  d: [B, Z] as the forward returned it (needed when dd != NULL). */
+int ava_b200_latent_heads_grad(const float* dmu, const float* du, const float* dd, const float* d, int B, int Z,
+                               float* g_heads, void* stream);
+/* Input gradient of the loss (VAE.forward with x.requires_grad): dx = dx_enc - precision * (x_rec - x),
+ * the encoder's part (layer 0's backward-data output; NULL counts as zero) plus the direct term of the
+ * reconstruction loss (ava/models/vae.py:319-320).  n % 4 == 0; dx may alias dx_enc. */
+int ava_b200_recon_input_grad(const float* dx_enc, const float* x, const float* x_rec, long long n, float precision,
+                              float* dx, void* stream);
 /* Reconstruction term (ava/models/vae.py:319-320): acc[1] += sum (x - x_rec)^2 and,
  * if g != NULL, g = precision * (x_rec - x) = dL/dx_rec.  tsums != NULL (with g): also the nine
  * border sums of g viewed as [n/(H*W)] single-channel H x W planes (mode 0 of
