@@ -28,6 +28,7 @@ struct SpecParams {
   int n_f;
   int max_frames;
   double spec_min, inv_range;
+  double fill;   // interp2d's fill value -1e12 after normalise + clip (0 unless spec_max < spec_min)
   float* out;
   double* out64;
 };
@@ -215,7 +216,7 @@ __global__ void __launch_bounds__(256) get_spec_kernel(const SpecParams P, const
     __syncthreads();
     // ---- output pass, row-major over [n_f, n_t]: the targets whose bracketing frames are the
     // entries (j, j+1) of this run with j + 1 < nrun; on the first run also everything that is
-    // out of range (fill value -> 0 after normalise + clip)
+    // out of range (the fill value after normalise + clip)
     // (a thread keeps its target times: slot and weight are looked up once per run, then it walks the
     // frequency rows; a warp's lanes are consecutive t of one row -> 128-byte coalesced stores)
     for (int t0 = 0; t0 < P.n_t; t0 += 128) {
@@ -234,7 +235,8 @@ __global__ void __launch_bounds__(256) get_spec_kernel(const SpecParams P, const
         double v = 0.0;
         bool write = false;
         if (!t_valid || fi < 0) {
-          write = first_run;                            // out of range: fill value -> 0 after normalise + clip
+          v = P.fill;                                   // out of range: fill value after normalise + clip
+          write = first_run;
         } else if (here) {
           const double wy = s_wy[f];
           const double s00 = lo[fi], s01 = hi[fi], s10 = lo[fi + 1], s11 = hi[fi + 1];
@@ -314,9 +316,10 @@ quantile_normalize_kernel(double* __restrict__ spec64, float* __restrict__ spec3
   const double t = pos - (double)lo;
   const double a = radix_select(v, m, lo, hist, s_state);
   const double b = radix_select(v, m, hi, hist, s_state);
-  // numpy.lib._function_base_impl._lerp: a + (b-a)*t, and b - (b-a)*(1-t) where t >= 0.5
+  // numpy.lib._function_base_impl._lerp: a + (b-a)*t, and b - (b-a)*(1-t) where t >= 0.5, each
+  // product rounded before the add (a contracted FMA rounds once and differs in the last bit)
   const double diff = b - a;
-  double qv = (t >= 0.5) ? b - diff * (1.0 - t) : a + diff * t;
+  double qv = (t >= 0.5) ? __dsub_rn(b, __dmul_rn(diff, 1.0 - t)) : __dadd_rn(a, __dmul_rn(diff, t));
   if (t == 0.0) qv = a;
   double mx = 0.0;
   for (int i = threadIdx.x; i < m; i += blockDim.x) {
@@ -424,6 +427,9 @@ extern "C" int ava_b200_get_spec_batch(const void* audio, int is_f32, const long
               "get_spec: nperseg=%d must be a power of two in [16,4096]", nperseg);
   AVA_REQUIRE(noverlap >= 0 && noverlap < nperseg, "get_spec: bad noverlap %d", noverlap);
   AVA_REQUIRE(spec_max != spec_min, "get_spec: spec_max_val == spec_min_val");
+  AVA_REQUIRE(is_f32 >= 0 && is_f32 <= 2, "get_spec: sample type %d (0 int16, 1 float32, 2 float64)", is_f32);
+  AVA_REQUIRE(n_f >= 1 && n_t >= 1, "get_spec: n_f=%d n_t=%d", n_f, n_t);
+  AVA_REQUIRE(out != nullptr || out64 != nullptr, "get_spec: no output (out and out64 both null)");
   if (n <= 0) return 0;
   SpecParams P;
   P.audio = audio;
@@ -446,6 +452,8 @@ extern "C" int ava_b200_get_spec_batch(const void* audio, int is_f32, const long
   P.max_frames = max_frames;
   P.spec_min = spec_min;
   P.inv_range = 1.0 / (spec_max - spec_min);
+  // ava/preprocessing/utils.py:99-104: fill value -1/EPSILON, then (x - min) / (max - min), clipped
+  P.fill = fmin(fmax((-1.0 / 1e-12 - spec_min) / (spec_max - spec_min), 0.0), 1.0);
   P.out = out;
   P.out64 = out64;
   // shared memory: G packed transforms (G*N ~ 2048 points), twiddles, CF log-spectrum slots within

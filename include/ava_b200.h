@@ -339,7 +339,8 @@ int ava_b200_bn_stats_exchange(const ava_b200_bn_sync_peers* h_peers, int rank, 
  *   window/scale: the analysis window [nperseg] (fp64) and 1/sum(window), computed by
  *               the host with the same scipy call the reference makes
  *   t_idx/t_frac [n,n_t]: lower frame index and weight of each target time;
- *               t_idx < 0 marks an out-of-range target (fill value -> 0 after clip)
+ *               t_idx < 0 marks an out-of-range target (the fill value -1e12 normalised and
+ *               clipped: 0, or 1 when spec_max < spec_min)
  *   f_idx/f_frac [n_f]: same for the target frequencies (shared by all windows)
  *   max_frames: upper bound on the number of STFT frames of any segment
  *   out: [n, n_f, n_t] fp32 (numpy_to_tensor's float32, ava/models/utils.py:444-446)
@@ -353,7 +354,10 @@ int ava_b200_get_spec_batch(const void* audio, int is_f32, const long long* seg_
 /* within_syll_normalize (ava/preprocessing/utils.py:106-109), per spectrogram of m = n_f*n_t values:
  *   spec -= np.quantile(spec, q); spec[spec < 0] = 0; spec /= spec.max() + 1e-12
  * in float64 on spec64 [n, m] in place (the quantile by an exact radix select + numpy's linear
- * interpolation); spec32 (optional) receives the float32 copy. */
+ * interpolation); spec32 (optional) receives the float32 copy.  The values must be >= 0 (the
+ * select orders them by bit pattern; -0.0 is read as +0.0), as get_spec's clipped output is.
+ * Bit-identical to numpy except for the sign of zero: every zero written is +0.0, where numpy
+ * keeps an input's -0.0 when the quantile is 0. */
 int ava_b200_quantile_normalize(double* spec64, float* spec32, int n, int m, double q, void* stream);
 
 /* Target-time tables of a batch of fixed-duration windows computed on the device (the
