@@ -54,6 +54,21 @@ SIGNATURES = {
     "ava_b200_pca_ws_bytes": (I,),
     "ava_b200_pca_fit": (P, I, LL, I, P, P, P, P, P, LL, P),
     "ava_b200_pca_transform": (P, I, LL, I, P, P, I, P, P),
+    "ava_b200_umap_knn_ws_bytes": (I, I),
+    "ava_b200_umap_knn": (P, I, I, I, I, P, P, P, LL, P),
+    "ava_b200_umap_smooth_knn": (P, P, I, I, D, P, P, P, P, P),
+    "ava_b200_umap_edge_keys": (P, I, I, P, P),
+    "ava_b200_umap_graph": (P, LL, I, P, P, I, P, P, P, P, P),
+    "ava_b200_umap_epochs_per_sample": (P, LL, P, I, D, P, P, P, P, P),
+    "ava_b200_umap_components_step": (P, P, I, P, P, P),
+    "ava_b200_umap_degree": (P, P, I, P, P),
+    "ava_b200_umap_spmm": (P, P, P, P, I, P, P, P, I, P, P),
+    "ava_b200_umap_gram_ws_bytes": (I, I),
+    "ava_b200_umap_gram": (P, I, P, I, I, P, P, LL, P),
+    "ava_b200_umap_combine": (P, I, P, I, I, P, P),
+    "ava_b200_umap_random": (ctypes.c_ulonglong, ctypes.c_ulonglong, LL, I, D, P, P),
+    "ava_b200_umap_init_layout": (P, P, D, I, I, P, P),
+    "ava_b200_umap_sgd_epoch": (P, I, I, P, P, P, P, P, P, LL, LL, I, D, D, D, D, ctypes.c_ulonglong, P),
     "ava_b200_last_error": (),
     "ava_b200_abi_version": (),
     "ava_b200_launch_count": (),
@@ -65,6 +80,8 @@ _RESTYPES = {
     "ava_b200_linear_ws_bytes": LL,
     "ava_b200_bias_grads_ws_bytes": LL,
     "ava_b200_pca_ws_bytes": LL,
+    "ava_b200_umap_knn_ws_bytes": LL,
+    "ava_b200_umap_gram_ws_bytes": LL,
 }
 # entry points whose int return value is a status code
 _STATUS = {n for n in SIGNATURES if n not in _RESTYPES and n not in ("ava_b200_abi_version", "ava_b200_get_conv_precision")}

@@ -1,0 +1,742 @@
+// UMAP of the latent means: the device stages of umap-learn 0.5's UMAP(metric='euclidean').fit_transform,
+// the projection the reference builds in ava/data/data_container.py (_make_latent_mean_umap_projection)
+// with umap.UMAP(n_components=2, n_neighbors=20, min_dist=0.1, metric='euclidean', random_state=42).
+//
+//   1. exact kNN (replaces umap.umap_.nearest_neighbors / NNDescent): brute force over all N^2 pairs.
+//      Pass 1, fp32: each thread owns one query row (in registers) and a sorted top-KP list (distances
+//      in registers, indices in a shared-memory column of its own); candidate rows stream through shared
+//      memory in tiles.  Squared distance in the difference form sum (x - y)^2.  KP >= k + 8 keeps a
+//      margin for fp32 near-ties; the query itself enters with distance -1, so it is always kept.
+//      Pass 2, fp64: a warp per query recomputes the KP candidates' distances from the input rows and
+//      ranks them by (distance, not-self, index); the first k are written.
+//      Cost: N^2 * D subtract + FMA pairs on the FP32 pipe (pass 1); pass 2 is O(N * KP * D).
+//   2. smooth_knn_dist + compute_membership_strengths (umap.umap_), one thread per row, fp64.
+//   3. the fuzzy union P = A + A^T - A.*A^T (umap.umap_.fuzzy_simplicial_set, set_op_mix_ratio = 1):
+//      the caller sorts and de-duplicates the directed-edge keys row * N + col (a sort is plumbing);
+//      the weights, row pointers and the SGD schedule (umap.umap_.make_epochs_per_sample, the set-up
+//      of umap.layouts.optimize_layout_euclidean) are computed here.
+//   4. spectral initialisation (umap.spectral.spectral_layout / multi_component_layout): connected
+//      components by min-label propagation, the normalised-Laplacian product of LOBPCG as a CSR SpMM
+//      (warp per row), fixed-order tall-skinny Gram and combination kernels, the final expansion,
+//      noise and per-axis rescale.
+//   5. the layout SGD (umap.layouts._optimize_layout_euclidean_single_epoch), one launch per epoch, one
+//      thread per edge, Hogwild updates of the shared fp32 embedding.
+//
+// Random numbers (negative samples, noise, random initialisations) come from a counter-based hash:
+// splitmix64 applied along the key (seed, stream, i, j), so every draw is a pure function of its key.
+// Every output of stages 1-4 is bitwise reproducible (no atomics in any sum); stage 5 is not, as
+// Hogwild updates race by design (umap-learn's parallel mode).
+#include <float.h>
+#include <limits.h>
+
+#include "common.cuh"
+
+namespace ava {
+
+// ------------------------------------------------------------------------------------------ hash
+__host__ __device__ __forceinline__ unsigned long long umap_mix(unsigned long long z) {
+  z += 0x9E3779B97F4A7C15ull;
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  return z ^ (z >> 31);
+}
+__host__ __device__ __forceinline__ unsigned long long umap_hash(unsigned long long seed, unsigned long long a,
+                                                                 unsigned long long b, unsigned long long c) {
+  return umap_mix(umap_mix(umap_mix(umap_mix(seed) ^ a) ^ b) ^ c);
+}
+// uniform in (0, 1): the top 53 bits, offset by half an ulp
+__device__ __forceinline__ double umap_unit(unsigned long long h) {
+  return ((double)(h >> 11) + 0.5) * (1.0 / 9007199254740992.0);
+}
+
+// ------------------------------------------------------------------------------------------ kNN
+constexpr int KNN_THREADS = 128;   // queries per CTA
+constexpr int KNN_TILE = 64;       // candidate rows per shared-memory tile
+
+template <typename T, int DP, int KP>
+__global__ void __launch_bounds__(KNN_THREADS, 1)
+knn_select_kernel(const T* __restrict__ x, int N, int D, int* __restrict__ cand) {
+  __shared__ __align__(16) float tile[KNN_TILE * DP];
+  extern __shared__ int sidx[];   // [KP][KNN_THREADS]
+  const int tid = threadIdx.x;
+  const int q = blockIdx.x * KNN_THREADS + tid;
+  float xq[DP];
+#pragma unroll
+  for (int d = 0; d < DP; ++d) xq[d] = (q < N && d < D) ? (float)x[(long long)q * D + d] : 0.f;
+  float dk[KP];
+#pragma unroll
+  for (int j = 0; j < KP; ++j) {
+    dk[j] = FLT_MAX;
+    sidx[j * KNN_THREADS + tid] = -1;
+  }
+  for (int c0 = 0; c0 < N; c0 += KNN_TILE) {
+    __syncthreads();
+    for (int e = tid; e < KNN_TILE * DP; e += KNN_THREADS) {
+      const int r = e / DP, d = e - r * DP;
+      tile[e] = (c0 + r < N && d < D) ? (float)x[(long long)(c0 + r) * D + d] : 0.f;
+    }
+    __syncthreads();
+    const int nc = min(KNN_TILE, N - c0);
+    for (int r = 0; r < nc; ++r) {
+      const float4* t4 = reinterpret_cast<const float4*>(tile + r * DP);
+      float s0 = 0.f, s1 = 0.f;
+#pragma unroll
+      for (int d4 = 0; d4 < DP / 4; ++d4) {
+        const float4 v = t4[d4];
+        const float e0 = xq[4 * d4] - v.x, e1 = xq[4 * d4 + 1] - v.y;
+        const float e2 = xq[4 * d4 + 2] - v.z, e3 = xq[4 * d4 + 3] - v.w;
+        s0 = fmaf(e0, e0, s0);
+        s1 = fmaf(e1, e1, s1);
+        s0 = fmaf(e2, e2, s0);
+        s1 = fmaf(e3, e3, s1);
+      }
+      const int c = c0 + r;
+      const float dist = (c == q) ? -1.f : s0 + s1;
+      if (dist < dk[KP - 1]) {
+#pragma unroll
+        for (int j = KP - 1; j > 0; --j) {
+          if (dist < dk[j - 1]) {
+            dk[j] = dk[j - 1];
+            sidx[j * KNN_THREADS + tid] = sidx[(j - 1) * KNN_THREADS + tid];
+          } else if (dist < dk[j]) {
+            dk[j] = dist;
+            sidx[j * KNN_THREADS + tid] = c;
+          }
+        }
+        if (dist < dk[0]) {
+          dk[0] = dist;
+          sidx[tid] = c;
+        }
+      }
+    }
+  }
+  if (q < N)
+    for (int j = 0; j < KP; ++j) cand[(long long)q * KP + j] = sidx[j * KNN_THREADS + tid];
+}
+
+// one warp per query: fp64 distances of the KP candidates, ranked by (distance, not-self, index)
+template <typename T>
+__global__ void knn_refine_kernel(const T* __restrict__ x, int N, int D, int KP, int k, const int* __restrict__ cand,
+                                  int* __restrict__ knn_idx, double* __restrict__ knn_dist) {
+  extern __shared__ double sref[];
+  const int warps = blockDim.x / 32, w = threadIdx.x / 32, lane = threadIdx.x % 32;
+  double* sd = sref + w * KP;
+  int* si = reinterpret_cast<int*>(sref + warps * KP) + w * KP;
+  const int q = blockIdx.x * warps + w;
+  if (q >= N) return;
+  for (int j = lane; j < KP; j += 32) {
+    const int c = cand[(long long)q * KP + j];
+    double s = INFINITY;
+    if (c >= 0) {
+      s = 0.0;
+      for (int d = 0; d < D; ++d) {
+        const double e = (double)x[(long long)q * D + d] - (double)x[(long long)c * D + d];
+        s = __fma_rn(e, e, s);
+      }
+    }
+    sd[j] = s;
+    si[j] = c;
+  }
+  __syncwarp();
+  for (int j = lane; j < KP; j += 32) {
+    const int c = si[j];
+    if (c < 0) continue;
+    const double dj = sd[j];
+    const int kj = (c == q) ? -1 : c;
+    int rank = 0;
+    for (int i = 0; i < KP; ++i) {
+      const int ci = si[i];
+      if (ci < 0) continue;
+      const double di = sd[i];
+      const int ki = (ci == q) ? -1 : ci;
+      rank += (di < dj) || (di == dj && ki < kj);
+    }
+    if (rank < k) {
+      knn_idx[(long long)q * k + rank] = c;
+      knn_dist[(long long)q * k + rank] = sqrt(dj);
+    }
+  }
+}
+
+static int knn_padded(int k) {
+  for (int kp : {16, 32, 64, 128})
+    if (kp >= k + 8 || kp == 128) return kp;
+  return 128;
+}
+static int knn_dpad(int D) {
+  for (int dp : {8, 16, 32, 64})
+    if (dp >= D) return dp;
+  return -1;
+}
+
+template <typename T, int DP, int KP>
+static int knn_launch(const T* x, int N, int D, int* cand, cudaStream_t s) {
+  const size_t smem = (size_t)KP * KNN_THREADS * sizeof(int);
+  auto kern = knn_select_kernel<T, DP, KP>;
+  if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  kern<<<(N + KNN_THREADS - 1) / KNN_THREADS, KNN_THREADS, smem, s>>>(x, N, D, cand);
+  return check_launch("umap knn_select_kernel");
+}
+
+template <typename T, int DP>
+static int knn_launch_k(const T* x, int N, int D, int KP, int* cand, cudaStream_t s) {
+  switch (KP) {
+    case 16: return knn_launch<T, DP, 16>(x, N, D, cand, s);
+    case 32: return knn_launch<T, DP, 32>(x, N, D, cand, s);
+    case 64: return knn_launch<T, DP, 64>(x, N, D, cand, s);
+    default: return knn_launch<T, DP, 128>(x, N, D, cand, s);
+  }
+}
+
+template <typename T>
+static int knn_run(const T* x, int N, int D, int k, int* knn_idx, double* knn_dist, int* cand, cudaStream_t s) {
+  const int KP = knn_padded(k);
+  int rc;
+  switch (knn_dpad(D)) {
+    case 8: rc = knn_launch_k<T, 8>(x, N, D, KP, cand, s); break;
+    case 16: rc = knn_launch_k<T, 16>(x, N, D, KP, cand, s); break;
+    case 32: rc = knn_launch_k<T, 32>(x, N, D, KP, cand, s); break;
+    default: rc = knn_launch_k<T, 64>(x, N, D, KP, cand, s); break;
+  }
+  if (rc) return rc;
+  constexpr int WARPS = 8;
+  const size_t smem = (size_t)WARPS * KP * (sizeof(double) + sizeof(int));
+  knn_refine_kernel<T><<<(N + WARPS - 1) / WARPS, WARPS * 32, smem, s>>>(x, N, D, KP, k, cand, knn_idx, knn_dist);
+  return check_launch("umap knn_refine_kernel");
+}
+
+// --------------------------------------------------------------------- smooth kNN, memberships
+constexpr int SMOOTH_N_ITER = 64;
+constexpr double SMOOTH_K_TOLERANCE = 1e-5;
+constexpr double MIN_K_DIST_SCALE = 1e-3;
+
+// fixed-order mean of all N*k distances (one CTA)
+__global__ void mean_kernel(const double* __restrict__ v, long long n, double* __restrict__ out) {
+  __shared__ double red[1024];
+  double s = 0.0;
+  for (long long i = threadIdx.x; i < n; i += blockDim.x) s += v[i];
+  red[threadIdx.x] = s;
+  __syncthreads();
+  for (int o = blockDim.x / 2; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) *out = red[0] / (double)n;
+}
+
+__global__ void smooth_knn_kernel(const int* __restrict__ knn_idx, const double* __restrict__ knn_dist, int N, int k,
+                                  double local_connectivity, const double* __restrict__ mean_all,
+                                  double* __restrict__ rho_out, double* __restrict__ sigma_out,
+                                  double* __restrict__ w) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  const double* di = knn_dist + (long long)i * k;
+  const double target = log2((double)k);
+  // rho: the local_connectivity-th nonzero distance (interpolated), or the largest if there are fewer
+  int n_nz = 0;
+  double last_nz = 0.0, row_sum = 0.0;
+  for (int j = 0; j < k; ++j) {
+    row_sum += di[j];
+    if (di[j] > 0.0) {
+      ++n_nz;
+      last_nz = di[j];
+    }
+  }
+  double rho = 0.0;
+  if ((double)n_nz >= local_connectivity) {
+    const int index = (int)floor(local_connectivity);
+    const double interpolation = local_connectivity - index;
+    int seen = 0;
+    double nz_prev = 0.0, nz_at = 0.0, nz_first = 0.0;
+    for (int j = 0; j < k; ++j)
+      if (di[j] > 0.0) {
+        if (seen == 0) nz_first = di[j];
+        if (seen == index - 1) nz_prev = di[j];
+        if (seen == index) nz_at = di[j];
+        ++seen;
+      }
+    if (index > 0) {
+      rho = nz_prev;
+      if (interpolation > SMOOTH_K_TOLERANCE) rho += interpolation * (nz_at - nz_prev);
+    } else {
+      rho = interpolation * nz_first;
+    }
+  } else if (n_nz > 0) {
+    rho = last_nz;   // distances are sorted: the last nonzero one is the largest
+  }
+  double lo = 0.0, hi = INFINITY, mid = 1.0;
+  for (int it = 0; it < SMOOTH_N_ITER; ++it) {
+    double psum = 0.0;
+    for (int j = 1; j < k; ++j) {
+      const double d = di[j] - rho;
+      psum += d > 0.0 ? exp(-(d / mid)) : 1.0;
+    }
+    if (fabs(psum - target) < SMOOTH_K_TOLERANCE) break;
+    if (psum > target) {
+      hi = mid;
+      mid = (lo + hi) / 2.0;
+    } else {
+      lo = mid;
+      if (hi == INFINITY) mid *= 2.0;
+      else mid = (lo + hi) / 2.0;
+    }
+  }
+  double sigma = mid;
+  const double floor_ref = rho > 0.0 ? row_sum / (double)k : *mean_all;
+  if (sigma < MIN_K_DIST_SCALE * floor_ref) sigma = MIN_K_DIST_SCALE * floor_ref;
+  rho_out[i] = rho;
+  sigma_out[i] = sigma;
+  for (int j = 0; j < k; ++j) {
+    const int c = knn_idx[(long long)i * k + j];
+    double v;
+    if (c == i) v = 0.0;
+    else if (di[j] - rho <= 0.0 || sigma == 0.0) v = 1.0;
+    else v = exp(-((di[j] - rho) / sigma));
+    w[(long long)i * k + j] = v;
+  }
+}
+
+// ------------------------------------------------------------------------------- fuzzy union
+// directed-edge keys: (i, j) and (j, i) for every neighbour j != i of i; -1 for the self entries
+__global__ void edge_keys_kernel(const int* __restrict__ knn_idx, int N, int k, long long* __restrict__ keys) {
+  const long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (e >= (long long)N * k) return;
+  const long long i = e / k;
+  const long long j = knn_idx[e];
+  keys[2 * e] = (j == i) ? -1 : i * N + j;
+  keys[2 * e + 1] = (j == i) ? -1 : j * N + i;
+}
+
+__device__ __forceinline__ double knn_weight(const int* __restrict__ knn_idx, const double* __restrict__ w, int k,
+                                             long long r, int c) {
+  const int* row = knn_idx + r * k;
+  for (int j = 0; j < k; ++j)
+    if (row[j] == c) return w[r * k + j];
+  return 0.0;
+}
+
+// keys: sorted, unique, non-negative.  P[r, c] = a + b - a*b with a = A[r, c], b = A[c, r]; rowptr[N + 1].
+__global__ void graph_weights_kernel(const long long* __restrict__ keys, long long nnz, int N,
+                                     const int* __restrict__ knn_idx, const double* __restrict__ w, int k,
+                                     int* __restrict__ rows, int* __restrict__ cols, double* __restrict__ vals,
+                                     long long* __restrict__ rowptr) {
+  const long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (p > nnz) return;
+  if (p == nnz) {
+    const long long last = nnz > 0 ? keys[nnz - 1] / N : -1;
+    for (long long r = last + 1; r <= N; ++r) rowptr[r] = nnz;
+    return;
+  }
+  const long long key = keys[p];
+  const long long r = key / N;
+  const int c = (int)(key - r * N);
+  const long long prev = p > 0 ? keys[p - 1] / N : -1;
+  for (long long rr = prev + 1; rr <= r; ++rr) rowptr[rr] = p;
+  const double a = knn_weight(knn_idx, w, k, r, c);
+  const double b = knn_weight(knn_idx, w, k, c, (int)r);
+  rows[p] = (int)r;
+  cols[p] = c;
+  vals[p] = a + b - a * b;
+}
+
+__global__ void epochs_per_sample_kernel(const double* __restrict__ vals, long long n, const double* __restrict__ vmax,
+                                         int n_epochs, double negative_sample_rate, double* __restrict__ eps,
+                                         double* __restrict__ eps_neg, double* __restrict__ next,
+                                         double* __restrict__ next_neg) {
+  const long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (e >= n) return;
+  const double ns = (double)n_epochs * (vals[e] / *vmax);
+  const double r = ns > 0.0 ? (double)n_epochs / ns : -1.0;
+  const double rn = r / negative_sample_rate;
+  eps[e] = r;
+  eps_neg[e] = rn;
+  next[e] = r;
+  next_neg[e] = rn;
+}
+
+// ---------------------------------------------------------------------- connected components
+// one round of min-label hooking; labels only decrease and always name a vertex of the same component
+__global__ void components_kernel(const long long* __restrict__ rowptr, const int* __restrict__ cols, int N,
+                                  int* __restrict__ label, int* __restrict__ changed) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  const int l = label[i];
+  int m = label[l];
+  for (long long p = rowptr[i]; p < rowptr[i + 1]; ++p) m = min(m, label[cols[p]]);
+  if (m < l) {
+    atomicMin(&label[i], m);
+    atomicMin(&label[l], m);
+    *changed = 1;
+  }
+}
+
+// ------------------------------------------------------------------------- spectral kernels
+// dis[i] = 1/sqrt(sum_j P[i, j])
+__global__ void degree_kernel(const long long* __restrict__ rowptr, const double* __restrict__ vals, int N,
+                              double* __restrict__ dis) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= N) return;
+  double s = 0.0;
+  for (long long p = rowptr[i]; p < rowptr[i + 1]; ++p) s += vals[p];
+  dis[i] = 1.0 / sqrt(s);
+}
+
+// Y[r, :] = X[r, :] - dis[v] * sum_j P[v, j] * dis[j] * X[pos[j], :] for v = verts[r]: the normalised
+// Laplacian I - D^-1/2 P D^-1/2 of the component whose vertices verts lists (pos: vertex -> row).
+// A warp per row; lanes stride the row's entries, then a fixed butterfly sums the lanes.
+template <int MM>
+__global__ void spmm_kernel(const long long* __restrict__ rowptr, const int* __restrict__ cols,
+                            const double* __restrict__ vals, const int* __restrict__ verts, int n,
+                            const int* __restrict__ pos, const double* __restrict__ dis, const double* __restrict__ X,
+                            int m, double* __restrict__ Y) {
+  const int r = blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32;
+  const int lane = threadIdx.x % 32;
+  if (r >= n) return;
+  const int v = verts[r];
+  double acc[MM];
+#pragma unroll
+  for (int c = 0; c < MM; ++c) acc[c] = 0.0;
+  for (long long p = rowptr[v] + lane; p < rowptr[v + 1]; p += 32) {
+    const int j = cols[p];
+    const double f = vals[p] * dis[j];
+    const double* xj = X + (long long)pos[j] * m;
+#pragma unroll
+    for (int c = 0; c < MM; ++c)
+      if (c < m) acc[c] = fma(f, xj[c], acc[c]);
+  }
+#pragma unroll
+  for (int c = 0; c < MM; ++c) {
+    const double s = warp_sum(acc[c]);
+    if (lane == c && c < m) Y[(long long)r * m + c] = X[(long long)r * m + c] - dis[v] * s;
+  }
+}
+
+// out[p, q] = A^T B for A [n, p], B [n, q] row-major: CTA g sums the rows of its contiguous chunk into
+// partial[g]; gram_finish adds the partials in CTA order.
+constexpr int GRAM_THREADS = 256;
+constexpr int GRAM_CTAS = 2 * kNumSMs;
+constexpr int GRAM_ROWS = 32;
+__global__ void __launch_bounds__(GRAM_THREADS)
+gram_kernel(const double* __restrict__ A, int p, const double* __restrict__ B, int q, int n,
+            double* __restrict__ partial) {
+  extern __shared__ double sg[];
+  double* sa = sg;
+  double* sb = sg + GRAM_ROWS * p;
+  const int outs = p * q;
+  const int per = (n + gridDim.x - 1) / gridDim.x;
+  const int r0 = blockIdx.x * per, r1 = min(n, r0 + per);
+  double acc[8];
+#pragma unroll
+  for (int t = 0; t < 8; ++t) acc[t] = 0.0;
+  for (int t0 = r0; t0 < r1; t0 += GRAM_ROWS) {
+    const int nr = min(GRAM_ROWS, r1 - t0);
+    __syncthreads();
+    for (int e = threadIdx.x; e < nr * p; e += blockDim.x) sa[e] = A[(long long)t0 * p + e];
+    for (int e = threadIdx.x; e < nr * q; e += blockDim.x) sb[e] = B[(long long)t0 * q + e];
+    __syncthreads();
+#pragma unroll
+    for (int t = 0; t < 8; ++t) {
+      const int o = threadIdx.x + t * GRAM_THREADS;
+      if (o < outs) {
+        const int i = o / q, j = o - i * q;
+        double s = acc[t];
+        for (int rr = 0; rr < nr; ++rr) s = fma(sa[rr * p + i], sb[rr * q + j], s);
+        acc[t] = s;
+      }
+    }
+  }
+#pragma unroll
+  for (int t = 0; t < 8; ++t) {
+    const int o = threadIdx.x + t * GRAM_THREADS;
+    if (o < outs) partial[(long long)blockIdx.x * outs + o] = acc[t];
+  }
+}
+__global__ void gram_finish_kernel(const double* __restrict__ partial, int outs, int ctas, double* __restrict__ out) {
+  const int o = blockIdx.x * blockDim.x + threadIdx.x;
+  if (o >= outs) return;
+  double s = 0.0;
+  for (int g = 0; g < ctas; ++g) s += partial[(long long)g * outs + o];
+  out[o] = s;
+}
+
+// Y[n, q] = A[n, p] . C[p, q]
+__global__ void combine_kernel(const double* __restrict__ A, int p, const double* __restrict__ C, int q, int n,
+                               double* __restrict__ Y) {
+  const long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (e >= (long long)n * q) return;
+  const long long r = e / q;
+  const int j = (int)(e - r * q);
+  double s = 0.0;
+  for (int i = 0; i < p; ++i) s = fma(A[r * p + i], C[(long long)i * q + j], s);
+  Y[e] = s;
+}
+
+// kind 0: uniform(-scale, scale); kind 1: normal(0, scale) (Box-Muller on two hashed uniforms)
+__global__ void random_kernel(unsigned long long seed, unsigned long long stream_id, long long n, int kind,
+                              double scale, double* __restrict__ out) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double u1 = umap_unit(umap_hash(seed, stream_id, (unsigned long long)i, 0));
+  if (kind == 0) {
+    out[i] = scale * (2.0 * u1 - 1.0);
+  } else {
+    const double u2 = umap_unit(umap_hash(seed, stream_id, (unsigned long long)i, 1));
+    out[i] = scale * sqrt(-2.0 * log(u1)) * cos(6.283185307179586 * u2);
+  }
+}
+
+// one CTA per axis: v = (float)(init * expansion) + (float)noise, then 10 * (v - min) / (max - min)
+__global__ void init_layout_kernel(const double* __restrict__ init, const double* __restrict__ noise,
+                                   double expansion, int N, int dim, float* __restrict__ emb) {
+  __shared__ float smin[1024], smax[1024];
+  const int d = blockIdx.x;
+  auto val = [&](long long i) {
+    float v = (float)(init[i * dim + d] * expansion);
+    if (noise) v = __fadd_rn(v, (float)noise[i * dim + d]);
+    return v;
+  };
+  float lo = FLT_MAX, hi = -FLT_MAX;
+  for (long long i = threadIdx.x; i < N; i += blockDim.x) {
+    const float v = val(i);
+    lo = fminf(lo, v);
+    hi = fmaxf(hi, v);
+  }
+  smin[threadIdx.x] = lo;
+  smax[threadIdx.x] = hi;
+  __syncthreads();
+  for (int o = blockDim.x / 2; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) {
+      smin[threadIdx.x] = fminf(smin[threadIdx.x], smin[threadIdx.x + o]);
+      smax[threadIdx.x] = fmaxf(smax[threadIdx.x], smax[threadIdx.x + o]);
+    }
+    __syncthreads();
+  }
+  const float mn = smin[0], range = __fsub_rn(smax[0], smin[0]);
+  for (long long i = threadIdx.x; i < N; i += blockDim.x)
+    emb[i * dim + d] = range > 0.f ? __fdiv_rn(__fmul_rn(10.f, __fsub_rn(val(i), mn)), range) : 0.f;
+}
+
+// --------------------------------------------------------------------------------- layout SGD
+constexpr int UMAP_MAX_DIM = 8;
+
+__device__ __forceinline__ double umap_clip(double v) { return v > 4.0 ? 4.0 : (v < -4.0 ? -4.0 : v); }
+
+__global__ void sgd_epoch_kernel(float* __restrict__ emb, int N, int dim, const int* __restrict__ head,
+                                 const int* __restrict__ tail, const double* __restrict__ eps,
+                                 const double* __restrict__ eps_neg, double* __restrict__ next,
+                                 double* __restrict__ next_neg, long long e0, long long e1, int epoch, double a,
+                                 double b, double gamma, double alpha, unsigned long long seed) {
+  const long long e = e0 + blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (e >= e1) return;
+  const double nxt = next[e];
+  if (!(nxt <= (double)epoch)) return;
+  const int j = head[e], kk = tail[e];
+  float cur[UMAP_MAX_DIM], oth[UMAP_MAX_DIM];
+  volatile float* ve = emb;   // Hogwild: re-read what other threads wrote
+  double d2 = 0.0;
+  #pragma unroll
+  for (int d = 0; d < UMAP_MAX_DIM; ++d) {
+    if (d >= dim) break;
+    cur[d] = ve[(long long)j * dim + d];
+    oth[d] = ve[(long long)kk * dim + d];
+    const double t = (double)cur[d] - (double)oth[d];
+    d2 = __dadd_rn(d2, __dmul_rn(t, t));
+  }
+  double gc = 0.0;
+  if (d2 > 0.0) gc = (-2.0 * a * b * pow(d2, b - 1.0)) / (a * pow(d2, b) + 1.0);
+  #pragma unroll
+  for (int d = 0; d < UMAP_MAX_DIM; ++d) {
+    if (d >= dim) break;
+    const double g = umap_clip(gc * ((double)cur[d] - (double)oth[d]));
+    const float c_new = (float)__dadd_rn((double)cur[d], __dmul_rn(g, alpha));
+    const float o_new = (float)__dadd_rn((double)oth[d], __dmul_rn(-g, alpha));
+    cur[d] = c_new;
+    oth[d] = o_new;
+    ve[(long long)j * dim + d] = c_new;
+    ve[(long long)kk * dim + d] = o_new;
+  }
+  next[e] = nxt + eps[e];
+  const double en = eps_neg[e];
+  const int n_neg = (int)(((double)epoch - next_neg[e]) / en);
+  for (int p = 0; p < n_neg; ++p) {
+    const int k = (int)(umap_hash(seed, (unsigned long long)epoch, (unsigned long long)e, (unsigned long long)p) %
+                        (unsigned long long)N);
+    if (k == j) continue;
+    double s = 0.0;
+    #pragma unroll
+  for (int d = 0; d < UMAP_MAX_DIM; ++d) {
+    if (d >= dim) break;
+      oth[d] = ve[(long long)k * dim + d];
+      const double t = (double)cur[d] - (double)oth[d];
+      s = __dadd_rn(s, __dmul_rn(t, t));
+    }
+    double rc = 0.0;
+    if (s > 0.0) rc = (2.0 * gamma * b) / ((0.001 + s) * (a * pow(s, b) + 1.0));
+    #pragma unroll
+  for (int d = 0; d < UMAP_MAX_DIM; ++d) {
+    if (d >= dim) break;
+      const double g = rc > 0.0 ? umap_clip(rc * ((double)cur[d] - (double)oth[d])) : 4.0;
+      cur[d] = (float)__dadd_rn((double)cur[d], __dmul_rn(g, alpha));
+      ve[(long long)j * dim + d] = cur[d];
+    }
+  }
+  next_neg[e] = next_neg[e] + (double)n_neg * en;
+}
+
+}  // namespace ava
+
+using namespace ava;
+
+#define UMAP_STREAM cudaStream_t s = (cudaStream_t)stream
+
+extern "C" long long ava_b200_umap_knn_ws_bytes(int N, int k) {
+  if (N < 1 || k < 1 || k > 100) return -1;
+  return (long long)N * knn_padded(k) * (long long)sizeof(int);
+}
+
+extern "C" int ava_b200_umap_knn(const void* x, int is_f32, int N, int D, int k, int* knn_idx, double* knn_dist,
+                                 void* ws, long long ws_bytes, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(x && knn_idx && knn_dist && ws, "umap_knn: null pointer");
+  AVA_REQUIRE(N >= 1 && k >= 1 && k <= 100 && k <= N, "umap_knn: need 1 <= k <= min(N, 100), got N=%d k=%d", N, k);
+  AVA_REQUIRE(D >= 1 && D <= 64, "umap_knn: D=%d outside 1..64", D);
+  AVA_REQUIRE(is_f32 == 0 || is_f32 == 1, "umap_knn: is_f32 must be 0 or 1");
+  AVA_REQUIRE(ws_bytes >= ava_b200_umap_knn_ws_bytes(N, k), "umap_knn: workspace too small");
+  if (is_f32)
+    return knn_run<float>((const float*)x, N, D, k, knn_idx, knn_dist, (int*)ws, s);
+  return knn_run<double>((const double*)x, N, D, k, knn_idx, knn_dist, (int*)ws, s);
+}
+
+extern "C" int ava_b200_umap_smooth_knn(const int* knn_idx, const double* knn_dist, int N, int k,
+                                        double local_connectivity, double* rho, double* sigma, double* weights,
+                                        double* ws, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(knn_idx && knn_dist && rho && sigma && weights && ws, "umap_smooth_knn: null pointer");
+  AVA_REQUIRE(N >= 1 && k >= 2, "umap_smooth_knn: need N >= 1 and k >= 2");
+  AVA_REQUIRE(local_connectivity >= 0.0 && local_connectivity <= k - 1,
+              "umap_smooth_knn: local_connectivity outside 0..k-1");
+  mean_kernel<<<1, 1024, 0, s>>>(knn_dist, (long long)N * k, ws);
+  if (check_launch("umap mean_kernel")) return 1;
+  smooth_knn_kernel<<<(N + 127) / 128, 128, 0, s>>>(knn_idx, knn_dist, N, k, local_connectivity, ws, rho, sigma,
+                                                    weights);
+  return check_launch("umap smooth_knn_kernel");
+}
+
+extern "C" int ava_b200_umap_edge_keys(const int* knn_idx, int N, int k, long long* keys, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(knn_idx && keys && N >= 1 && k >= 1, "umap_edge_keys: bad arguments");
+  const long long n = (long long)N * k;
+  edge_keys_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(knn_idx, N, k, keys);
+  return check_launch("umap edge_keys_kernel");
+}
+
+extern "C" int ava_b200_umap_graph(const long long* keys, long long nnz, int N, const int* knn_idx,
+                                   const double* weights, int k, int* rows, int* cols, double* vals,
+                                   long long* rowptr, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(keys && knn_idx && weights && rows && cols && vals && rowptr, "umap_graph: null pointer");
+  AVA_REQUIRE(N >= 1 && k >= 1 && nnz >= 0, "umap_graph: bad sizes");
+  graph_weights_kernel<<<(unsigned)((nnz + 1 + 255) / 256), 256, 0, s>>>(keys, nnz, N, knn_idx, weights, k, rows,
+                                                                       cols, vals, rowptr);
+  return check_launch("umap graph_weights_kernel");
+}
+
+extern "C" int ava_b200_umap_epochs_per_sample(const double* vals, long long n, const double* vmax, int n_epochs,
+                                               double negative_sample_rate, double* eps, double* eps_neg,
+                                               double* next, double* next_neg, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(vals && vmax && eps && eps_neg && next && next_neg, "umap_epochs_per_sample: null pointer");
+  AVA_REQUIRE(n >= 0 && n_epochs >= 1 && negative_sample_rate > 0.0, "umap_epochs_per_sample: bad arguments");
+  if (n == 0) return 0;
+  epochs_per_sample_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(vals, n, vmax, n_epochs, negative_sample_rate,
+                                                                     eps, eps_neg, next, next_neg);
+  return check_launch("umap epochs_per_sample_kernel");
+}
+
+extern "C" int ava_b200_umap_components_step(const long long* rowptr, const int* cols, int N, int* labels,
+                                             int* changed, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(rowptr && cols && labels && changed && N >= 1, "umap_components_step: bad arguments");
+  components_kernel<<<(N + 255) / 256, 256, 0, s>>>(rowptr, cols, N, labels, changed);
+  return check_launch("umap components_kernel");
+}
+
+extern "C" int ava_b200_umap_degree(const long long* rowptr, const double* vals, int N, double* dis, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(rowptr && vals && dis && N >= 1, "umap_degree: bad arguments");
+  degree_kernel<<<(N + 255) / 256, 256, 0, s>>>(rowptr, vals, N, dis);
+  return check_launch("umap degree_kernel");
+}
+
+extern "C" int ava_b200_umap_spmm(const long long* rowptr, const int* cols, const double* vals, const int* verts,
+                                  int n, const int* pos, const double* dis, const double* X, int m, double* Y,
+                                  void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(rowptr && cols && vals && verts && pos && dis && X && Y, "umap_spmm: null pointer");
+  AVA_REQUIRE(n >= 1 && m >= 1 && m <= 32, "umap_spmm: need n >= 1 and 1 <= m <= 32");
+  constexpr int WARPS = 8;
+  const unsigned grid = (unsigned)((n + WARPS - 1) / WARPS);
+  if (m <= 8) spmm_kernel<8><<<grid, WARPS * 32, 0, s>>>(rowptr, cols, vals, verts, n, pos, dis, X, m, Y);
+  else if (m <= 16) spmm_kernel<16><<<grid, WARPS * 32, 0, s>>>(rowptr, cols, vals, verts, n, pos, dis, X, m, Y);
+  else spmm_kernel<32><<<grid, WARPS * 32, 0, s>>>(rowptr, cols, vals, verts, n, pos, dis, X, m, Y);
+  return check_launch("umap spmm_kernel");
+}
+
+extern "C" long long ava_b200_umap_gram_ws_bytes(int p, int q) {
+  if (p < 1 || q < 1 || p * q > 8 * GRAM_THREADS) return -1;
+  return (long long)GRAM_CTAS * p * q * (long long)sizeof(double);
+}
+
+extern "C" int ava_b200_umap_gram(const double* A, int p, const double* B, int q, int n, double* out, void* ws,
+                                  long long ws_bytes, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(A && B && out && ws, "umap_gram: null pointer");
+  AVA_REQUIRE(n >= 1 && p >= 1 && q >= 1 && p * q <= 8 * GRAM_THREADS, "umap_gram: need p*q <= %d",
+              8 * GRAM_THREADS);
+  AVA_REQUIRE(ws_bytes >= ava_b200_umap_gram_ws_bytes(p, q), "umap_gram: workspace too small");
+  const size_t smem = (size_t)GRAM_ROWS * (p + q) * sizeof(double);
+  gram_kernel<<<GRAM_CTAS, GRAM_THREADS, smem, s>>>(A, p, B, q, n, (double*)ws);
+  if (check_launch("umap gram_kernel")) return 1;
+  gram_finish_kernel<<<(p * q + 255) / 256, 256, 0, s>>>((const double*)ws, p * q, GRAM_CTAS, out);
+  return check_launch("umap gram_finish_kernel");
+}
+
+extern "C" int ava_b200_umap_combine(const double* A, int p, const double* C, int q, int n, double* Y, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(A && C && Y && n >= 1 && p >= 1 && q >= 1, "umap_combine: bad arguments");
+  const long long t = (long long)n * q;
+  combine_kernel<<<(unsigned)((t + 255) / 256), 256, 0, s>>>(A, p, C, q, n, Y);
+  return check_launch("umap combine_kernel");
+}
+
+extern "C" int ava_b200_umap_random(unsigned long long seed, unsigned long long stream_id, long long n, int kind,
+                                    double scale, double* out, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(out && n >= 0 && (kind == 0 || kind == 1), "umap_random: bad arguments");
+  if (n == 0) return 0;
+  random_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(seed, stream_id, n, kind, scale, out);
+  return check_launch("umap random_kernel");
+}
+
+extern "C" int ava_b200_umap_init_layout(const double* init, const double* noise, double expansion, int N, int dim,
+                                         float* emb, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(init && emb && N >= 1 && dim >= 1 && dim <= UMAP_MAX_DIM, "umap_init_layout: bad arguments");
+  init_layout_kernel<<<dim, 1024, 0, s>>>(init, noise, expansion, N, dim, emb);
+  return check_launch("umap init_layout_kernel");
+}
+
+extern "C" int ava_b200_umap_sgd_epoch(float* emb, int N, int dim, const int* head, const int* tail,
+                                       const double* eps, const double* eps_neg, double* next, double* next_neg,
+                                       long long e0, long long e1, int epoch, double a, double b, double gamma,
+                                       double alpha, unsigned long long seed, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(emb && head && tail && eps && eps_neg && next && next_neg, "umap_sgd_epoch: null pointer");
+  AVA_REQUIRE(N >= 1 && dim >= 1 && dim <= UMAP_MAX_DIM && e0 >= 0 && e1 >= e0 && epoch >= 0,
+              "umap_sgd_epoch: bad arguments");
+  if (e1 == e0) return 0;
+  const long long n = e1 - e0;
+  sgd_epoch_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(emb, N, dim, head, tail, eps, eps_neg, next, next_neg,
+                                                             e0, e1, epoch, a, b, gamma, alpha, seed);
+  return check_launch("umap sgd_epoch_kernel");
+}

@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AVA_B200_ABI_VERSION 6
+#define AVA_B200_ABI_VERSION 7
 #define AVA_NUM_BN_LAYERS 14
 #define AVA_STATS_STRIDE 64 /* doubles per layer in a stats block: [0..31]=sum, [32..63]=sum of squares */
 
@@ -395,6 +395,76 @@ int ava_b200_pca_fit(const void* x, int is_f32, long long N, int D, double* mean
                      double* comps, void* ws, long long ws_bytes, void* stream);
 int ava_b200_pca_transform(const void* x, int is_f32, long long N, int D, const double* mean, const double* comps,
                            int K, double* out, void* stream);
+
+/* ------------------------------------------------- UMAP of the latent means (csrc/umap.cu)
+ * The device stages of umap-learn 0.5's UMAP(metric='euclidean').fit_transform, the projection the
+ * reference builds in ava/data/data_container.py (_make_latent_mean_umap_projection).  The Python class
+ * LatentUMAP (data/latent_umap.py) strings them together; the sorts, prefix sums and compactions
+ * between the stages are its plumbing (torch), every number is computed here.
+ *
+ * Exact k nearest neighbours (replaces umap.umap_.nearest_neighbors, NNDescent): x [N, D] rows, float64
+ * (is_f32 = 0) or float32 (1), D <= 64, 1 <= k <= min(N, 100).  An fp32 brute-force pass keeps the best
+ * KP >= k + 8 candidates per row (KP in {16, 32, 64, 128}); an fp64 pass recomputes their distances
+ * from the input rows and writes the first k by (distance, not-self, index): knn_idx [N, k] int32 (the row
+ * itself first), knn_dist [N, k] Euclidean, float64.  ws: ava_b200_umap_knn_ws_bytes(N, k) bytes. */
+long long ava_b200_umap_knn_ws_bytes(int N, int k);
+int ava_b200_umap_knn(const void* x, int is_f32, int N, int D, int k, int* knn_idx, double* knn_dist, void* ws,
+                      long long ws_bytes, void* stream);
+/* umap.umap_.smooth_knn_dist (n_iter 64, tolerance 1e-5, MIN_K_DIST_SCALE 1e-3 against the row's mean
+ * distance, or the mean of all N*k distances -- a fixed-order sum -- where rho = 0) followed by
+ * umap.umap_.compute_membership_strengths, in fp64: rho [N], sigma [N], weights [N, k] (0 for the row
+ * itself).  ws: 1 double of scratch. */
+int ava_b200_umap_smooth_knn(const int* knn_idx, const double* knn_dist, int N, int k, double local_connectivity,
+                             double* rho, double* sigma, double* weights, double* ws, void* stream);
+/* The fuzzy union of umap.umap_.fuzzy_simplicial_set (set_op_mix_ratio 1): P = A + A^T - A.*A^T.
+ * edge_keys writes 2*N*k keys: row*N + col for (i, j) and (j, i) of every neighbour j != i, -1 for the
+ * self entries.  The caller sorts them and drops duplicates and -1 (nnz keys remain); graph then writes
+ * the CSR of P: rows/cols/vals [nnz] in row-major, column-sorted order and rowptr [N + 1] (int64). */
+int ava_b200_umap_edge_keys(const int* knn_idx, int N, int k, long long* keys, void* stream);
+int ava_b200_umap_graph(const long long* keys, long long nnz, int N, const int* knn_idx, const double* weights,
+                        int k, int* rows, int* cols, double* vals, long long* rowptr, void* stream);
+/* umap.umap_.make_epochs_per_sample on the pruned edge weights (vmax: device pointer to their maximum)
+ * and the set-up of umap.layouts.optimize_layout_euclidean: eps = n_epochs / (n_epochs * w / vmax) (-1 where
+ * that is 0), eps_neg = eps / negative_sample_rate, next = eps, next_neg = eps_neg; all [n]. */
+int ava_b200_umap_epochs_per_sample(const double* vals, long long n, const double* vmax, int n_epochs,
+                                    double negative_sample_rate, double* eps, double* eps_neg, double* next,
+                                    double* next_neg, void* stream);
+/* Connected components of the symmetric CSR graph (scipy.sparse.csgraph.connected_components as
+ * umap.spectral calls it): one round of min-label hooking.  Start from labels[i] = i and repeat with
+ * *changed zeroed until a round leaves it 0; then labels[i] = the smallest vertex of i's component. */
+int ava_b200_umap_components_step(const long long* rowptr, const int* cols, int N, int* labels, int* changed,
+                                  void* stream);
+/* dis[i] = 1 / sqrt(row sum i of P): the D^-1/2 of umap.spectral.spectral_layout. */
+int ava_b200_umap_degree(const long long* rowptr, const double* vals, int N, double* dis, void* stream);
+/* The normalised Laplacian of one component applied to a block (the product of the eigensolver that replaces
+ * scipy.sparse.linalg.eigsh in umap.spectral): for r < n, v = verts[r],
+ *   Y[r, :] = X[r, :] - dis[v] * sum_j P[v, j] dis[j] X[pos[j], :],   X, Y [n, m] row-major, m <= 32,
+ * pos: vertex -> row of its component.  A warp per row; bitwise reproducible. */
+int ava_b200_umap_spmm(const long long* rowptr, const int* cols, const double* vals, const int* verts, int n,
+                       const int* pos, const double* dis, const double* X, int m, double* Y, void* stream);
+/* out [p, q] = A^T B for A [n, p], B [n, q] row-major (p*q <= 2048), summed in a fixed order; ws:
+ * ava_b200_umap_gram_ws_bytes(p, q) bytes.  combine: Y [n, q] = A [n, p] . C [p, q]. */
+long long ava_b200_umap_gram_ws_bytes(int p, int q);
+int ava_b200_umap_gram(const double* A, int p, const double* B, int q, int n, double* out, void* ws,
+                       long long ws_bytes, void* stream);
+int ava_b200_umap_combine(const double* A, int p, const double* C, int q, int n, double* Y, void* stream);
+/* out[i] = draw i of stream `stream_id` under `seed` (counter-based: the splitmix64 finaliser applied
+ * along (seed, stream_id, i, 0|1)): kind 0 uniform(-scale, scale), kind 1 normal(0, scale). */
+int ava_b200_umap_random(unsigned long long seed, unsigned long long stream_id, long long n, int kind, double scale,
+                         double* out, void* stream);
+/* The end of umap.umap_.simplicial_set_embedding's initialisation: per axis d,
+ * v = (float)(init * expansion) + (float)noise (noise may be NULL), then emb = 10 (v - min) / (max - min)
+ * in fp32 (0 where max == min).  init [N, dim] float64, emb [N, dim] float32, dim <= 8. */
+int ava_b200_umap_init_layout(const double* init, const double* noise, double expansion, int N, int dim,
+                              float* emb, void* stream);
+/* One epoch n of umap.layouts._optimize_layout_euclidean_single_epoch over the edges [e0, e1) (head ->
+ * tail, both moved by the attraction; negatives move the head), Hogwild on the fp32 embedding [N, dim].
+ * Negative vertex p of edge e in epoch n: umap_hash(seed, n, e, p) mod N (the hash of
+ * ava_b200_umap_random).  alpha is the epoch's learning rate. */
+int ava_b200_umap_sgd_epoch(float* emb, int N, int dim, const int* head, const int* tail, const double* eps,
+                            const double* eps_neg, double* next, double* next_neg, long long e0, long long e1,
+                            int epoch, double a, double b, double gamma, double alpha, unsigned long long seed,
+                            void* stream);
 
 #ifdef __cplusplus
 }
