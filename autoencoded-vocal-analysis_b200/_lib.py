@@ -54,7 +54,7 @@ SIGNATURES = {
     "ava_b200_pca_ws_bytes": (I,),
     "ava_b200_pca_fit": (P, I, LL, I, P, P, P, P, P, LL, P),
     "ava_b200_pca_transform": (P, I, LL, I, P, P, I, P, P),
-    "ava_b200_umap_knn_ws_bytes": (I, I),
+    "ava_b200_umap_knn_ws_bytes": (I, I, I),
     "ava_b200_umap_knn": (P, I, I, I, I, P, P, P, LL, P),
     "ava_b200_umap_smooth_knn": (P, P, I, I, D, P, P, P, P, P),
     "ava_b200_umap_edge_keys": (P, I, I, P, P),

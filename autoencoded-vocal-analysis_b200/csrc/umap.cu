@@ -3,12 +3,16 @@
 // with umap.UMAP(n_components=2, n_neighbors=20, min_dist=0.1, metric='euclidean', random_state=42).
 //
 //   1. exact kNN (replaces umap.umap_.nearest_neighbors / NNDescent): brute force over all N^2 pairs.
+//      Pass 0: the rows shifted by the mean of the first rows and scaled by a power of two to |y| < 1,
+//      rounded to fp32 (so the fp32 pass sees O(1) values whatever the data's offset and scale).
 //      Pass 1, fp32: each thread owns one query row (in registers) and a sorted top-KP list (distances
 //      in registers, indices in a shared-memory column of its own); candidate rows stream through shared
 //      memory in tiles.  Squared distance in the difference form sum (x - y)^2.  KP >= k + 8 keeps a
 //      margin for fp32 near-ties; the query itself enters with distance -1, so it is always kept.
 //      Pass 2, fp64: a warp per query recomputes the KP candidates' distances from the input rows and
-//      ranks them by (distance, not-self, index); the first k are written.
+//      ranks them by (distance, not-self, index); the first k are written.  The row is certified when
+//      its k-th distance is strictly below a rounding-error bound on the distance of every candidate
+//      pass 1 dropped (knn_reject_bound); the rest are rescanned over all rows in fp64 and ranked again.
 //      Cost: N^2 * D subtract + FMA pairs on the FP32 pipe (pass 1); pass 2 is O(N * KP * D).
 //   2. smooth_knn_dist + compute_membership_strengths (umap.umap_), one thread per row, fp64.
 //   3. the fuzzy union P = A + A^T - A.*A^T (umap.umap_.fuzzy_simplicial_set, set_op_mix_ratio = 1):
@@ -28,6 +32,8 @@
 // Hogwild updates race by design (umap-learn's parallel mode).
 #include <float.h>
 #include <limits.h>
+
+#include <algorithm>
 
 #include "common.cuh"
 
@@ -52,46 +58,173 @@ __device__ __forceinline__ double umap_unit(unsigned long long h) {
 // ------------------------------------------------------------------------------------------ kNN
 constexpr int KNN_THREADS = 128;   // queries per CTA
 constexpr int KNN_TILE = 64;       // candidate rows per shared-memory tile
+constexpr int KNN_MAX_D = 64;
+constexpr int KNN_SHIFT_ROWS = 1024;
 
-template <typename T, int DP, int KP>
+// Workspace: cand [N][KP] int | d32 [N] float (the worst kept fp32 distance of each row) | list [N] int
+// (the rows the certificate rejects) | y [N][D] float (the scaled rows) | shift [64] double | range
+// (max |x - shift| as fp64 bits) | count.
+struct KnnWs {
+  int* cand;
+  float* y;
+  float* d32;
+  int* list;
+  double* shift;
+  unsigned long long* range;
+  int* count;
+};
+static long long knn_ws_layout(int N, int D, int KP, void* base, KnnWs* w) {
+  const long long n = N;
+  const long long o_d32 = n * KP * 4, o_list = o_d32 + n * 4, o_y = o_list + n * 4;
+  const long long o_hdr = (o_y + n * D * 4 + 7) / 8 * 8;
+  const long long o_range = o_hdr + KNN_MAX_D * 8, o_count = o_range + 8;
+  if (w) {
+    char* b = (char*)base;
+    w->cand = (int*)b;
+    w->d32 = (float*)(b + o_d32);
+    w->list = (int*)(b + o_list);
+    w->y = (float*)(b + o_y);
+    w->shift = (double*)(b + o_hdr);
+    w->range = (unsigned long long*)(b + o_range);
+    w->count = (int*)(b + o_count);
+  }
+  return o_count + 8;
+}
+
+// The fp32 pass selects on y = (x - shift) 2^-e, with shift the mean of the first rows and e the exponent
+// of M = max |x - shift| (M = ms 2^e, ms in [0.5, 1)): the values are O(1) whatever the data's offset and
+// scale.  2^-e is applied as two factors so that neither overflows for any finite M.
+struct KnnScale {
+  double f1, f2;
+};
+__device__ __forceinline__ KnnScale knn_scale(const unsigned long long* range) {
+  const double M = __longlong_as_double((long long)*range);
+  int e = 0;
+  if (M > 0.0) frexp(M, &e);
+  KnnScale s;
+  s.f1 = ldexp(1.0, -(e / 2));
+  s.f2 = ldexp(1.0, -(e - e / 2));
+  return s;
+}
+
+// shift[d] = mean of the first KNN_SHIFT_ROWS rows; zeroes the range and the rejected-row count
+template <typename T>
+__global__ void knn_shift_kernel(const T* __restrict__ x, int N, int D, double* __restrict__ shift,
+                                 unsigned long long* __restrict__ range, int* __restrict__ count) {
+  const int d = threadIdx.x;
+  if (d == 0) {
+    *range = 0ull;
+    *count = 0;
+  }
+  if (d >= D) return;
+  const int R = min(N, KNN_SHIFT_ROWS);
+  double s = 0.0;
+  for (int r = 0; r < R; ++r) s += (double)x[(long long)r * D + d];
+  shift[d] = s / (double)R;
+}
+
+// range = max |x - shift| over all N*D values (the bits of a non-negative double order like the value)
+template <typename T>
+__global__ void knn_range_kernel(const T* __restrict__ x, long long n, int D, const double* __restrict__ shift,
+                                 unsigned long long* __restrict__ range) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  int d = (int)(i % D);
+  const int dstep = (int)(stride % D);
+  double m = 0.0;
+  for (; i < n; i += stride) {
+    m = fmax(m, fabs((double)x[i] - shift[d]));
+    d += dstep;
+    if (d >= D) d -= D;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if (threadIdx.x % 32 == 0 && m > 0.0) atomicMax(range, (unsigned long long)__double_as_longlong(m));
+}
+
+// y = (float)((x - shift) 2^-e), the values the fp32 pass selects on
+template <typename T>
+__global__ void knn_scaled_kernel(const T* __restrict__ x, long long n, int D, const double* __restrict__ shift,
+                                  const unsigned long long* __restrict__ range, float* __restrict__ y) {
+  const KnnScale sc = knn_scale(range);
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  int d = (int)(i % D);
+  const int dstep = (int)(stride % D);
+  for (; i < n; i += stride) {
+    y[i] = (float)((((double)x[i] - shift[d]) * sc.f1) * sc.f2);
+    d += dstep;
+    if (d >= D) d -= D;
+  }
+}
+
+// Top-KP candidates of each query row by squared Euclidean distance, in the difference form.
+// ACC = float: the selection pass over all rows of x = the scaled rows y; also records each row's worst kept
+//   distance d32[q], which bounds the distance of every candidate it did not keep.
+// ACC = double: the rescan of the rows list[0 .. *count) on the input rows x, with the same formula (and so
+//   the same bits) as knn_refine_kernel; ties go to the lower index, as in the refine ranking.
+template <typename T, typename ACC, int DP, int KP>
 __global__ void __launch_bounds__(KNN_THREADS, 1)
-knn_select_kernel(const T* __restrict__ x, int N, int D, int* __restrict__ cand) {
-  __shared__ __align__(16) float tile[KNN_TILE * DP];
+knn_select_kernel(const T* __restrict__ x, int N, int D, const int* __restrict__ list, const int* __restrict__ count,
+                  int* __restrict__ cand, float* __restrict__ d32) {
+  constexpr bool F64 = sizeof(ACC) == 8;
+  __shared__ __align__(16) ACC tile[KNN_TILE * DP];
   extern __shared__ int sidx[];   // [KP][KNN_THREADS]
   const int tid = threadIdx.x;
-  const int q = blockIdx.x * KNN_THREADS + tid;
-  float xq[DP];
+  int q;
+  if (F64) {
+    const int n_list = *count;
+    if (blockIdx.x * KNN_THREADS >= n_list) return;
+    const int p = blockIdx.x * KNN_THREADS + tid;
+    q = p < n_list ? list[p] : -1;
+  } else {
+    q = blockIdx.x * KNN_THREADS + tid;
+    if (q >= N) q = -1;
+  }
+  ACC xq[DP];
 #pragma unroll
-  for (int d = 0; d < DP; ++d) xq[d] = (q < N && d < D) ? (float)x[(long long)q * D + d] : 0.f;
-  float dk[KP];
+  for (int d = 0; d < DP; ++d) xq[d] = (q >= 0 && d < D) ? (ACC)x[(long long)q * D + d] : (ACC)0;
+  ACC dk[KP];
 #pragma unroll
   for (int j = 0; j < KP; ++j) {
-    dk[j] = FLT_MAX;
+    dk[j] = F64 ? (ACC)INFINITY : (ACC)FLT_MAX;
     sidx[j * KNN_THREADS + tid] = -1;
   }
   for (int c0 = 0; c0 < N; c0 += KNN_TILE) {
     __syncthreads();
     for (int e = tid; e < KNN_TILE * DP; e += KNN_THREADS) {
       const int r = e / DP, d = e - r * DP;
-      tile[e] = (c0 + r < N && d < D) ? (float)x[(long long)(c0 + r) * D + d] : 0.f;
+      tile[e] = (c0 + r < N && d < D) ? (ACC)x[(long long)(c0 + r) * D + d] : (ACC)0;
     }
     __syncthreads();
     const int nc = min(KNN_TILE, N - c0);
     for (int r = 0; r < nc; ++r) {
-      const float4* t4 = reinterpret_cast<const float4*>(tile + r * DP);
-      float s0 = 0.f, s1 = 0.f;
+      ACC dist;
+      if constexpr (F64) {
+        double s = 0.0;
 #pragma unroll
-      for (int d4 = 0; d4 < DP / 4; ++d4) {
-        const float4 v = t4[d4];
-        const float e0 = xq[4 * d4] - v.x, e1 = xq[4 * d4 + 1] - v.y;
-        const float e2 = xq[4 * d4 + 2] - v.z, e3 = xq[4 * d4 + 3] - v.w;
-        s0 = fmaf(e0, e0, s0);
-        s1 = fmaf(e1, e1, s1);
-        s0 = fmaf(e2, e2, s0);
-        s1 = fmaf(e3, e3, s1);
+        for (int d = 0; d < DP; ++d) {
+          const double e = xq[d] - tile[r * DP + d];
+          s = __fma_rn(e, e, s);
+        }
+        dist = fmin(s, DBL_MAX);   // an overflowed distance still fills an empty slot
+      } else {
+        const float4* t4 = reinterpret_cast<const float4*>(tile + r * DP);
+        float s0 = 0.f, s1 = 0.f;
+#pragma unroll
+        for (int d4 = 0; d4 < DP / 4; ++d4) {
+          const float4 v = t4[d4];
+          const float e0 = xq[4 * d4] - v.x, e1 = xq[4 * d4 + 1] - v.y;
+          const float e2 = xq[4 * d4 + 2] - v.z, e3 = xq[4 * d4 + 3] - v.w;
+          s0 = fmaf(e0, e0, s0);
+          s1 = fmaf(e1, e1, s1);
+          s0 = fmaf(e2, e2, s0);
+          s1 = fmaf(e3, e3, s1);
+        }
+        dist = s0 + s1;
       }
       const int c = c0 + r;
-      const float dist = (c == q) ? -1.f : s0 + s1;
+      if (c == q) dist = (ACC)-1;
       if (dist < dk[KP - 1]) {
 #pragma unroll
         for (int j = KP - 1; j > 0; --j) {
@@ -110,20 +243,53 @@ knn_select_kernel(const T* __restrict__ x, int N, int D, int* __restrict__ cand)
       }
     }
   }
-  if (q < N)
+  if (q >= 0) {
     for (int j = 0; j < KP; ++j) cand[(long long)q * KP + j] = sidx[j * KNN_THREADS + tid];
+    if (!F64) d32[q] = (float)dk[KP - 1];
+  }
 }
 
-// one warp per query: fp64 distances of the KP candidates, ranked by (distance, not-self, index)
+// A lower bound, in the input's units, on the distance of every candidate the fp32 pass did not keep for a
+// row whose worst kept fp32 squared distance is t32 (each of those has a computed fp32 distance >= t32).
+// With u = 2^-24 and ms = M 2^-e <= 1 the largest scaled |value|:
+//  - each scaled value is within delta = (u + 2^-52) ms + 2^-149 of the exact (x - shift) 2^-e;
+//  - the fp32 sum of DP squared differences (two chains of DP/2 FMAs and one add; subtraction results that
+//    are subnormal are exact) is at most (1 + g)(exact sum of the rounded values) + (DP + 1) 2^-149,
+//    g = (DP/2 + 3) u (1.001);
+// so the true scaled distance is at least sqrt((t32 - (DP + 1) 2^-149) / (1 + g)) - 2 delta sqrt(D).  The
+// result is shrunk by 2^-40 to cover the rounding of this evaluation and of the fp64 distances it meets.
+__device__ __forceinline__ double knn_reject_bound(float t32, const unsigned long long* range, int D, int DP) {
+  const double M = __longlong_as_double((long long)*range);
+  int e = 0;
+  const double ms = M > 0.0 ? frexp(M, &e) : 0.0;
+  const double u = 0x1p-24;
+  const double g = (DP / 2 + 3) * u * 1.001;
+  const double delta = (u + 0x1p-52) * ms + 0x1p-149;
+  const double a = sqrt(fmax((double)t32 - (DP + 1) * 0x1p-149, 0.0) / (1.0 + g));
+  const double lb = a - 2.0 * delta * sqrt((double)D);
+  return lb > 0.0 ? ldexp(lb * (1.0 - 0x1p-40), e) : 0.0;
+}
+
+// One warp per query: fp64 distances of the KP candidates, ranked by (distance, not-self, index); the first
+// k are written.  certify: queries 0..N-1, and a row whose k-th distance is not strictly below
+// knn_reject_bound (its candidates may miss a true neighbour) is appended to list for the fp64 rescan.
+// Otherwise: the rows list[0 .. *count).
 template <typename T>
-__global__ void knn_refine_kernel(const T* __restrict__ x, int N, int D, int KP, int k, const int* __restrict__ cand,
-                                  int* __restrict__ knn_idx, double* __restrict__ knn_dist) {
+__global__ void knn_refine_kernel(const T* __restrict__ x, int N, int D, int DP, int KP, int k,
+                                  const int* __restrict__ cand, int certify, const float* __restrict__ d32,
+                                  const unsigned long long* __restrict__ range, int* __restrict__ list,
+                                  int* __restrict__ count, int* __restrict__ knn_idx, double* __restrict__ knn_dist) {
   extern __shared__ double sref[];
   const int warps = blockDim.x / 32, w = threadIdx.x / 32, lane = threadIdx.x % 32;
   double* sd = sref + w * KP;
   int* si = reinterpret_cast<int*>(sref + warps * KP) + w * KP;
-  const int q = blockIdx.x * warps + w;
-  if (q >= N) return;
+  int q = blockIdx.x * warps + w;
+  if (certify) {
+    if (q >= N) return;
+  } else {
+    if (q >= *count) return;
+    q = list[q];
+  }
   for (int j = lane; j < KP; j += 32) {
     const int c = cand[(long long)q * KP + j];
     double s = INFINITY;
@@ -138,6 +304,7 @@ __global__ void knn_refine_kernel(const T* __restrict__ x, int N, int D, int KP,
     si[j] = c;
   }
   __syncwarp();
+  double kth = 0.0;   // the k-th fp64 squared distance
   for (int j = lane; j < KP; j += 32) {
     const int c = si[j];
     if (c < 0) continue;
@@ -155,7 +322,12 @@ __global__ void knn_refine_kernel(const T* __restrict__ x, int N, int D, int KP,
       knn_idx[(long long)q * k + rank] = c;
       knn_dist[(long long)q * k + rank] = sqrt(dj);
     }
+    if (rank == k - 1) kth = dj;
   }
+  if (!certify || N <= KP) return;   // every row was a candidate
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) kth = fmax(kth, __shfl_xor_sync(0xffffffffu, kth, o));
+  if (lane == 0 && !(sqrt(kth) < knn_reject_bound(d32[q], range, D, DP))) list[atomicAdd(count, 1)] = q;
 }
 
 static int knn_padded(int k) {
@@ -169,40 +341,65 @@ static int knn_dpad(int D) {
   return -1;
 }
 
-template <typename T, int DP, int KP>
-static int knn_launch(const T* x, int N, int D, int* cand, cudaStream_t s) {
+template <typename T, typename ACC, int DP, int KP>
+static int knn_launch(const T* x, int N, int D, const KnnWs& w, cudaStream_t s) {
   const size_t smem = (size_t)KP * KNN_THREADS * sizeof(int);
-  auto kern = knn_select_kernel<T, DP, KP>;
-  if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  kern<<<(N + KNN_THREADS - 1) / KNN_THREADS, KNN_THREADS, smem, s>>>(x, N, D, cand);
-  return check_launch("umap knn_select_kernel");
+  auto kern = knn_select_kernel<T, ACC, DP, KP>;
+  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+    set_error("umap knn_select_kernel: cudaFuncSetAttribute failed");
+    return 1;
+  }
+  kern<<<(N + KNN_THREADS - 1) / KNN_THREADS, KNN_THREADS, smem, s>>>(x, N, D, w.list, w.count, w.cand, w.d32);
+  return check_launch(sizeof(ACC) == 4 ? "umap knn_select_kernel" : "umap knn_select_kernel (fp64 rescan)");
 }
 
-template <typename T, int DP>
-static int knn_launch_k(const T* x, int N, int D, int KP, int* cand, cudaStream_t s) {
+template <typename T, typename ACC, int DP>
+static int knn_launch_k(const T* x, int N, int D, int KP, const KnnWs& w, cudaStream_t s) {
   switch (KP) {
-    case 16: return knn_launch<T, DP, 16>(x, N, D, cand, s);
-    case 32: return knn_launch<T, DP, 32>(x, N, D, cand, s);
-    case 64: return knn_launch<T, DP, 64>(x, N, D, cand, s);
-    default: return knn_launch<T, DP, 128>(x, N, D, cand, s);
+    case 16: return knn_launch<T, ACC, DP, 16>(x, N, D, w, s);
+    case 32: return knn_launch<T, ACC, DP, 32>(x, N, D, w, s);
+    case 64: return knn_launch<T, ACC, DP, 64>(x, N, D, w, s);
+    default: return knn_launch<T, ACC, DP, 128>(x, N, D, w, s);
   }
 }
 
-template <typename T>
-static int knn_run(const T* x, int N, int D, int k, int* knn_idx, double* knn_dist, int* cand, cudaStream_t s) {
-  const int KP = knn_padded(k);
-  int rc;
+template <typename T, typename ACC>
+static int knn_select(const T* x, int N, int D, int KP, const KnnWs& w, cudaStream_t s) {
   switch (knn_dpad(D)) {
-    case 8: rc = knn_launch_k<T, 8>(x, N, D, KP, cand, s); break;
-    case 16: rc = knn_launch_k<T, 16>(x, N, D, KP, cand, s); break;
-    case 32: rc = knn_launch_k<T, 32>(x, N, D, KP, cand, s); break;
-    default: rc = knn_launch_k<T, 64>(x, N, D, KP, cand, s); break;
+    case 8: return knn_launch_k<T, ACC, 8>(x, N, D, KP, w, s);
+    case 16: return knn_launch_k<T, ACC, 16>(x, N, D, KP, w, s);
+    case 32: return knn_launch_k<T, ACC, 32>(x, N, D, KP, w, s);
+    default: return knn_launch_k<T, ACC, 64>(x, N, D, KP, w, s);
   }
-  if (rc) return rc;
+}
+
+// shift and range; fp32 selection; fp64 refine with the certificate; fp64 rescan and refine of the rows it
+// rejects (the last two launches find an empty list and return at once in the usual case)
+template <typename T>
+static int knn_run(const T* x, int N, int D, int k, int* knn_idx, double* knn_dist, void* ws, cudaStream_t s) {
+  const int KP = knn_padded(k), DP = knn_dpad(D);
+  KnnWs w;
+  knn_ws_layout(N, D, KP, ws, &w);
+  knn_shift_kernel<T><<<1, KNN_MAX_D, 0, s>>>(x, N, D, w.shift, w.range, w.count);
+  if (check_launch("umap knn_shift_kernel")) return 1;
+  const long long n = (long long)N * D;
+  knn_range_kernel<T><<<(unsigned)std::min<long long>((n + 255) / 256, 4 * kNumSMs), 256, 0, s>>>(x, n, D, w.shift,
+                                                                                                  w.range);
+  if (check_launch("umap knn_range_kernel")) return 1;
+  knn_scaled_kernel<T><<<(unsigned)std::min<long long>((n + 255) / 256, 8 * kNumSMs), 256, 0, s>>>(x, n, D, w.shift,
+                                                                                                   w.range, w.y);
+  if (check_launch("umap knn_scaled_kernel")) return 1;
+  if (knn_select<float, float>(w.y, N, D, KP, w, s)) return 1;
   constexpr int WARPS = 8;
   const size_t smem = (size_t)WARPS * KP * (sizeof(double) + sizeof(int));
-  knn_refine_kernel<T><<<(N + WARPS - 1) / WARPS, WARPS * 32, smem, s>>>(x, N, D, KP, k, cand, knn_idx, knn_dist);
-  return check_launch("umap knn_refine_kernel");
+  const unsigned grid = (unsigned)((N + WARPS - 1) / WARPS);
+  knn_refine_kernel<T><<<grid, WARPS * 32, smem, s>>>(x, N, D, DP, KP, k, w.cand, 1, w.d32, w.range, w.list, w.count,
+                                                      knn_idx, knn_dist);
+  if (check_launch("umap knn_refine_kernel")) return 1;
+  if (knn_select<T, double>(x, N, D, KP, w, s)) return 1;
+  knn_refine_kernel<T><<<grid, WARPS * 32, smem, s>>>(x, N, D, DP, KP, k, w.cand, 0, w.d32, w.range, w.list, w.count,
+                                                      knn_idx, knn_dist);
+  return check_launch("umap knn_refine_kernel (rescanned rows)");
 }
 
 // --------------------------------------------------------------------- smooth kNN, memberships
@@ -257,7 +454,8 @@ __global__ void smooth_knn_kernel(const int* __restrict__ knn_idx, const double*
       }
     if (index > 0) {
       rho = nz_prev;
-      if (interpolation > SMOOTH_K_TOLERANCE) rho += interpolation * (nz_at - nz_prev);
+      // umap-learn's rounding (no contraction into an FMA), so that rho repeats its bits
+      if (interpolation > SMOOTH_K_TOLERANCE) rho = __dadd_rn(rho, __dmul_rn(interpolation, nz_at - nz_prev));
     } else {
       rho = interpolation * nz_first;
     }
@@ -336,7 +534,7 @@ __global__ void graph_weights_kernel(const long long* __restrict__ keys, long lo
   const double b = knn_weight(knn_idx, w, k, c, (int)r);
   rows[p] = (int)r;
   cols[p] = c;
-  vals[p] = a + b - a * b;
+  vals[p] = __dsub_rn(__dadd_rn(a, b), __dmul_rn(a, b));   // (a + b) - ab, as scipy's A + A^T - A.*A^T rounds
 }
 
 __global__ void epochs_per_sample_kernel(const double* __restrict__ vals, long long n, const double* __restrict__ vmax,
@@ -589,9 +787,9 @@ using namespace ava;
 
 #define UMAP_STREAM cudaStream_t s = (cudaStream_t)stream
 
-extern "C" long long ava_b200_umap_knn_ws_bytes(int N, int k) {
-  if (N < 1 || k < 1 || k > 100) return -1;
-  return (long long)N * knn_padded(k) * (long long)sizeof(int);
+extern "C" long long ava_b200_umap_knn_ws_bytes(int N, int D, int k) {
+  if (N < 1 || D < 1 || D > KNN_MAX_D || k < 1 || k > 100) return -1;
+  return knn_ws_layout(N, D, knn_padded(k), nullptr, nullptr);
 }
 
 extern "C" int ava_b200_umap_knn(const void* x, int is_f32, int N, int D, int k, int* knn_idx, double* knn_dist,
@@ -601,10 +799,9 @@ extern "C" int ava_b200_umap_knn(const void* x, int is_f32, int N, int D, int k,
   AVA_REQUIRE(N >= 1 && k >= 1 && k <= 100 && k <= N, "umap_knn: need 1 <= k <= min(N, 100), got N=%d k=%d", N, k);
   AVA_REQUIRE(D >= 1 && D <= 64, "umap_knn: D=%d outside 1..64", D);
   AVA_REQUIRE(is_f32 == 0 || is_f32 == 1, "umap_knn: is_f32 must be 0 or 1");
-  AVA_REQUIRE(ws_bytes >= ava_b200_umap_knn_ws_bytes(N, k), "umap_knn: workspace too small");
-  if (is_f32)
-    return knn_run<float>((const float*)x, N, D, k, knn_idx, knn_dist, (int*)ws, s);
-  return knn_run<double>((const double*)x, N, D, k, knn_idx, knn_dist, (int*)ws, s);
+  AVA_REQUIRE(ws_bytes >= ava_b200_umap_knn_ws_bytes(N, D, k), "umap_knn: workspace too small");
+  if (is_f32) return knn_run<float>((const float*)x, N, D, k, knn_idx, knn_dist, ws, s);
+  return knn_run<double>((const double*)x, N, D, k, knn_idx, knn_dist, ws, s);
 }
 
 extern "C" int ava_b200_umap_smooth_knn(const int* knn_idx, const double* knn_dist, int N, int k,
@@ -613,8 +810,7 @@ extern "C" int ava_b200_umap_smooth_knn(const int* knn_idx, const double* knn_di
   UMAP_STREAM;
   AVA_REQUIRE(knn_idx && knn_dist && rho && sigma && weights && ws, "umap_smooth_knn: null pointer");
   AVA_REQUIRE(N >= 1 && k >= 2, "umap_smooth_knn: need N >= 1 and k >= 2");
-  AVA_REQUIRE(local_connectivity >= 0.0 && local_connectivity <= k - 1,
-              "umap_smooth_knn: local_connectivity outside 0..k-1");
+  AVA_REQUIRE(local_connectivity >= 0.0, "umap_smooth_knn: local_connectivity must be >= 0");
   mean_kernel<<<1, 1024, 0, s>>>(knn_dist, (long long)N * k, ws);
   if (check_launch("umap mean_kernel")) return 1;
   smooth_knn_kernel<<<(N + 127) / 128, 128, 0, s>>>(knn_idx, knn_dist, N, k, local_connectivity, ws, rho, sigma,
@@ -682,8 +878,16 @@ extern "C" int ava_b200_umap_spmm(const long long* rowptr, const int* cols, cons
   return check_launch("umap spmm_kernel");
 }
 
+// p*q outputs over 8 accumulators per thread; GRAM_ROWS (p + q) doubles of staged rows within the 48 KB of
+// shared memory a launch gets without opting in
+constexpr int GRAM_MAX_PQ = 8 * GRAM_THREADS;
+constexpr int GRAM_MAX_P_PLUS_Q = 48 * 1024 / (GRAM_ROWS * (int)sizeof(double));
+static bool gram_shape_ok(int p, int q) {
+  return p >= 1 && q >= 1 && p <= GRAM_MAX_PQ && q <= GRAM_MAX_PQ && p * q <= GRAM_MAX_PQ && p + q <= GRAM_MAX_P_PLUS_Q;
+}
+
 extern "C" long long ava_b200_umap_gram_ws_bytes(int p, int q) {
-  if (p < 1 || q < 1 || p * q > 8 * GRAM_THREADS) return -1;
+  if (!gram_shape_ok(p, q)) return -1;
   return (long long)GRAM_CTAS * p * q * (long long)sizeof(double);
 }
 
@@ -691,8 +895,8 @@ extern "C" int ava_b200_umap_gram(const double* A, int p, const double* B, int q
                                   long long ws_bytes, void* stream) {
   UMAP_STREAM;
   AVA_REQUIRE(A && B && out && ws, "umap_gram: null pointer");
-  AVA_REQUIRE(n >= 1 && p >= 1 && q >= 1 && p * q <= 8 * GRAM_THREADS, "umap_gram: need p*q <= %d",
-              8 * GRAM_THREADS);
+  AVA_REQUIRE(n >= 1 && gram_shape_ok(p, q), "umap_gram: need n >= 1, p, q >= 1, p*q <= %d and p + q <= %d, got "
+              "n=%d p=%d q=%d", GRAM_MAX_PQ, GRAM_MAX_P_PLUS_Q, n, p, q);
   AVA_REQUIRE(ws_bytes >= ava_b200_umap_gram_ws_bytes(p, q), "umap_gram: workspace too small");
   const size_t smem = (size_t)GRAM_ROWS * (p + q) * sizeof(double);
   gram_kernel<<<GRAM_CTAS, GRAM_THREADS, smem, s>>>(A, p, B, q, n, (double*)ws);

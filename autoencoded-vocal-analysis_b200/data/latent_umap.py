@@ -82,7 +82,7 @@ def knn(x, k):
     (indices [N, k] int32, Euclidean distances [N, k] float64), the row itself first."""
     N, D = x.shape
     dev = x.device
-    ws_bytes = int(_lib.lib().ava_b200_umap_knn_ws_bytes(N, k))
+    ws_bytes = int(_lib.lib().ava_b200_umap_knn_ws_bytes(N, D, k))
     ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
     idx = torch.empty(N, k, dtype=torch.int32, device=dev)
     dist = torch.empty(N, k, dtype=torch.float64, device=dev)

@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AVA_B200_ABI_VERSION 7
+#define AVA_B200_ABI_VERSION 8
 #define AVA_NUM_BN_LAYERS 14
 #define AVA_STATS_STRIDE 64 /* doubles per layer in a stats block: [0..31]=sum, [32..63]=sum of squares */
 
@@ -403,11 +403,18 @@ int ava_b200_pca_transform(const void* x, int is_f32, long long N, int D, const 
  * between the stages are its plumbing (torch), every number is computed here.
  *
  * Exact k nearest neighbours (replaces umap.umap_.nearest_neighbors, NNDescent): x [N, D] rows, float64
- * (is_f32 = 0) or float32 (1), D <= 64, 1 <= k <= min(N, 100).  An fp32 brute-force pass keeps the best
- * KP >= k + 8 candidates per row (KP in {16, 32, 64, 128}); an fp64 pass recomputes their distances
- * from the input rows and writes the first k by (distance, not-self, index): knn_idx [N, k] int32 (the row
- * itself first), knn_dist [N, k] Euclidean, float64.  ws: ava_b200_umap_knn_ws_bytes(N, k) bytes. */
-long long ava_b200_umap_knn_ws_bytes(int N, int k);
+ * (is_f32 = 0) or float32 (1), finite, D <= 64, 1 <= k <= min(N, 100).  Writes the first k rows by
+ * (distance, not-self, index) of fp64 difference-form distances: knn_idx [N, k] int32 (the row itself
+ * first), knn_dist [N, k] Euclidean, float64; exact at any scale and offset of the data (up to fp64
+ * overflow of the squared distances).  An fp32 brute-force pass on y = (x - shift) 2^-e (shift: the mean
+ * of the first 1024 rows; e: the exponent of M = max |x - shift|, so |y| < 1) keeps the best KP >= k + 8
+ * candidates per row (KP in {16, 32, 64, 128}) and an fp64 pass ranks them.  A row is certified when its
+ * k-th fp64 distance is strictly below a lower bound on the distance of every candidate it dropped:
+ *   2^e ((sqrt(t32 - (DP + 1) 2^-149) / (1 + g)) - 2 delta sqrt(D)) (1 - 2^-40),
+ * t32 the worst kept fp32 squared distance, DP the padded D, g = (DP/2 + 3) 2^-24 (1.001),
+ * delta = (2^-24 + 2^-52) M 2^-e + 2^-149; or when N <= KP.  Other rows are rescanned in fp64.
+ * ws: ava_b200_umap_knn_ws_bytes(N, D, k) bytes. */
+long long ava_b200_umap_knn_ws_bytes(int N, int D, int k);
 int ava_b200_umap_knn(const void* x, int is_f32, int N, int D, int k, int* knn_idx, double* knn_dist, void* ws,
                       long long ws_bytes, void* stream);
 /* umap.umap_.smooth_knn_dist (n_iter 64, tolerance 1e-5, MIN_K_DIST_SCALE 1e-3 against the row's mean
@@ -442,7 +449,7 @@ int ava_b200_umap_degree(const long long* rowptr, const double* vals, int N, dou
  * pos: vertex -> row of its component.  A warp per row; bitwise reproducible. */
 int ava_b200_umap_spmm(const long long* rowptr, const int* cols, const double* vals, const int* verts, int n,
                        const int* pos, const double* dis, const double* X, int m, double* Y, void* stream);
-/* out [p, q] = A^T B for A [n, p], B [n, q] row-major (p*q <= 2048), summed in a fixed order; ws:
+/* out [p, q] = A^T B for A [n, p], B [n, q] row-major (p*q <= 2048 and p + q <= 192), summed in a fixed order; ws:
  * ava_b200_umap_gram_ws_bytes(p, q) bytes.  combine: Y [n, q] = A [n, p] . C [p, q]. */
 long long ava_b200_umap_gram_ws_bytes(int p, int q);
 int ava_b200_umap_gram(const double* A, int p, const double* B, int q, int n, double* out, void* ws,
