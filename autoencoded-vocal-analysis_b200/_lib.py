@@ -69,6 +69,11 @@ SIGNATURES = {
     "ava_b200_umap_random": (ctypes.c_ulonglong, ctypes.c_ulonglong, LL, I, D, P, P),
     "ava_b200_umap_init_layout": (P, P, D, I, I, P, P),
     "ava_b200_umap_sgd_epoch": (P, I, I, P, P, P, P, P, P, LL, LL, I, D, D, D, D, ctypes.c_ulonglong, P),
+    "ava_b200_umap_knn_query_ws_bytes": (I, I, I, I),
+    "ava_b200_umap_knn_query": (P, I, P, I, I, I, I, P, P, P, LL, P),
+    "ava_b200_umap_smooth_knn_query": (P, P, I, I, D, P, P, P, P, P),
+    "ava_b200_umap_init_transform": (P, P, I, I, P, I, I, P, P),
+    "ava_b200_umap_sgd_transform": (P, I, P, I, I, P, P, P, P, P, P, I, D, D, D, D, ctypes.c_ulonglong, P),
     "ava_b200_last_error": (),
     "ava_b200_abi_version": (),
     "ava_b200_launch_count": (),
@@ -82,6 +87,7 @@ _RESTYPES = {
     "ava_b200_pca_ws_bytes": LL,
     "ava_b200_umap_knn_ws_bytes": LL,
     "ava_b200_umap_gram_ws_bytes": LL,
+    "ava_b200_umap_knn_query_ws_bytes": LL,
 }
 # entry points whose int return value is a status code
 _STATUS = {n for n in SIGNATURES if n not in _RESTYPES and n not in ("ava_b200_abi_version", "ava_b200_get_conv_precision")}

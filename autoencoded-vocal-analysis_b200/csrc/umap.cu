@@ -60,23 +60,32 @@ constexpr int KNN_THREADS = 128;   // queries per CTA
 constexpr int KNN_TILE = 64;       // candidate rows per shared-memory tile
 constexpr int KNN_MAX_D = 64;
 constexpr int KNN_SHIFT_ROWS = 1024;
+// The data rows are split into S slices, one per grid row, when the query CTAs alone would leave SMs idle
+// (knn_slices).  Each slice keeps its own top-KP; the refine pass ranks the S * KP candidates of a query.
+constexpr int KNN_CTAS_PER_SM = 4;       // knn_select_kernel<float, float, 32, 32, *>: 102 registers x 128 threads
+constexpr int KNN_MAX_CAND = 256;        // S * KP: the refine pass ranks them in shared memory, in O(S^2 KP^2)
+constexpr int KNN_MIN_SLICE_ROWS = 1024;
+constexpr int KNN_REFINE_WARPS = 8;
 
-// Workspace: cand [N][KP] int | d32 [N] float (the worst kept fp32 distance of each row) | list [N] int
-// (the rows the certificate rejects) | y [N][D] float (the scaled rows) | shift [64] double | range
-// (max |x - shift| as fp64 bits) | count.
+// Workspace: cand [Nq][S][KP] int | d32 [Nq][S] float (the worst kept fp32 distance of each query in each slice) |
+// list [Nq] int (the queries the certificate rejects) | y [N][D] float (the scaled data rows) | yq [Nq][D] float (the
+// scaled queries; absent when the data is its own query set) | shift [64] double | range (max |x - shift| over the
+// data and the queries, as fp64 bits) | count.
 struct KnnWs {
   int* cand;
   float* y;
+  float* yq;
   float* d32;
   int* list;
   double* shift;
   unsigned long long* range;
   int* count;
 };
-static long long knn_ws_layout(int N, int D, int KP, void* base, KnnWs* w) {
-  const long long n = N;
-  const long long o_d32 = n * KP * 4, o_list = o_d32 + n * 4, o_y = o_list + n * 4;
-  const long long o_hdr = (o_y + n * D * 4 + 7) / 8 * 8;
+static long long knn_ws_layout(int Nq, int N, int D, int KP, int S, bool self, void* base, KnnWs* w) {
+  const long long nq = Nq, n = N;
+  const long long o_d32 = nq * S * KP * 4, o_list = o_d32 + nq * S * 4, o_y = o_list + nq * 4;
+  const long long o_yq = o_y + n * D * 4;
+  const long long o_hdr = (o_yq + (self ? 0 : nq * D * 4) + 7) / 8 * 8;
   const long long o_range = o_hdr + KNN_MAX_D * 8, o_count = o_range + 8;
   if (w) {
     char* b = (char*)base;
@@ -84,6 +93,7 @@ static long long knn_ws_layout(int N, int D, int KP, void* base, KnnWs* w) {
     w->d32 = (float*)(b + o_d32);
     w->list = (int*)(b + o_list);
     w->y = (float*)(b + o_y);
+    w->yq = self ? w->y : (float*)(b + o_yq);
     w->shift = (double*)(b + o_hdr);
     w->range = (unsigned long long*)(b + o_range);
     w->count = (int*)(b + o_count);
@@ -91,9 +101,35 @@ static long long knn_ws_layout(int N, int D, int KP, void* base, KnnWs* w) {
   return o_count + 8;
 }
 
-// The fp32 pass selects on y = (x - shift) 2^-e, with shift the mean of the first rows and e the exponent
-// of M = max |x - shift| (M = ms 2^e, ms in [0.5, 1)): the values are O(1) whatever the data's offset and
-// scale.  2^-e is applied as two factors so that neither overflows for any finite M.
+// The number of slices: 1 when the Q = ceil(Nq / 128) query CTAs fill one wave of KNN_CTAS_PER_SM per SM; otherwise
+// the S whose Q S CTAs fill their last wave best, among S * KP <= KNN_MAX_CAND and slices of at least
+// KNN_MIN_SLICE_ROWS rows; a larger S is taken only if it fills 2% more than the best smaller one.
+static int knn_slices(int Nq, int N, int KP) {
+  const long long ctas = (Nq + KNN_THREADS - 1) / KNN_THREADS;
+  const long long slots = (long long)KNN_CTAS_PER_SM * kNumSMs;
+  if (ctas >= slots) return 1;
+  int best = 1;
+  double best_fill = 0.0;
+  for (int S = 1; S * KP <= KNN_MAX_CAND && (S == 1 || N / S >= KNN_MIN_SLICE_ROWS); ++S) {
+    const long long c = ctas * S;
+    const double fill = (double)c / (double)((c + slots - 1) / slots * slots);
+    if (fill > best_fill * 1.02) {
+      best = S;
+      best_fill = fill;
+    }
+  }
+  return best;
+}
+// rows per slice: all N for one slice, else a whole number of tiles (the last slices may be short or empty)
+static int knn_slice_rows(int N, int S) {
+  if (S == 1) return N;
+  const int per = (N + S - 1) / S;
+  return (per + KNN_TILE - 1) / KNN_TILE * KNN_TILE;
+}
+
+// The fp32 pass selects on y = (x - shift) 2^-e, with shift the mean of the first data rows and e the exponent of
+// M = max |x - shift| over the data and the queries (M = ms 2^e, ms in [0.5, 1)): the values are O(1) whatever the
+// offset and scale.  2^-e is applied as two factors so that neither overflows for any finite M.
 struct KnnScale {
   double f1, f2;
 };
@@ -123,7 +159,7 @@ __global__ void knn_shift_kernel(const T* __restrict__ x, int N, int D, double* 
   shift[d] = s / (double)R;
 }
 
-// range = max |x - shift| over all N*D values (the bits of a non-negative double order like the value)
+// range = max(range, max |x - shift| over all n values) (the bits of a non-negative double order like the value)
 template <typename T>
 __global__ void knn_range_kernel(const T* __restrict__ x, long long n, int D, const double* __restrict__ shift,
                                  unsigned long long* __restrict__ range) {
@@ -158,19 +194,24 @@ __global__ void knn_scaled_kernel(const T* __restrict__ x, long long n, int D, c
   }
 }
 
-// Top-KP candidates of each query row by squared Euclidean distance, in the difference form.
-// ACC = float: the selection pass over all rows of x = the scaled rows y; also records each row's worst kept
-//   distance d32[q], which bounds the distance of every candidate it did not keep.
-// ACC = double: the rescan of the rows list[0 .. *count) on the input rows x, with the same formula (and so
-//   the same bits) as knn_refine_kernel; ties go to the lower index, as in the refine ranking.
-template <typename T, typename ACC, int DP, int KP>
+// Top-KP candidates of each query row xq[q] among the data rows of slice blockIdx.y (rows [y L, y L + L) of x), by
+// squared Euclidean distance in the difference form, written to cand[q][slice].
+// ACC = float: the selection pass on the scaled rows; also records the worst kept distance d32[q][slice], which bounds
+//   the distance of every candidate of the slice it did not keep.
+// ACC = double: the rescan of the queries list[0 .. *count) on the input rows, with the same formula (and so the same
+//   bits) as knn_refine_kernel; ties go to the lower index, as in the refine ranking.
+// SELF: the data is its own query set (xq == x), and query q enters its own list with distance -1, so it is kept.
+template <typename T, typename ACC, int DP, int KP, bool SELF>
 __global__ void __launch_bounds__(KNN_THREADS, 1)
-knn_select_kernel(const T* __restrict__ x, int N, int D, const int* __restrict__ list, const int* __restrict__ count,
-                  int* __restrict__ cand, float* __restrict__ d32) {
+knn_select_kernel(const T* __restrict__ xq, int Nq, const T* __restrict__ x, int N, int D, int L,
+                  const int* __restrict__ list, const int* __restrict__ count, int* __restrict__ cand,
+                  float* __restrict__ d32) {
   constexpr bool F64 = sizeof(ACC) == 8;
   __shared__ __align__(16) ACC tile[KNN_TILE * DP];
   extern __shared__ int sidx[];   // [KP][KNN_THREADS]
   const int tid = threadIdx.x;
+  const int S = gridDim.y, slice = blockIdx.y;
+  const int c_lo = slice * L, c_hi = min(N, c_lo + L);
   int q;
   if (F64) {
     const int n_list = *count;
@@ -179,32 +220,32 @@ knn_select_kernel(const T* __restrict__ x, int N, int D, const int* __restrict__
     q = p < n_list ? list[p] : -1;
   } else {
     q = blockIdx.x * KNN_THREADS + tid;
-    if (q >= N) q = -1;
+    if (q >= Nq) q = -1;
   }
-  ACC xq[DP];
+  ACC xr[DP];
 #pragma unroll
-  for (int d = 0; d < DP; ++d) xq[d] = (q >= 0 && d < D) ? (ACC)x[(long long)q * D + d] : (ACC)0;
+  for (int d = 0; d < DP; ++d) xr[d] = (q >= 0 && d < D) ? (ACC)xq[(long long)q * D + d] : (ACC)0;
   ACC dk[KP];
 #pragma unroll
   for (int j = 0; j < KP; ++j) {
     dk[j] = F64 ? (ACC)INFINITY : (ACC)FLT_MAX;
     sidx[j * KNN_THREADS + tid] = -1;
   }
-  for (int c0 = 0; c0 < N; c0 += KNN_TILE) {
+  for (int c0 = c_lo; c0 < c_hi; c0 += KNN_TILE) {
     __syncthreads();
     for (int e = tid; e < KNN_TILE * DP; e += KNN_THREADS) {
       const int r = e / DP, d = e - r * DP;
-      tile[e] = (c0 + r < N && d < D) ? (ACC)x[(long long)(c0 + r) * D + d] : (ACC)0;
+      tile[e] = (c0 + r < c_hi && d < D) ? (ACC)x[(long long)(c0 + r) * D + d] : (ACC)0;
     }
     __syncthreads();
-    const int nc = min(KNN_TILE, N - c0);
+    const int nc = min(KNN_TILE, c_hi - c0);
     for (int r = 0; r < nc; ++r) {
       ACC dist;
       if constexpr (F64) {
         double s = 0.0;
 #pragma unroll
         for (int d = 0; d < DP; ++d) {
-          const double e = xq[d] - tile[r * DP + d];
+          const double e = xr[d] - tile[r * DP + d];
           s = __fma_rn(e, e, s);
         }
         dist = fmin(s, DBL_MAX);   // an overflowed distance still fills an empty slot
@@ -214,8 +255,8 @@ knn_select_kernel(const T* __restrict__ x, int N, int D, const int* __restrict__
 #pragma unroll
         for (int d4 = 0; d4 < DP / 4; ++d4) {
           const float4 v = t4[d4];
-          const float e0 = xq[4 * d4] - v.x, e1 = xq[4 * d4 + 1] - v.y;
-          const float e2 = xq[4 * d4 + 2] - v.z, e3 = xq[4 * d4 + 3] - v.w;
+          const float e0 = xr[4 * d4] - v.x, e1 = xr[4 * d4 + 1] - v.y;
+          const float e2 = xr[4 * d4 + 2] - v.z, e3 = xr[4 * d4 + 3] - v.w;
           s0 = fmaf(e0, e0, s0);
           s1 = fmaf(e1, e1, s1);
           s0 = fmaf(e2, e2, s0);
@@ -224,7 +265,7 @@ knn_select_kernel(const T* __restrict__ x, int N, int D, const int* __restrict__
         dist = s0 + s1;
       }
       const int c = c0 + r;
-      if (c == q) dist = (ACC)-1;
+      if (SELF && c == q) dist = (ACC)-1;
       if (dist < dk[KP - 1]) {
 #pragma unroll
         for (int j = KP - 1; j > 0; --j) {
@@ -244,8 +285,9 @@ knn_select_kernel(const T* __restrict__ x, int N, int D, const int* __restrict__
     }
   }
   if (q >= 0) {
-    for (int j = 0; j < KP; ++j) cand[(long long)q * KP + j] = sidx[j * KNN_THREADS + tid];
-    if (!F64) d32[q] = (float)dk[KP - 1];
+    int* out = cand + ((long long)q * S + slice) * KP;
+    for (int j = 0; j < KP; ++j) out[j] = sidx[j * KNN_THREADS + tid];
+    if (!F64) d32[(long long)q * S + slice] = (float)dk[KP - 1];
   }
 }
 
@@ -270,33 +312,36 @@ __device__ __forceinline__ double knn_reject_bound(float t32, const unsigned lon
   return lb > 0.0 ? ldexp(lb * (1.0 - 0x1p-40), e) : 0.0;
 }
 
-// One warp per query: fp64 distances of the KP candidates, ranked by (distance, not-self, index); the first
-// k are written.  certify: queries 0..N-1, and a row whose k-th distance is not strictly below
-// knn_reject_bound (its candidates may miss a true neighbour) is appended to list for the fp64 rescan.
-// Otherwise: the rows list[0 .. *count).
-template <typename T>
-__global__ void knn_refine_kernel(const T* __restrict__ x, int N, int D, int DP, int KP, int k,
-                                  const int* __restrict__ cand, int certify, const float* __restrict__ d32,
-                                  const unsigned long long* __restrict__ range, int* __restrict__ list,
-                                  int* __restrict__ count, int* __restrict__ knn_idx, double* __restrict__ knn_dist) {
+// One warp per query: fp64 distances of its S * KP candidates (the slices' lists, which share no row), ranked by
+// (distance, index), with the query itself first when SELF; the first k are written.  certify: queries 0..Nq-1, and a
+// query whose k-th distance is not strictly below knn_reject_bound of the smallest of its slices' worst kept fp32
+// distances (a slice's dropped candidates are at least its own bound away) is appended to list for the fp64 rescan;
+// all_kept: no slice dropped a candidate.  Otherwise: the queries list[0 .. *count).
+template <typename T, bool SELF>
+__global__ void knn_refine_kernel(const T* __restrict__ xq, int Nq, const T* __restrict__ x, int D, int DP, int S,
+                                  int KP, int k, const int* __restrict__ cand, int certify, int all_kept,
+                                  const float* __restrict__ d32, const unsigned long long* __restrict__ range,
+                                  int* __restrict__ list, int* __restrict__ count, int* __restrict__ knn_idx,
+                                  double* __restrict__ knn_dist) {
   extern __shared__ double sref[];
+  const int C = S * KP;
   const int warps = blockDim.x / 32, w = threadIdx.x / 32, lane = threadIdx.x % 32;
-  double* sd = sref + w * KP;
-  int* si = reinterpret_cast<int*>(sref + warps * KP) + w * KP;
+  double* sd = sref + w * C;
+  int* si = reinterpret_cast<int*>(sref + warps * C) + w * C;
   int q = blockIdx.x * warps + w;
   if (certify) {
-    if (q >= N) return;
+    if (q >= Nq) return;
   } else {
     if (q >= *count) return;
     q = list[q];
   }
-  for (int j = lane; j < KP; j += 32) {
-    const int c = cand[(long long)q * KP + j];
+  for (int j = lane; j < C; j += 32) {
+    const int c = cand[(long long)q * C + j];
     double s = INFINITY;
     if (c >= 0) {
       s = 0.0;
       for (int d = 0; d < D; ++d) {
-        const double e = (double)x[(long long)q * D + d] - (double)x[(long long)c * D + d];
+        const double e = (double)xq[(long long)q * D + d] - (double)x[(long long)c * D + d];
         s = __fma_rn(e, e, s);
       }
     }
@@ -305,17 +350,17 @@ __global__ void knn_refine_kernel(const T* __restrict__ x, int N, int D, int DP,
   }
   __syncwarp();
   double kth = 0.0;   // the k-th fp64 squared distance
-  for (int j = lane; j < KP; j += 32) {
+  for (int j = lane; j < C; j += 32) {
     const int c = si[j];
     if (c < 0) continue;
     const double dj = sd[j];
-    const int kj = (c == q) ? -1 : c;
+    const int kj = (SELF && c == q) ? -1 : c;
     int rank = 0;
-    for (int i = 0; i < KP; ++i) {
+    for (int i = 0; i < C; ++i) {
       const int ci = si[i];
       if (ci < 0) continue;
       const double di = sd[i];
-      const int ki = (ci == q) ? -1 : ci;
+      const int ki = (SELF && ci == q) ? -1 : ci;
       rank += (di < dj) || (di == dj && ki < kj);
     }
     if (rank < k) {
@@ -324,10 +369,14 @@ __global__ void knn_refine_kernel(const T* __restrict__ x, int N, int D, int DP,
     }
     if (rank == k - 1) kth = dj;
   }
-  if (!certify || N <= KP) return;   // every row was a candidate
+  if (!certify || all_kept) return;
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) kth = fmax(kth, __shfl_xor_sync(0xffffffffu, kth, o));
-  if (lane == 0 && !(sqrt(kth) < knn_reject_bound(d32[q], range, D, DP))) list[atomicAdd(count, 1)] = q;
+  if (lane == 0) {
+    float t32 = FLT_MAX;
+    for (int sl = 0; sl < S; ++sl) t32 = fminf(t32, d32[(long long)q * S + sl]);
+    if (!(sqrt(kth) < knn_reject_bound(t32, range, D, DP))) list[atomicAdd(count, 1)] = q;
+  }
 }
 
 static int knn_padded(int k) {
@@ -341,64 +390,99 @@ static int knn_dpad(int D) {
   return -1;
 }
 
-template <typename T, typename ACC, int DP, int KP>
-static int knn_launch(const T* x, int N, int D, const KnnWs& w, cudaStream_t s) {
+struct KnnShape {
+  int Nq, N, D, KP, S, L;
+};
+
+template <typename T, typename ACC, int DP, int KP, bool SELF>
+static int knn_launch(const T* xq, const T* x, const KnnShape& sh, const KnnWs& w, cudaStream_t s) {
   const size_t smem = (size_t)KP * KNN_THREADS * sizeof(int);
-  auto kern = knn_select_kernel<T, ACC, DP, KP>;
+  auto kern = knn_select_kernel<T, ACC, DP, KP, SELF>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
     set_error("umap knn_select_kernel: cudaFuncSetAttribute failed");
     return 1;
   }
-  kern<<<(N + KNN_THREADS - 1) / KNN_THREADS, KNN_THREADS, smem, s>>>(x, N, D, w.list, w.count, w.cand, w.d32);
+  const dim3 grid((sh.Nq + KNN_THREADS - 1) / KNN_THREADS, sh.S);
+  kern<<<grid, KNN_THREADS, smem, s>>>(xq, sh.Nq, x, sh.N, sh.D, sh.L, w.list, w.count, w.cand, w.d32);
   return check_launch(sizeof(ACC) == 4 ? "umap knn_select_kernel" : "umap knn_select_kernel (fp64 rescan)");
 }
 
-template <typename T, typename ACC, int DP>
-static int knn_launch_k(const T* x, int N, int D, int KP, const KnnWs& w, cudaStream_t s) {
-  switch (KP) {
-    case 16: return knn_launch<T, ACC, DP, 16>(x, N, D, w, s);
-    case 32: return knn_launch<T, ACC, DP, 32>(x, N, D, w, s);
-    case 64: return knn_launch<T, ACC, DP, 64>(x, N, D, w, s);
-    default: return knn_launch<T, ACC, DP, 128>(x, N, D, w, s);
+template <typename T, typename ACC, int DP, bool SELF>
+static int knn_launch_k(const T* xq, const T* x, const KnnShape& sh, const KnnWs& w, cudaStream_t s) {
+  switch (sh.KP) {
+    case 16: return knn_launch<T, ACC, DP, 16, SELF>(xq, x, sh, w, s);
+    case 32: return knn_launch<T, ACC, DP, 32, SELF>(xq, x, sh, w, s);
+    case 64: return knn_launch<T, ACC, DP, 64, SELF>(xq, x, sh, w, s);
+    default: return knn_launch<T, ACC, DP, 128, SELF>(xq, x, sh, w, s);
   }
 }
 
-template <typename T, typename ACC>
-static int knn_select(const T* x, int N, int D, int KP, const KnnWs& w, cudaStream_t s) {
-  switch (knn_dpad(D)) {
-    case 8: return knn_launch_k<T, ACC, 8>(x, N, D, KP, w, s);
-    case 16: return knn_launch_k<T, ACC, 16>(x, N, D, KP, w, s);
-    case 32: return knn_launch_k<T, ACC, 32>(x, N, D, KP, w, s);
-    default: return knn_launch_k<T, ACC, 64>(x, N, D, KP, w, s);
+template <typename T, typename ACC, bool SELF>
+static int knn_select(const T* xq, const T* x, const KnnShape& sh, const KnnWs& w, cudaStream_t s) {
+  switch (knn_dpad(sh.D)) {
+    case 8: return knn_launch_k<T, ACC, 8, SELF>(xq, x, sh, w, s);
+    case 16: return knn_launch_k<T, ACC, 16, SELF>(xq, x, sh, w, s);
+    case 32: return knn_launch_k<T, ACC, 32, SELF>(xq, x, sh, w, s);
+    default: return knn_launch_k<T, ACC, 64, SELF>(xq, x, sh, w, s);
   }
 }
 
-// shift and range; fp32 selection; fp64 refine with the certificate; fp64 rescan and refine of the rows it
-// rejects (the last two launches find an empty list and return at once in the usual case)
+static KnnShape knn_shape(int Nq, int N, int D, int k) {
+  KnnShape sh;
+  sh.Nq = Nq;
+  sh.N = N;
+  sh.D = D;
+  sh.KP = knn_padded(k);
+  sh.S = knn_slices(Nq, N, sh.KP);
+  sh.L = knn_slice_rows(N, sh.S);
+  return sh;
+}
+
+// range and scaled rows of one row set
 template <typename T>
-static int knn_run(const T* x, int N, int D, int k, int* knn_idx, double* knn_dist, void* ws, cudaStream_t s) {
-  const int KP = knn_padded(k), DP = knn_dpad(D);
+static int knn_scale_rows(const T* x, int rows, int D, const KnnWs& w, float* y, bool range_only, cudaStream_t s) {
+  const long long n = (long long)rows * D;
+  if (range_only) {
+    knn_range_kernel<T><<<(unsigned)std::min<long long>((n + 255) / 256, 4 * kNumSMs), 256, 0, s>>>(x, n, D, w.shift,
+                                                                                                    w.range);
+    return check_launch("umap knn_range_kernel");
+  }
+  knn_scaled_kernel<T><<<(unsigned)std::min<long long>((n + 255) / 256, 8 * kNumSMs), 256, 0, s>>>(x, n, D, w.shift,
+                                                                                                   w.range, y);
+  return check_launch("umap knn_scaled_kernel");
+}
+
+// Queries xq [Nq, D] against data x [N, D] (SELF: xq == x).  Shift and range (over both sets); fp32 selection per
+// slice; fp64 refine with the certificate; fp64 rescan and refine of the queries it rejects (the last two launches
+// find an empty list and return at once in the usual case).
+template <typename T, bool SELF>
+static int knn_run(const T* xq, int Nq, const T* x, int N, int D, int k, int* knn_idx, double* knn_dist, void* ws,
+                   cudaStream_t s) {
+  const KnnShape sh = knn_shape(Nq, N, D, k);
+  const int DP = knn_dpad(D);
   KnnWs w;
-  knn_ws_layout(N, D, KP, ws, &w);
+  knn_ws_layout(Nq, N, D, sh.KP, sh.S, SELF, ws, &w);
   knn_shift_kernel<T><<<1, KNN_MAX_D, 0, s>>>(x, N, D, w.shift, w.range, w.count);
   if (check_launch("umap knn_shift_kernel")) return 1;
-  const long long n = (long long)N * D;
-  knn_range_kernel<T><<<(unsigned)std::min<long long>((n + 255) / 256, 4 * kNumSMs), 256, 0, s>>>(x, n, D, w.shift,
-                                                                                                  w.range);
-  if (check_launch("umap knn_range_kernel")) return 1;
-  knn_scaled_kernel<T><<<(unsigned)std::min<long long>((n + 255) / 256, 8 * kNumSMs), 256, 0, s>>>(x, n, D, w.shift,
-                                                                                                   w.range, w.y);
-  if (check_launch("umap knn_scaled_kernel")) return 1;
-  if (knn_select<float, float>(w.y, N, D, KP, w, s)) return 1;
-  constexpr int WARPS = 8;
-  const size_t smem = (size_t)WARPS * KP * (sizeof(double) + sizeof(int));
-  const unsigned grid = (unsigned)((N + WARPS - 1) / WARPS);
-  knn_refine_kernel<T><<<grid, WARPS * 32, smem, s>>>(x, N, D, DP, KP, k, w.cand, 1, w.d32, w.range, w.list, w.count,
-                                                      knn_idx, knn_dist);
+  if (knn_scale_rows(x, N, D, w, w.y, true, s)) return 1;
+  if (!SELF && knn_scale_rows(xq, Nq, D, w, w.yq, true, s)) return 1;
+  if (knn_scale_rows(x, N, D, w, w.y, false, s)) return 1;
+  if (!SELF && knn_scale_rows(xq, Nq, D, w, w.yq, false, s)) return 1;
+  if (knn_select<float, float, SELF>(w.yq, w.y, sh, w, s)) return 1;
+  const size_t smem = (size_t)KNN_REFINE_WARPS * sh.S * sh.KP * (sizeof(double) + sizeof(int));
+  auto refine = knn_refine_kernel<T, SELF>;
+  if (cudaFuncSetAttribute(refine, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+    set_error("umap knn_refine_kernel: cudaFuncSetAttribute failed");
+    return 1;
+  }
+  const unsigned grid = (unsigned)((Nq + KNN_REFINE_WARPS - 1) / KNN_REFINE_WARPS);
+  const int all_kept = sh.L <= sh.KP;
+  refine<<<grid, KNN_REFINE_WARPS * 32, smem, s>>>(xq, Nq, x, D, DP, sh.S, sh.KP, k, w.cand, 1, all_kept, w.d32,
+                                                   w.range, w.list, w.count, knn_idx, knn_dist);
   if (check_launch("umap knn_refine_kernel")) return 1;
-  if (knn_select<T, double>(x, N, D, KP, w, s)) return 1;
-  knn_refine_kernel<T><<<grid, WARPS * 32, smem, s>>>(x, N, D, DP, KP, k, w.cand, 0, w.d32, w.range, w.list, w.count,
-                                                      knn_idx, knn_dist);
+  if (knn_select<T, double, SELF>(xq, x, sh, w, s)) return 1;
+  refine<<<grid, KNN_REFINE_WARPS * 32, smem, s>>>(xq, Nq, x, D, DP, sh.S, sh.KP, k, w.cand, 0, all_kept, w.d32,
+                                                   w.range, w.list, w.count, knn_idx, knn_dist);
   return check_launch("umap knn_refine_kernel (rescanned rows)");
 }
 
@@ -421,6 +505,8 @@ __global__ void mean_kernel(const double* __restrict__ v, long long n, double* _
   if (threadIdx.x == 0) *out = red[0] / (double)n;
 }
 
+// BIPARTITE: the rows are queries against another row set (umap-learn's transform), so no entry is the row itself
+template <bool BIPARTITE>
 __global__ void smooth_knn_kernel(const int* __restrict__ knn_idx, const double* __restrict__ knn_dist, int N, int k,
                                   double local_connectivity, const double* __restrict__ mean_all,
                                   double* __restrict__ rho_out, double* __restrict__ sigma_out,
@@ -487,7 +573,7 @@ __global__ void smooth_knn_kernel(const int* __restrict__ knn_idx, const double*
   for (int j = 0; j < k; ++j) {
     const int c = knn_idx[(long long)i * k + j];
     double v;
-    if (c == i) v = 0.0;
+    if (!BIPARTITE && c == i) v = 0.0;
     else if (di[j] - rho <= 0.0 || sigma == 0.0) v = 1.0;
     else v = exp(-((di[j] - rho) / sigma));
     w[(long long)i * k + j] = v;
@@ -781,6 +867,113 @@ __global__ void sgd_epoch_kernel(float* __restrict__ emb, int N, int dim, const 
   next_neg[e] = next_neg[e] + (double)n_neg * en;
 }
 
+
+// --------------------------------------------------------------------------------- transform
+constexpr unsigned long long UMAP_S_TRANSFORM = 5ull << 32;   // stream tag of the transform's negative samples
+
+// umap.umap_.init_graph_transform: one thread per query row over its k (column, weight) entries in column order.
+// A weight of exactly 1 puts the row at that column's embedding; otherwise out += (w / row_sum) emb[col], the
+// product in fp64 and each sum rounded to fp32, as numba evaluates the float32 += float64 expression.
+__global__ void init_transform_kernel(const int* __restrict__ cols, const double* __restrict__ w, int Nq, int k,
+                                      const float* __restrict__ emb, int dim, float* __restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= Nq) return;
+  const int* ci = cols + (long long)i * k;
+  const double* wi = w + (long long)i * k;
+  double row_sum = 0.0;
+  for (int j = 0; j < k; ++j) row_sum = __dadd_rn(row_sum, wi[j]);
+  float o[UMAP_MAX_DIM];
+#pragma unroll
+  for (int d = 0; d < UMAP_MAX_DIM; ++d) o[d] = 0.f;
+  for (int j = 0; j < k; ++j) {
+    const float* e = emb + (long long)ci[j] * dim;
+    if (wi[j] == 1.0) {
+#pragma unroll
+      for (int d = 0; d < UMAP_MAX_DIM; ++d)
+        if (d < dim) o[d] = e[d];
+      break;
+    }
+    const double f = __ddiv_rn(wi[j], row_sum);
+#pragma unroll
+    for (int d = 0; d < UMAP_MAX_DIM; ++d)
+      if (d < dim) o[d] = (float)__dadd_rn((double)o[d], __dmul_rn(f, (double)e[d]));
+  }
+#pragma unroll
+  for (int d = 0; d < UMAP_MAX_DIM; ++d)
+    if (d < dim) out[(long long)i * dim + d] = o[d];
+}
+
+// umap.layouts.optimize_layout_euclidean(move_other=False) for the transform, all epochs in one launch.  Every edge
+// moves only its head, a query row, and reads only the fitted embedding, so one thread owns one query row: it keeps
+// the row in registers and walks its own edges [rowptr[i], rowptr[i + 1]) epoch by epoch.  No two threads write the
+// same memory, so the result is the sequential algorithm's and repeats bit for bit.  The arithmetic is
+// sgd_epoch_kernel's, except that a negative sample is never skipped (it is drawn from the other set).
+__global__ void sgd_transform_kernel(float* __restrict__ emb_q, int Nq, const float* __restrict__ emb, int N, int dim,
+                                     const long long* __restrict__ rowptr, const int* __restrict__ tail,
+                                     const double* __restrict__ eps, const double* __restrict__ eps_neg,
+                                     double* __restrict__ next, double* __restrict__ next_neg, int n_epochs, double a,
+                                     double b, double gamma, double alpha0, unsigned long long seed) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= Nq) return;
+  float cur[UMAP_MAX_DIM], oth[UMAP_MAX_DIM];
+#pragma unroll
+  for (int d = 0; d < UMAP_MAX_DIM; ++d) cur[d] = d < dim ? emb_q[(long long)i * dim + d] : 0.f;
+  const long long p0 = rowptr[i], p1 = rowptr[i + 1];
+  for (int n = 0; n < n_epochs; ++n) {
+    const double alpha = alpha0 * (1.0 - (double)n / (double)n_epochs);
+    for (long long e = p0; e < p1; ++e) {
+      const double nxt = next[e];
+      if (!(nxt <= (double)n)) continue;
+      const float* te = emb + (long long)tail[e] * dim;
+      double d2 = 0.0;
+#pragma unroll
+      for (int d = 0; d < UMAP_MAX_DIM; ++d) {
+        if (d >= dim) break;
+        oth[d] = __ldg(te + d);
+        const double t = (double)cur[d] - (double)oth[d];
+        d2 = __dadd_rn(d2, __dmul_rn(t, t));
+      }
+      double gc = 0.0;
+      if (d2 > 0.0) gc = (-2.0 * a * b * pow(d2, b - 1.0)) / (a * pow(d2, b) + 1.0);
+#pragma unroll
+      for (int d = 0; d < UMAP_MAX_DIM; ++d) {
+        if (d >= dim) break;
+        const double g = umap_clip(gc * ((double)cur[d] - (double)oth[d]));
+        cur[d] = (float)__dadd_rn((double)cur[d], __dmul_rn(g, alpha));
+      }
+      next[e] = nxt + eps[e];
+      const double en = eps_neg[e];
+      const double nn = next_neg[e];
+      const int n_neg = (int)(((double)n - nn) / en);
+      for (int p = 0; p < n_neg; ++p) {
+        const int kk = (int)(umap_hash(seed, (unsigned long long)n, (unsigned long long)e, (unsigned long long)p) %
+                             (unsigned long long)N);
+        const float* ke = emb + (long long)kk * dim;
+        double s = 0.0;
+#pragma unroll
+        for (int d = 0; d < UMAP_MAX_DIM; ++d) {
+          if (d >= dim) break;
+          oth[d] = __ldg(ke + d);
+          const double t = (double)cur[d] - (double)oth[d];
+          s = __dadd_rn(s, __dmul_rn(t, t));
+        }
+        double rc = 0.0;
+        if (s > 0.0) rc = (2.0 * gamma * b) / ((0.001 + s) * (a * pow(s, b) + 1.0));
+#pragma unroll
+        for (int d = 0; d < UMAP_MAX_DIM; ++d) {
+          if (d >= dim) break;
+          const double g = rc > 0.0 ? umap_clip(rc * ((double)cur[d] - (double)oth[d])) : 4.0;
+          cur[d] = (float)__dadd_rn((double)cur[d], __dmul_rn(g, alpha));
+        }
+      }
+      next_neg[e] = nn + (double)n_neg * en;
+    }
+  }
+#pragma unroll
+  for (int d = 0; d < UMAP_MAX_DIM; ++d)
+    if (d < dim) emb_q[(long long)i * dim + d] = cur[d];
+}
+
 }  // namespace ava
 
 using namespace ava;
@@ -789,7 +982,8 @@ using namespace ava;
 
 extern "C" long long ava_b200_umap_knn_ws_bytes(int N, int D, int k) {
   if (N < 1 || D < 1 || D > KNN_MAX_D || k < 1 || k > 100) return -1;
-  return knn_ws_layout(N, D, knn_padded(k), nullptr, nullptr);
+  const int KP = knn_padded(k);
+  return knn_ws_layout(N, N, D, KP, knn_slices(N, N, KP), true, nullptr, nullptr);
 }
 
 extern "C" int ava_b200_umap_knn(const void* x, int is_f32, int N, int D, int k, int* knn_idx, double* knn_dist,
@@ -800,8 +994,8 @@ extern "C" int ava_b200_umap_knn(const void* x, int is_f32, int N, int D, int k,
   AVA_REQUIRE(D >= 1 && D <= 64, "umap_knn: D=%d outside 1..64", D);
   AVA_REQUIRE(is_f32 == 0 || is_f32 == 1, "umap_knn: is_f32 must be 0 or 1");
   AVA_REQUIRE(ws_bytes >= ava_b200_umap_knn_ws_bytes(N, D, k), "umap_knn: workspace too small");
-  if (is_f32) return knn_run<float>((const float*)x, N, D, k, knn_idx, knn_dist, ws, s);
-  return knn_run<double>((const double*)x, N, D, k, knn_idx, knn_dist, ws, s);
+  if (is_f32) return knn_run<float, true>((const float*)x, N, (const float*)x, N, D, k, knn_idx, knn_dist, ws, s);
+  return knn_run<double, true>((const double*)x, N, (const double*)x, N, D, k, knn_idx, knn_dist, ws, s);
 }
 
 extern "C" int ava_b200_umap_smooth_knn(const int* knn_idx, const double* knn_dist, int N, int k,
@@ -813,8 +1007,8 @@ extern "C" int ava_b200_umap_smooth_knn(const int* knn_idx, const double* knn_di
   AVA_REQUIRE(local_connectivity >= 0.0, "umap_smooth_knn: local_connectivity must be >= 0");
   mean_kernel<<<1, 1024, 0, s>>>(knn_dist, (long long)N * k, ws);
   if (check_launch("umap mean_kernel")) return 1;
-  smooth_knn_kernel<<<(N + 127) / 128, 128, 0, s>>>(knn_idx, knn_dist, N, k, local_connectivity, ws, rho, sigma,
-                                                    weights);
+  smooth_knn_kernel<false><<<(N + 127) / 128, 128, 0, s>>>(knn_idx, knn_dist, N, k, local_connectivity, ws, rho,
+                                                           sigma, weights);
   return check_launch("umap smooth_knn_kernel");
 }
 
@@ -943,4 +1137,64 @@ extern "C" int ava_b200_umap_sgd_epoch(float* emb, int N, int dim, const int* he
   sgd_epoch_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(emb, N, dim, head, tail, eps, eps_neg, next, next_neg,
                                                              e0, e1, epoch, a, b, gamma, alpha, seed);
   return check_launch("umap sgd_epoch_kernel");
+}
+
+extern "C" long long ava_b200_umap_knn_query_ws_bytes(int Nq, int N, int D, int k) {
+  if (Nq < 0 || N < 1 || D < 1 || D > KNN_MAX_D || k < 1 || k > 100) return -1;
+  const KnnShape sh = knn_shape(Nq, N, D, k);
+  return knn_ws_layout(Nq, N, D, sh.KP, sh.S, false, nullptr, nullptr);
+}
+
+extern "C" int ava_b200_umap_knn_query(const void* q, int Nq, const void* x, int N, int is_f32, int D, int k,
+                                       int* knn_idx, double* knn_dist, void* ws, long long ws_bytes, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(x && ws && (Nq == 0 || (q && knn_idx && knn_dist)), "umap_knn_query: null pointer");
+  AVA_REQUIRE(Nq >= 0 && N >= 1 && k >= 1 && k <= 100 && k <= N,
+              "umap_knn_query: need Nq >= 0 and 1 <= k <= min(N, 100), got Nq=%d N=%d k=%d", Nq, N, k);
+  AVA_REQUIRE(D >= 1 && D <= 64, "umap_knn_query: D=%d outside 1..64", D);
+  AVA_REQUIRE(is_f32 == 0 || is_f32 == 1, "umap_knn_query: is_f32 must be 0 or 1");
+  AVA_REQUIRE(ws_bytes >= ava_b200_umap_knn_query_ws_bytes(Nq, N, D, k), "umap_knn_query: workspace too small");
+  if (Nq == 0) return 0;
+  if (is_f32) return knn_run<float, false>((const float*)q, Nq, (const float*)x, N, D, k, knn_idx, knn_dist, ws, s);
+  return knn_run<double, false>((const double*)q, Nq, (const double*)x, N, D, k, knn_idx, knn_dist, ws, s);
+}
+
+extern "C" int ava_b200_umap_smooth_knn_query(const int* knn_idx, const double* knn_dist, int Nq, int k,
+                                              double local_connectivity, double* rho, double* sigma, double* weights,
+                                              double* ws, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(knn_idx && knn_dist && rho && sigma && weights && ws, "umap_smooth_knn_query: null pointer");
+  AVA_REQUIRE(Nq >= 1 && k >= 2, "umap_smooth_knn_query: need Nq >= 1 and k >= 2");
+  AVA_REQUIRE(local_connectivity >= 0.0, "umap_smooth_knn_query: local_connectivity must be >= 0");
+  mean_kernel<<<1, 1024, 0, s>>>(knn_dist, (long long)Nq * k, ws);
+  if (check_launch("umap mean_kernel")) return 1;
+  smooth_knn_kernel<true><<<(Nq + 127) / 128, 128, 0, s>>>(knn_idx, knn_dist, Nq, k,
+                                                           std::max(0.0, local_connectivity - 1.0), ws, rho, sigma,
+                                                           weights);
+  return check_launch("umap smooth_knn_kernel (bipartite)");
+}
+
+extern "C" int ava_b200_umap_init_transform(const int* cols, const double* weights, int Nq, int k, const float* emb,
+                                            int N, int dim, float* out, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(cols && weights && emb && out, "umap_init_transform: null pointer");
+  AVA_REQUIRE(Nq >= 1 && k >= 1 && k <= N && dim >= 1 && dim <= UMAP_MAX_DIM, "umap_init_transform: bad arguments");
+  init_transform_kernel<<<(Nq + 127) / 128, 128, 0, s>>>(cols, weights, Nq, k, emb, dim, out);
+  return check_launch("umap init_transform_kernel");
+}
+
+extern "C" int ava_b200_umap_sgd_transform(float* emb_q, int Nq, const float* emb, int N, int dim,
+                                           const long long* rowptr, const int* tail, const double* eps,
+                                           const double* eps_neg, double* next, double* next_neg, int n_epochs,
+                                           double a, double b, double gamma, double initial_alpha,
+                                           unsigned long long seed, void* stream) {
+  UMAP_STREAM;
+  AVA_REQUIRE(emb_q && emb && rowptr && tail && eps && eps_neg && next && next_neg, "umap_sgd_transform: null pointer");
+  AVA_REQUIRE(Nq >= 1 && N >= 1 && dim >= 1 && dim <= UMAP_MAX_DIM && n_epochs >= 0,
+              "umap_sgd_transform: bad arguments");
+  if (n_epochs == 0) return 0;
+  sgd_transform_kernel<<<(Nq + 127) / 128, 128, 0, s>>>(emb_q, Nq, emb, N, dim, rowptr, tail, eps, eps_neg, next,
+                                                        next_neg, n_epochs, a, b, gamma, initial_alpha,
+                                                        umap_hash(seed, UMAP_S_TRANSFORM, 0, 0));
+  return check_launch("umap sgd_transform_kernel");
 }

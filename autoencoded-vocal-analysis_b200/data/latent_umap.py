@@ -28,6 +28,12 @@ positions are the PCA projection of their data-space centroids (umap-learn runs 
 the centroids), scaled to unit minimum spacing.  Stages 1-4 are bitwise reproducible from call to
 call; the layout is not (Hogwild), as umap-learn's parallel layout is not.
 
+``fit`` keeps the fitted rows and embedding on the device, and ``transform`` places new rows into that
+embedding without moving it (umap-learn's ``UMAP.transform``): exact neighbours of each new row among the
+fitted rows, the bipartite memberships (local_connectivity - 1), umap-learn's ``init_graph_transform``, and
+an SGD in which only the new rows move, one launch for all epochs with a thread per new row.  It has no
+races, so a transform repeats bit for bit and equals the sequential algorithm.
+
 ``DataContainer`` does not request ``latent_mean_umap`` through this class yet: the field still raises
 NotImplementedError there.  Wiring it is a few lines in ``DataContainer._make_field``.
 
@@ -45,7 +51,8 @@ MAX_D = 64            # the latent widths LatentPCA takes
 MAX_NEIGHBORS = 100   # top-k lists live in registers
 MAX_COMPONENTS = 8
 
-# streams of the counter-based generator (ava_b200_umap_random): tag << 32 | index
+# streams of the counter-based generator (ava_b200_umap_random): tag << 32 | index; tag 5 is the
+# transform's negative sampling (ava_b200_umap_sgd_transform derives its seed from it)
 _S_RANDOM_INIT, _S_NOISE, _S_LOBPCG, _S_FILL = 1, 2, 3, 4
 
 _LOBPCG_TOL = 1e-4      # residual norm of a unit eigenvector, relative to the largest wanted eigenvalue
@@ -72,6 +79,13 @@ def default_n_epochs(n):
     return 500 if n <= 10000 else 200
 
 
+def transform_n_epochs(n_epochs, n_queries):
+    """umap-learn's transform epochs: 100 up to 10 000 queries, 30 above, or n_epochs // 3."""
+    if n_epochs is None:
+        return 100 if n_queries <= 10000 else 30
+    return int(n_epochs) // 3
+
+
 def _stream(dev):
     return torch.cuda.current_stream(dev).cuda_stream
 
@@ -89,6 +103,82 @@ def knn(x, k):
     _lib.call("ava_b200_umap_knn", x.data_ptr(), 1 if x.dtype == torch.float32 else 0, N, D, k, idx.data_ptr(),
               dist.data_ptr(), ws.data_ptr(), ws_bytes, _stream(dev))
     return idx, dist
+
+
+def knn_query(q, x, k):
+    """Exact k nearest rows of x [N, D] for each row of q [Nq, D] (both float32 or both float64, on the
+    device): (indices [Nq, k] int32, Euclidean distances [Nq, k] float64), ranked by (distance, index)."""
+    Nq, D = q.shape
+    N = x.shape[0]
+    dev = x.device
+    ws_bytes = int(_lib.lib().ava_b200_umap_knn_query_ws_bytes(Nq, N, D, k))
+    ws = torch.empty(max(ws_bytes, 1), dtype=torch.uint8, device=dev)
+    idx = torch.empty(Nq, k, dtype=torch.int32, device=dev)
+    dist = torch.empty(Nq, k, dtype=torch.float64, device=dev)
+    _lib.call("ava_b200_umap_knn_query", q.data_ptr() if Nq else None, Nq, x.data_ptr(), N,
+              1 if x.dtype == torch.float32 else 0, D, k, idx.data_ptr() if Nq else None,
+              dist.data_ptr() if Nq else None, ws.data_ptr(), ws_bytes, _stream(dev))
+    return idx, dist
+
+
+def query_graph(knn_idx, knn_dist, local_connectivity=1.0):
+    """The bipartite graph of umap-learn's transform (queries x fitted rows, k entries per row):
+    rho, sigma, and cols / weights [Nq, k] with each row sorted by column.  local_connectivity is the
+    fitted model's (the kernel uses max(0, local_connectivity - 1))."""
+    Nq, k = knn_idx.shape
+    dev = knn_idx.device
+    rho = torch.empty(Nq, dtype=torch.float64, device=dev)
+    sigma = torch.empty(Nq, dtype=torch.float64, device=dev)
+    w = torch.empty(Nq, k, dtype=torch.float64, device=dev)
+    scratch = torch.empty(1, dtype=torch.float64, device=dev)
+    _lib.call("ava_b200_umap_smooth_knn_query", knn_idx.data_ptr(), knn_dist.data_ptr(), Nq, k,
+              float(local_connectivity), rho.data_ptr(), sigma.data_ptr(), w.data_ptr(), scratch.data_ptr(),
+              _stream(dev))
+    cols, order = torch.sort(knn_idx, dim=1)   # the columns of a row are distinct
+    return dict(rho=rho, sigma=sigma, cols=cols.contiguous(), weights=torch.gather(w, 1, order).contiguous())
+
+
+def init_transform(graph, emb):
+    """umap-learn's init_graph_transform from the unpruned graph: float32 [Nq, dim] on the device."""
+    Nq, k = graph["cols"].shape
+    N, dim = emb.shape
+    out = torch.empty(Nq, dim, dtype=torch.float32, device=emb.device)
+    _lib.call("ava_b200_umap_init_transform", graph["cols"].data_ptr(), graph["weights"].data_ptr(), Nq, k,
+              emb.data_ptr(), N, dim, out.data_ptr(), _stream(emb.device))
+    return out
+
+
+def transform_schedule(graph, n_epochs, negative_sample_rate=5.0):
+    """The transform's pruned edges (weights below max / n_epochs dropped) as row pointers and tails in
+    row-major, column-sorted order, with their SGD schedule."""
+    w = graph["weights"]
+    dev = w.device
+    Nq = w.shape[0]
+    vmax = w.max()
+    keep = w >= vmax / float(n_epochs)
+    rowptr = torch.zeros(Nq + 1, dtype=torch.int64, device=dev)
+    rowptr[1:] = torch.cumsum(keep.sum(1), 0)
+    vals = w[keep].contiguous()
+    out = dict(rowptr=rowptr, tail=graph["cols"][keep].contiguous(), weights=vals)
+    n = vals.numel()
+    for name in ("eps", "eps_neg", "next", "next_neg"):
+        out[name] = torch.empty(n, dtype=torch.float64, device=dev)
+    vmax_t = vmax.reshape(1).contiguous()
+    _lib.call("ava_b200_umap_epochs_per_sample", vals.data_ptr(), n, vmax_t.data_ptr(), int(n_epochs),
+              float(negative_sample_rate), out["eps"].data_ptr(), out["eps_neg"].data_ptr(), out["next"].data_ptr(),
+              out["next_neg"].data_ptr(), _stream(dev))
+    return out
+
+
+def sgd_transform(emb_q, emb, sched, n_epochs, a, b, gamma, initial_alpha, seed):
+    """All n_epochs of the transform's layout in one launch, in place on emb_q; emb (the fitted
+    embedding) is only read."""
+    Nq, dim = emb_q.shape
+    _lib.call("ava_b200_umap_sgd_transform", emb_q.data_ptr(), Nq, emb.data_ptr(), emb.shape[0], dim,
+              sched["rowptr"].data_ptr(), sched["tail"].data_ptr(), sched["eps"].data_ptr(),
+              sched["eps_neg"].data_ptr(), sched["next"].data_ptr(), sched["next_neg"].data_ptr(), int(n_epochs),
+              float(a), float(b), float(gamma), float(initial_alpha), seed & (2 ** 64 - 1), _stream(emb_q.device))
+    return emb_q
 
 
 def fuzzy_graph(knn_idx, knn_dist, local_connectivity=1.0):
@@ -363,7 +453,8 @@ def sgd_epoch(emb, sched, epoch, a, b, gamma, alpha, seed, e0=0, e1=None):
 
 
 class LatentUMAP:
-    """``umap.UMAP`` restricted to ``metric='euclidean'`` and ``fit_transform``, on the device.
+    """``umap.UMAP`` restricted to ``metric='euclidean'``, on the device: ``fit``, ``fit_transform`` and
+    ``transform``.
 
     The reference's projection (ava/data/data_container.py, _make_latent_mean_umap_projection) is
     ``LatentUMAP(n_components=2, n_neighbors=20, min_dist=0.1, random_state=42)``.  The defaults here
@@ -372,7 +463,9 @@ class LatentUMAP:
     Attributes after a fit: ``embedding_`` (numpy float32 [N, n_components]), ``graph_`` (the fuzzy
     simplicial set as a scipy CSR on the host, built when first read), ``knn_indices_`` and
     ``knn_dists_`` (numpy), ``a_``, ``b_``, ``n_epochs_``.  Same seed, same data: the neighbours, graph
-    and initialisation repeat bit for bit; the layout repeats up to the Hogwild races of its SGD."""
+    and initialisation repeat bit for bit; the layout repeats up to the Hogwild races of its SGD.
+    ``transform`` places new rows into the fitted embedding without moving it, and repeats bit for bit.
+    A fitted model pickles with its state on the host and transforms on any device after unpickling."""
 
     def __init__(self, n_neighbors=15, n_components=2, min_dist=0.1, spread=1.0, metric='euclidean', n_epochs=None,
                  learning_rate=1.0, init='spectral', negative_sample_rate=5, repulsion_strength=1.0,
@@ -425,16 +518,21 @@ class LatentUMAP:
             return int(self.random_state.randint(0, 2 ** 63 - 1, dtype=np.int64))
         return int(self.random_state)
 
-    def fit_transform_device(self, x):
-        """x: [N, D] numpy array or tensor, float32 or float64, D <= 64.  Returns the float32
-        [N, n_components] embedding as a tensor on the device."""
-        self._validate()
+    def _as_rows(self, x):
         if not torch.is_tensor(x):
             x = torch.from_numpy(np.ascontiguousarray(x))
         if x.dim() != 2:
             raise ValueError("expected a [N, D] array, got shape %s" % (tuple(x.shape),))
         if x.dtype not in (torch.float32, torch.float64):
             x = x.to(torch.float64)
+        return x
+
+    def fit(self, x):
+        """x: [N, D] numpy array or tensor, float32 or float64, D <= 64.  Fits the embedding and keeps
+        what ``transform`` needs on the device: the fitted rows (a contiguous device tensor is kept, not
+        copied), the float32 embedding, the neighbour count, ``a_``, ``b_`` and the seed.  Returns self."""
+        self._validate()
+        x = self._as_rows(x)
         N, D = x.shape
         if D > MAX_D or D < 1:
             raise ValueError("LatentUMAP takes 1 to %d input dimensions, got %d" % (MAX_D, D))
@@ -459,8 +557,8 @@ class LatentUMAP:
                 self.knn_dists_ = np.zeros((1, 1))
                 self._graph_dev = None
                 emb = torch.zeros(1, dim, dtype=torch.float32, device=dev)
-                self.embedding_ = emb.cpu().numpy()
-                return emb
+                self._keep_fit(x, emb, 1, 0)
+                return self
             k = int(self.n_neighbors)
             if N <= k:
                 warnings.warn("n_neighbors=%d is not smaller than the number of rows %d; using %d neighbours"
@@ -485,13 +583,77 @@ class LatentUMAP:
             self._graph_dev = graph
             self.knn_indices_ = idx.cpu().numpy()
             self.knn_dists_ = dist.cpu().numpy()
-            self.embedding_ = emb.cpu().numpy()
-        return emb
+            self._keep_fit(x, emb, k, seed)
+        return self
+
+    def _keep_fit(self, x, emb, k, seed):
+        self._fit_x, self._fit_emb, self._k, self._seed_ = x, emb, k, seed
+        self.embedding_ = emb.cpu().numpy()
+
+    def fit_transform_device(self, x):
+        """``fit(x)``, then the float32 [N, n_components] embedding as a tensor on the device."""
+        return self.fit(x)._fit_emb
 
     def fit_transform(self, x):
         """[N, D] -> numpy float32 [N, n_components] (what ``umap.UMAP.fit_transform`` returns)."""
-        self.fit_transform_device(x)
+        self.fit(x)
         return self.embedding_
+
+    def transform_device(self, x):
+        """Place new rows x [Nq, D] into the fitted embedding without moving it (umap-learn's
+        ``transform``): a float32 [Nq, n_components] tensor on the device.  The queries are converted to
+        the fitted rows' dtype.  A query set bitwise equal to the fitted rows returns a copy of the
+        embedding.  The layout's random draws come from the fit's seed, so repeated transforms of the
+        same rows are bitwise equal."""
+        if getattr(self, "_fit_x", None) is None:
+            raise RuntimeError("LatentUMAP.transform needs a fitted model: call fit first")
+        x = self._as_rows(x)
+        N, D = self._fit_x.shape
+        if x.shape[1] != D:
+            raise ValueError("the model was fitted on %d columns, got %d" % (D, x.shape[1]))
+        same_dtype = x.dtype == self._fit_x.dtype
+        x = x.to(self._fit_x.dtype)
+        if not bool(torch.isfinite(x).all()):
+            raise ValueError("x contains NaN or inf")
+        dev = self._device(x)
+        dim = int(self.n_components)
+        if x.shape[0] == 0:
+            return torch.empty(0, dim, dtype=torch.float32, device=dev)
+        # the fitted state follows the device of the latest call (it is on the host after unpickling)
+        self._fit_x = self._fit_x.to(dev)
+        self._fit_emb = self._fit_emb.to(dev)
+        x = x.to(dev).contiguous()
+        xf, emb = self._fit_x, self._fit_emb
+        with torch.cuda.device(dev):
+            if N == 1:
+                return emb[:1].repeat(x.shape[0], 1)
+            bits = torch.int32 if xf.dtype == torch.float32 else torch.int64
+            if same_dtype and x.shape == xf.shape and torch.equal(x.view(bits), xf.view(bits)):
+                return emb.clone()
+            idx, dist = knn_query(x, xf, self._k)
+            graph = query_graph(idx, dist, self.local_connectivity)
+            out = init_transform(graph, emb)
+            n_epochs = transform_n_epochs(self.n_epochs, x.shape[0])
+            if n_epochs > 0:
+                sched = transform_schedule(graph, n_epochs, self.negative_sample_rate)
+                sgd_transform(out, emb, sched, n_epochs, self.a_, self.b_, self.repulsion_strength,
+                              self.learning_rate / 4.0, self._seed_)
+        return out
+
+    def transform(self, x):
+        """[Nq, D] -> numpy float32 [Nq, n_components] (what ``umap.UMAP.transform`` returns)."""
+        return self.transform_device(x).cpu().numpy()
+
+    def __getstate__(self):
+        """A fitted model pickles with its state on the host; ``transform`` moves it to the device it runs on."""
+        st = self.__dict__.copy()
+        if st.get("_graph_dev") is not None:
+            st["_graph"] = self.graph_
+        st["_graph_dev"] = None
+        for name in ("_fit_x", "_fit_emb"):
+            if torch.is_tensor(st.get(name)):
+                st[name] = st[name].cpu()
+        return st
 
     @property
     def graph_(self):

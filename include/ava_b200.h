@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define AVA_B200_ABI_VERSION 8
+#define AVA_B200_ABI_VERSION 9
 #define AVA_NUM_BN_LAYERS 14
 #define AVA_STATS_STRIDE 64 /* doubles per layer in a stats block: [0..31]=sum, [32..63]=sum of squares */
 
@@ -413,16 +413,38 @@ int ava_b200_pca_transform(const void* x, int is_f32, long long N, int D, const 
  *   2^e ((sqrt(t32 - (DP + 1) 2^-149) / (1 + g)) - 2 delta sqrt(D)) (1 - 2^-40),
  * t32 the worst kept fp32 squared distance, DP the padded D, g = (DP/2 + 3) 2^-24 (1.001),
  * delta = (2^-24 + 2^-52) M 2^-e + 2^-149; or when N <= KP.  Other rows are rescanned in fp64.
+ * When the ceil(N / 128) query CTAs do not fill one wave, the rows are split into S slices (see
+ * ava_b200_umap_knn_query); the lists are exact and unique under the ranking order, so S changes no output.
  * ws: ava_b200_umap_knn_ws_bytes(N, D, k) bytes. */
 long long ava_b200_umap_knn_ws_bytes(int N, int D, int k);
 int ava_b200_umap_knn(const void* x, int is_f32, int N, int D, int k, int* knn_idx, double* knn_dist, void* ws,
                       long long ws_bytes, void* stream);
+/* Exact k nearest rows of x [N, D] for each query row of q [Nq, D] (umap-learn's transform searches its fitted
+ * index): the same dtype for both (is_f32), finite, D <= 64, 1 <= k <= min(N, 100), Nq >= 0.  Writes the first k
+ * rows by (distance, index) of fp64 difference-form distances, with no preference for any row: knn_idx [Nq, k]
+ * int32 (a query equal to a data row has it first, at distance 0; equal data rows come lowest index first),
+ * knn_dist [Nq, k] Euclidean, float64.  The same passes as ava_b200_umap_knn, with the shift taken from the data
+ * and the range M over the data and the queries together, so queries far outside the data stay exact.  When the
+ * Q = ceil(Nq / 128) query CTAs do not fill one wave of 4 CTAs per SM, the data rows are split into S slices
+ * (S * KP <= 256, slices of >= 1024 rows, the S whose Q S CTAs fill their last wave best; a larger S only if it
+ * fills 2% more), each keeping its own top KP; the fp64 pass ranks all S * KP candidates, and the certificate uses the
+ * smallest of the slices' worst kept fp32 distances.  ws: ava_b200_umap_knn_query_ws_bytes(Nq, N, D, k) bytes. */
+long long ava_b200_umap_knn_query_ws_bytes(int Nq, int N, int D, int k);
+int ava_b200_umap_knn_query(const void* q, int Nq, const void* x, int N, int is_f32, int D, int k, int* knn_idx,
+                            double* knn_dist, void* ws, long long ws_bytes, void* stream);
 /* umap.umap_.smooth_knn_dist (n_iter 64, tolerance 1e-5, MIN_K_DIST_SCALE 1e-3 against the row's mean
  * distance, or the mean of all N*k distances -- a fixed-order sum -- where rho = 0) followed by
  * umap.umap_.compute_membership_strengths, in fp64: rho [N], sigma [N], weights [N, k] (0 for the row
  * itself).  ws: 1 double of scratch. */
 int ava_b200_umap_smooth_knn(const int* knn_idx, const double* knn_dist, int N, int k, double local_connectivity,
                              double* rho, double* sigma, double* weights, double* ws, void* stream);
+/* The memberships of umap-learn's transform: smooth_knn_dist of the query lists of ava_b200_umap_knn_query with
+ * local_connectivity max(0, local_connectivity - 1) (pass the fitted model's value; the MIN_K_DIST_SCALE floor is
+ * against the mean of the Nq*k query distances), then compute_membership_strengths(bipartite=True): no entry is
+ * zeroed, as no query is a data row.  rho [Nq], sigma [Nq], weights [Nq, k] in the lists' order; ws: 1 double. */
+int ava_b200_umap_smooth_knn_query(const int* knn_idx, const double* knn_dist, int Nq, int k,
+                                   double local_connectivity, double* rho, double* sigma, double* weights, double* ws,
+                                   void* stream);
 /* The fuzzy union of umap.umap_.fuzzy_simplicial_set (set_op_mix_ratio 1): P = A + A^T - A.*A^T.
  * edge_keys writes 2*N*k keys: row*N + col for (i, j) and (j, i) of every neighbour j != i, -1 for the
  * self entries.  The caller sorts them and drops duplicates and -1 (nnz keys remain); graph then writes
@@ -472,6 +494,24 @@ int ava_b200_umap_sgd_epoch(float* emb, int N, int dim, const int* head, const i
                             const double* eps_neg, double* next, double* next_neg, long long e0, long long e1,
                             int epoch, double a, double b, double gamma, double alpha, unsigned long long seed,
                             void* stream);
+/* umap.umap_.init_graph_transform: for each query row i, over its k entries in increasing column order
+ * (cols/weights [Nq, k], the unpruned bipartite graph with each row sorted by column): a weight of exactly 1 sets
+ * out[i] = emb[col] and ends the row; otherwise out[i] += (w / row_sum) emb[col], row_sum the sequential fp64 sum
+ * of the row's weights in column order, each product in fp64 and each sum rounded to fp32 (no FMA).  emb [N, dim]
+ * is the fitted float32 embedding, out [Nq, dim] float32, dim <= 8. */
+int ava_b200_umap_init_transform(const int* cols, const double* weights, int Nq, int k, const float* emb, int N,
+                                 int dim, float* out, void* stream);
+/* umap.layouts.optimize_layout_euclidean(move_other=False) over all n_epochs of the transform in one launch: the
+ * pruned edges of query row i are [rowptr[i], rowptr[i + 1]) (tail: the fitted row; eps, eps_neg, next, next_neg
+ * from ava_b200_umap_epochs_per_sample), emb_q [Nq, dim] starts at the initialisation and is updated in place; the
+ * fitted embedding emb [N, dim] is only read.  Epoch n uses alpha = initial_alpha (1 - n / n_epochs).  The
+ * attraction moves the head only; negative sample p of edge e in epoch n is row
+ * umap_hash(umap_hash(seed, 5 << 32, 0, 0), n, e, p) mod N of emb, never skipped (at distance 0 the step is +4 per
+ * axis).  One thread per query row: race-free, so bitwise reproducible and equal to the sequential algorithm. */
+int ava_b200_umap_sgd_transform(float* emb_q, int Nq, const float* emb, int N, int dim, const long long* rowptr,
+                                const int* tail, const double* eps, const double* eps_neg, double* next,
+                                double* next_neg, int n_epochs, double a, double b, double gamma,
+                                double initial_alpha, unsigned long long seed, void* stream);
 
 #ifdef __cplusplus
 }
